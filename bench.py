@@ -24,8 +24,13 @@ evaluation ("strong" scaling: total work fixed).
 --impl reference: the reference's algorithm on the host cores, nothing extrapolated - every step is one full
 `bolt_gradient_estimation` as oracle/estimation.py restates it (scipy sparse kernels, factor.L().dot(Z) and all 128
 probe columns), on the multifrontal LAPACK factor with the analysis repeated per evaluation as the reference does.
-A step takes ~1-2 minutes, so the arm runs one warm-up and then as many timed steps as fit in --ref-budget seconds
-(at least one) and prints the number it EXECUTED in "steps" (the request is kept in "steps_requested").
+A step takes ~1-2 minutes, so the arm runs one warm-up (none with --warmup 0) and then --steps timed steps; with
+--ref-budget SECONDS it stops early once the next step would exceed the budget (at least one runs).  It prints the
+number it EXECUTED in "steps" (the request is kept in "steps_requested").
+
+--dump-outputs DIR writes what the last timed step computed (nll, gradient and, in the GPU arm, logdet, fixed
+effects, V^-1 y, V^-1 r, V^-1 C and the probe block W on a seeded sample of rows) as DIR/<name>.npy.  The inputs
+are generated from fixed seeds, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -41,11 +46,7 @@ import scipy.sparse as sp
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
-# The contract is ONE JSON line on stdout.  Libraries write to file descriptor 1 behind Python's back (NCCL prints
-# its version banner there on the first collective), so fd 1 is pointed at stderr for the whole run and the result
-# line goes to a private duplicate of the original stdout.
-_RESULT_OUT = os.fdopen(os.dup(1), "w")
-os.dup2(2, 1)
+_RESULT_OUT = None          # set by main(): importing this module leaves the process's stdout alone
 
 
 def emit(obj):
@@ -173,6 +174,29 @@ def measured_peaks():
         return {}
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(path, values, per_row=None, n=0):
+    """--dump-outputs: writes every array as <path>/<name>.npy in float64, so that two builds run with the same
+    arguments can be compared output for output.  `values` are written whole; the device tensors of `per_row` (n rows
+    each) are cut to one fixed, seeded sample of rows, the same rows for every tensor, as many as the 64 MB the whole
+    dump may take allow."""
+    os.makedirs(path, exist_ok=True)
+    out = {k: np.atleast_1d(np.asarray(v, dtype=np.float64)) for k, v in values.items()}
+    if per_row:
+        import torch
+        row_bytes = sum(8 * int(np.prod(v.shape[1:])) for v in per_row.values())
+        room = DUMP_BYTES - sum(a.nbytes for a in out.values()) - 1024 * (len(out) + len(per_row))   # npy headers
+        m = min(n, room // row_bytes)
+        rows = np.sort(np.random.default_rng(0).choice(n, m, replace=False)) if m < n else np.arange(n)
+        for k, v in per_row.items():
+            out[k] = v[torch.from_numpy(rows).to(v.device)].double().cpu().numpy()
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+    log("outputs of the last step written to %s: %s" % (path, {k: a.shape for k, a in out.items()}))
+
+
 # ------------------------------------------------------------------------------------------------ CPU arm
 def cpu_reml_sample(mats, cov, y, sig, reml, sim_num, sample_cols):
     """BOUNDED sample of one oracle REML evaluation on the host: assembly, analysis, factorization, logdet and
@@ -238,6 +262,12 @@ def cpu_he(mats, cov, y):
 
 # ------------------------------------------------------------------------------------------------ main
 def main():
+    # The contract is ONE JSON line on stdout.  Libraries write to file descriptor 1 behind Python's back (NCCL prints
+    # its version banner there on the first collective), so fd 1 is pointed at stderr for the whole run and the result
+    # line goes to a private duplicate of the original stdout.
+    global _RESULT_OUT
+    _RESULT_OUT = os.fdopen(os.dup(1), "w")
+    os.dup2(2, 1)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=3)
@@ -252,9 +282,19 @@ def main():
     ap.add_argument("--skip-he", action="store_true")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--cpu-cols", type=int, default=8)
-    ap.add_argument("--ref-budget", type=float, default=300.0, help="seconds of timed steps in --impl reference")
+    ap.add_argument("--ref-budget", type=float, default=None,
+                    help="--impl reference: stop early once the next timed step would take the steps past this many "
+                         "seconds (at least one runs); by default all --steps run")
     ap.add_argument("--skip-fit", action="store_true", help="skip the full REML() fit (wall time incl. setup)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float64, at most 64 MB; arrays "
+                         "with one row per individual are cut to a fixed, seeded sample of rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.ref_budget is not None:
+        # the probes are reseeded per step: a wall-time cut would make the dumped step depend on the machine's speed
+        ap.error("--dump-outputs cannot be combined with --ref-budget")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -281,15 +321,19 @@ def main():
             if i >= nwarm:
                 vals.append(dt)
             i += 1
-            if len(vals) >= args.steps or (len(vals) >= 1 and sum(vals) + dt > args.ref_budget):
+            if len(vals) >= args.steps or (args.ref_budget is not None and len(vals) >= 1 and
+                                           sum(vals) + dt > args.ref_budget):
                 break
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"nll": nll_c, "grad": grad_c})
         v = float(np.mean(vals))
         sample = ("oracle port, nothing extrapolated: %d full evaluations (oracle.estimation.reml_evaluation = the "
                   "reference's bolt_gradient_estimation line by line: scipy assembly, METIS analysis + multifrontal "
                   "LAPACK factorization repeated per call, logdet, fixed-effect solves, factor.L().dot(Z) and the "
-                  "solve for all %d probe columns, scipy SpMM reductions) after %d warm-up; %d steps were requested, "
-                  "the time budget (--ref-budget %.0f s) allowed %d" % (len(vals), args.probes, nwarm, args.steps,
-                                                                         args.ref_budget, len(vals)))
+                  "solve for all %d probe columns, scipy SpMM reductions) after %d warm-up; %d steps were requested"
+                  % (len(vals), args.probes, nwarm, args.steps))
+        if args.ref_budget is not None:
+            sample += ", the time budget (--ref-budget %g s) allowed %d" % (args.ref_budget, len(vals))
         emit({"impl": "reference", "metric": "reml_iter_time", "value": v, "unit": "s",
               "n_gpus": args.gpus, "steps": len(vals), "warmup": nwarm, "steps_requested": args.steps,
               "warmup_requested": args.warmup, "ms_per_step": v * 1e3, "higher_is_better": False,
@@ -359,6 +403,11 @@ def main():
     launches = E.launch_count()
     clocks = sampler.stop()
     step_ms = max_over_ranks(e0.elapsed_time(e1) / args.steps)
+    if args.dump_outputs and rank == 0:
+        # what evaluate() returns and keeps in ses.last; with N ranks W holds rank 0's probe columns
+        last = ses.last
+        dump_outputs(args.dump_outputs, {"nll": nll, "grad": grad, "logdet": last["logdet"], "beta": last["beta"]},
+                     {k: last[k] for k in ("Viy", "Vir", "ViC", "W")}, n)
 
     # factorization alone (Cholesky GFLOP/s of the metric) and solve / reduction phases
     def ev(fn, reps=2):
