@@ -201,6 +201,7 @@ class RemlSession(object):
         self.matset = _eng.MatSet(self.mats_host)
         self._groups = self.matset.pattern_groups(2)
         self._sym = [self.matset.is_symmetric(k) for k in range(K)]
+        self._ident = [self._is_identity(k) for k in range(K)]
         self.timings['upload_s'] = time.time() - t0
         t1 = time.time()
         leaders = sorted(set(self.matset.pattern_id(k) for k in range(K)))
@@ -334,10 +335,10 @@ class RemlSession(object):
             return _eng.upload_columns(Z, col_begin, col_end, torch), None
         return (Z[:, col_begin:col_end] if sliced else Z).contiguous().to("cuda", non_blocking=True), None
 
-    def probes(self, sim_num, Z=None, col_begin=0, col_end=None, pre=None):
+    def probes(self, sim_num, Z=None, col_begin=0, col_end=None, pre=None, probe_stream=None):
         """W = V^-1 (L Z)[argsort P]   (reference :49-52) for the probe columns [col_begin, col_end) of the
         n x sim_num block Z.  rng == 'device' draws ONLY those columns, from the counter-based stream keyed by
-        (functor.seed, evaluation index, row, global column): the same values for any number of GPUs.
+        (functor.seed, evaluation index or probe_stream, row, global column): the same values for any number of GPUs.
         pre: what prefetch_probes returned for the same arguments."""
         torch = self.torch
         col_end = sim_num if col_end is None else col_end
@@ -352,7 +353,8 @@ class RemlSession(object):
             elif self.functor.rng == 'host_buffer':       # caller-supplied host block (pinned tensor or ndarray)
                 Z = self.functor.probe_source(self.n, sim_num)
             else:
-                Z = self.eng.probe_normals(self.n, col_end - col_begin, col_begin, self.functor.seed, self.n_eval)
+                stream = self.n_eval if probe_stream is None else probe_stream
+                Z = self.eng.probe_normals(self.n, col_end - col_begin, col_begin, self.functor.seed, stream)
                 col_begin, col_end = 0, Z.shape[1]
         sliced = bool(col_begin or col_end != Z.shape[1])
         if not torch.is_tensor(Z):
@@ -369,8 +371,52 @@ class RemlSession(object):
         U = self.eng.lmul(Z)
         return self.eng.solve_(U)
 
-    def evaluate(self, sigmas, reml, sim_num, Z=None):
-        """One REML evaluation: nll and d nll / d sigma  (reference :77-117 without the exp chain rule)."""
+    def _is_identity(self, k):
+        m = self.mats_host[k]
+        return m.nnz == self.n and np.array_equal(m.indices, np.arange(self.n)) and np.all(m.data == 1.0)
+
+    def _ai_start(self, u, ViC):
+        """First half of the average-information matrix at u = P y = V^-1 r: B = [A_1 u | ... | A_K u] (one
+        store-enabled pass of the group SpMM per pattern group; the identity's column is u itself), the c x K
+        projection block ViC' B, and the K-column FORWARD half-sweep F = L^-1 P B queued on the auxiliary stream so
+        that it runs beside the quadratic-form pass the caller issues next.  _ai_finish joins the two."""
+        torch = self.torch
+        u1 = u.unsqueeze(1).contiguous()
+        B = torch.empty(self.n, self.K, dtype=torch.float64, device="cuda")
+        for ks in self._groups:
+            rest = [k for k in ks if not self._ident[k]]
+            for k in ks:
+                if self._ident[k]:
+                    B[:, k] = u
+            if rest:
+                _, stored = self.matset.coldot_multi(rest, u1, 0)
+                for g, k in enumerate(rest):
+                    B[:, k] = stored[g, :, 0]
+        CtB = ViC.t() @ B                              # read before the in-place solve below
+        self.eng.aux_begin()
+        try:
+            self.eng.solve_(B, mode=1)
+        finally:
+            self.eng.aux_end()
+        return B, CtB
+
+    def _ai_finish(self, pending, chol, reml):
+        """AI_ij = 1/2 b_i' P b_j = 1/2 [F_i'F_j - (ViC'b_i)' (C'V^-1C)^-1 (ViC'b_j)]: b'V^-1 b' = (L^-1 P b)'(L^-1 P b'),
+        and a Gram matrix does not depend on the row order.  ML (reml=False) drops the projection term."""
+        F, CtB = pending
+        self.eng.aux_join()
+        AI = (F.t() @ F).cpu().numpy()
+        if reml:
+            CtB = CtB.cpu().numpy()
+            AI -= CtB.T @ la.cho_solve(chol, CtB)
+        AI = 0.5 * AI
+        return 0.5 * (AI + AI.T)
+
+    def evaluate(self, sigmas, reml, sim_num, Z=None, ai=False, probe_stream=None):
+        """One REML evaluation: nll and d nll / d sigma  (reference :77-117 without the exp chain rule).
+        ai=True also returns the average-information matrix AI = -compute_hess (symmetric components only):
+        (nll, grad, AI).  probe_stream: index of the device probe stream (rng='device') to draw from instead of the
+        evaluation counter; an AI-REML fit keeps one for all its iterations."""
         torch = self.torch
         # probe columns are sharded across ranks when torch.distributed is initialised
         rank, world = _shard.rank_world()
@@ -381,11 +427,15 @@ class RemlSession(object):
         n = self.n
         pending = self._fixed_effects_start(self.overlap)   # narrow solve on the auxiliary stream ...
         # ... beside the probe pipeline
-        W = self.probes(sim_num, Z, lo, hi, pre=pre)
+        W = self.probes(sim_num, Z, lo, hi, pre=pre, probe_stream=probe_stream)
         self.n_eval += 1
         ViC, chol, beta, Viy = self._fixed_effects_finish(pending)
         beta_t = torch.from_numpy(beta).to("cuda")
         Vir = Viy - ViC @ beta_t                       # V^-1 (y - C beta) by linearity
+        if ai:
+            if not all(self._sym):
+                raise ValueError("the average-information matrix needs symmetric components")
+            ai_pending = self._ai_start(Vir, ViC)      # forward sweep on the auxiliary stream ...
         r = self.y - self.C @ beta_t
         nll = 0.5 * (float(r @ Vir) + n * LOG_2PI + logdet)
         if reml:
@@ -436,6 +486,8 @@ class RemlSession(object):
             for k in range(K):
                 grad[k] -= 0.5 * np.trace(la.cho_solve(chol, gram_h[k]))
         self.last = dict(logdet=logdet, beta=beta, ViC=ViC, Vir=Vir, Viy=Viy, W=W, chol=chol)
+        if ai:                                         # ... joined here; every rank computes it in full
+            return nll, grad, self._ai_finish(ai_pending, chol, reml)
         return nll, grad
 
 
@@ -518,16 +570,92 @@ def bolt_gradient_estimation(log_sig2g_array, cholesky_func, mats, covariates, y
     return nll, grad
 
 
-def estimate_var_comps(cholesky_func, mats, covariates, y, reml=True, sim_num=100, verbose=True, aireml=False):
-    """reference :120-144."""
+def _he_start(mats, covariates, y):
+    """reference :123-128: HE estimates of the first K-1 components, the rest to the identity, normalised."""
     he_est = HE(mats[:-1], covariates, y, compute_stderr=False)
     he_est = np.concatenate((he_est, [1 - he_est.sum()]))
     x0 = he_est
     if np.any(x0 < 0):
         x0 = np.ones((len(mats)))
-    x0 = x0 / x0.sum()
+    return x0 / x0.sum()
+
+
+# AI-REML (Gilmour, Thompson & Cullis 1995; with Monte-Carlo traces and one probe block per fit as in BOLT-REML,
+# Loh et al. 2015).  y is standardised by REML(), so an absolute floor is meaningful.
+AIREML_FLOOR = 1e-6       # smallest variance component
+AIREML_TOL = 1e-4         # stop when max |delta log sigma| < AIREML_TOL
+AIREML_MAX_ITER = 30
+
+
+def _aireml_step(sig, grad, AI):
+    """Fisher scoring in theta = log sigma: g_t = sigma o grad, H_t = D AI D, delta = -H_t^-1 g_t.
+    Boundary: a component on the floor whose score still points down (grad > 0) is fixed; a free component whose
+    linearised step is delta_k <= -1 (sigma_k (1 + delta_k) <= 0) goes to the floor in this step and is fixed, and the
+    others take the step of the reduced system with that move included.  The step is scaled to max |delta| <= 1.
+    Returns (new sigma, size of the step: max |delta| before the scaling, jumps to the floor included)."""
+    sig, grad = np.asarray(sig, dtype=float), np.asarray(grad, dtype=float)
+    K = sig.size
+    gt = sig * grad
+    Ht = sig[:, None] * AI * sig[None, :]
+    fixed = (sig <= AIREML_FLOOR) & (grad > 0)
+    while True:
+        free = np.flatnonzero(~fixed)
+        lin = np.where(fixed, (AIREML_FLOOR - sig) / sig, 0.0)     # linearised move of the fixed components
+        delta = np.zeros(K)
+        if free.size:
+            delta[free] = -np.linalg.solve(Ht[np.ix_(free, free)], gt[free] + Ht[free] @ lin)
+        hit = ~fixed & (delta <= -1.0)
+        if not hit.any():
+            break
+        fixed |= hit
+    size = float(np.max(np.abs(delta[free]))) if free.size else 0.0
+    if size > 1.0:
+        delta = delta / size
+    new = np.where(fixed, np.minimum(sig, AIREML_FLOOR), np.maximum(sig * np.exp(delta), AIREML_FLOOR))
+    if fixed.any():
+        size = max(size, float(np.max(np.log(sig[fixed] / new[fixed]))))
+    return new, size
+
+
+def _aireml_fit(functor, mats, covariates, y, reml, sim_num, verbose):
+    """HE start + AI-REML on the session.  Every iteration uses the SAME probe block (one numpy draw, one
+    probe_source call or one device stream index), so the fit is a deterministic root-finding problem.  Every rank
+    computes the AI matrix in full and takes the same step.  Returns (sigma, {'iterations', 'converged'})."""
+    sig = _he_start(mats, covariates, y)
+    ses = functor._session(mats, covariates, y)
+    if not all(ses._sym):
+        raise ValueError("aireml=True needs symmetric components (AI = -hess holds only for symmetric A_k); "
+                         "asymmetric: %s" % [k for k in range(ses.K) if not ses._sym[k]])
+    Z, stream = None, None
+    if functor.rng == 'numpy':
+        Z = np.random.randn(ses.n, sim_num)
+    elif functor.rng == 'host_buffer':
+        Z = functor.probe_source(ses.n, sim_num)
+    else:
+        stream = ses.n_eval
+    converged, it = False, 0
+    while it < AIREML_MAX_ITER:
+        it += 1
+        if verbose:
+            t0 = time.time()
+        nll, grad, AI = ses.evaluate(sig, reml, sim_num, Z=Z, ai=True, probe_stream=stream)
+        sig, size = _aireml_step(sig, grad, AI)
+        if verbose:
+            print('AI-REML iteration %d: nll %0.8e, sigma %s, max |step| %.3e, %.2f seconds'
+                  % (it, nll, sig, size, time.time() - t0))
+        if size < AIREML_TOL:
+            converged = True
+            break
+    if not converged:
+        print('optimization failed with message: AI-REML did not converge in %d iterations' % AIREML_MAX_ITER)
+    return sig, {"iterations": it, "converged": converged}
+
+
+def estimate_var_comps(cholesky_func, mats, covariates, y, reml=True, sim_num=100, verbose=True, aireml=False):
+    """reference :120-144.  aireml=True: average-information REML (_aireml_fit) instead of L-BFGS-B."""
     if aireml:
-        raise NotImplementedError('AI-REML is broken')
+        return _aireml_fit(_need_functor(cholesky_func), mats, covariates, y, reml, sim_num, verbose)[0]
+    x0 = _he_start(mats, covariates, y)
     optObj = optimize.minimize(bolt_gradient_estimation, np.log(x0),
                                args=(cholesky_func, mats, covariates, y, reml, sim_num, verbose, True),
                                jac=True, method='L-BFGS-B', options={'eps': 1e-5, 'ftol': 1e-7})
@@ -598,13 +726,17 @@ def compute_varcomp_stderr(mats, covariates, factor, y, sim_num):
     return np.sqrt(np.diag(inv_neg_hess) * (1 + 1.0 / sim_num))
 
 
-def REML(cholesky_func, mats, covariates, y, reml=True, sim_num=100, verbose=False):
+def REML(cholesky_func, mats, covariates, y, reml=True, sim_num=100, verbose=False, aireml=False):
     """reference :177-189.  Returns the reference's three keys plus 'nll' (the log-likelihood the reference
-    computes at :103 but drops) and 'engine' statistics."""
+    computes at :103 but drops) and 'engine' statistics.  aireml=True fits the variance components by AI-REML
+    (see _aireml_fit) and adds the key 'aireml': {'iterations', 'converged'}."""
     functor = _need_functor(cholesky_func)
     y = y / y.std()
     mats = mats + [sparse.eye(y.shape[0]).tocsr()]
-    varcomp_estimates = estimate_var_comps(functor, mats, covariates, y, reml, sim_num, verbose)
+    if aireml:
+        varcomp_estimates, ai_info = _aireml_fit(functor, mats, covariates, y, reml, sim_num, verbose)
+    else:
+        varcomp_estimates = estimate_var_comps(functor, mats, covariates, y, reml, sim_num, verbose)
     ses = functor._session(mats, covariates, y)
     factor = ses.factor_at(varcomp_estimates)
     ViC, chol, fixed_effects, Viy = ses.fixed_effects()
@@ -617,11 +749,14 @@ def REML(cholesky_func, mats, covariates, y, reml=True, sim_num=100, verbose=Fal
         nll += 0.5 * 2 * np.sum(np.log(np.diag(chol[0])))
     hess = _hess_device(ses, ses.eng, pre=(ViC, chol, Viy))
     sigmas_sigmas = np.sqrt(np.diag(la.inv(-hess)) * (1 + 1.0 / sim_num))
-    return {"covariance coefficients": varcomp_estimates,
-            "covariates coefficients": fixed_effects,
-            "covariance std": sigmas_sigmas,
-            "nll": nll,
-            "engine": ses.eng.stats()}
+    out = {"covariance coefficients": varcomp_estimates,
+           "covariates coefficients": fixed_effects,
+           "covariance std": sigmas_sigmas,
+           "nll": nll,
+           "engine": ses.eng.stats()}
+    if aireml:
+        out["aireml"] = ai_info
+    return out
 
 
 # ------------------------------------------------------------------------------------------- Haseman-Elston
