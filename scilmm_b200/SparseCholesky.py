@@ -13,7 +13,6 @@ which is the structural change against the reference (it re-analyses on every ca
 There is no CPU fallback: without the CUDA library these functions raise.
 """
 import hashlib
-import os
 import time
 
 import numpy as np
@@ -239,12 +238,11 @@ class RemlSession(object):
         # tiled copies (fill-reducing order, 64 rows x 64 distinct columns) of the symmetric matrices for the
         # quadratic-form / Gram pass of compute_gradients; tiny matrices (the identity) keep the row-per-warp kernel
         t1 = time.time()
-        self.use_tiles = os.environ.get("SLMM_TILES", "1") != "0"
-        if self.use_tiles:
-            for ks in self._groups:
-                if all(self._sym[k] for k in ks) and self.matset.nnz[ks[0]] >= 8 * self.n:
-                    for k in ks:
-                        self.matset.build_tiles(k, self.eng)
+        self.use_tiles = True
+        for ks in self._groups:
+            if all(self._sym[k] for k in ks) and self.matset.nnz[ks[0]] >= 8 * self.n:
+                for k in ks:
+                    self.matset.build_tiles(k, self.eng)
         self.timings['tiles_s'] = time.time() - t1
         self.C = _eng.to_device(np.asarray(covariates, dtype=np.float64), torch)
         self.y = _eng.to_device(np.asarray(y, dtype=np.float64), torch)

@@ -265,21 +265,6 @@ struct Launch {
   int64_t aux_off = 0;
 };
 
-static bool skinny_dmma_on(int flavour) {       // SLMM_F1_DMMA=0 / SLMM_F2_DMMA=0: register-blocked streaming kernels only
-  static int on[3] = {-1, -1, -1};
-  if (on[flavour] < 0) {
-    const char* e = getenv(flavour == 1 ? "SLMM_F1_DMMA" : "SLMM_F2_DMMA");
-    on[flavour] = (e && e[0] == '0') ? 0 : 1;
-  }
-  return on[flavour] == 1;
-}
-
-static bool tma_enabled() {
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("SLMM_TMA"); on = (e && e[0] == '0') ? 0 : 1; }
-  return on == 1;
-}
-
 // cuTensorMapEncodeTiled through the runtime's driver entry point (the library does not link libcuda: it must load
 // on machines without a driver for the host-only analysis).  2-D FP64 tensor: dim 0 = rows (contiguous), dim 1 = k
 // with a stride of `ld` elements; boxes of 16 x 16 elements, 128-byte swizzle.
@@ -376,14 +361,14 @@ struct Schedule {
 struct PhaseBuilder {
   std::vector<GemmOp> big, small, sk1, sk2;   // sk1 / sk2: narrow-RHS streaming flavours (skinny_ops.cuh)
   std::vector<GemmOp> tma;                    // big-tile ops whose operands a tensor map can describe (dense_tiles_tma.cuh)
-  int skinny_mt = 0;                          // > 0: ops with M <= 16 take the streaming kernels (row template MT)
+  int skinny_mt = 0;                          // > 0: ops with M <= skinny_mt take the streaming kernels (row template MT)
   int ws_id = 0;                              // which split-K workspace this builder's partial products use
   std::vector<PotrfOp> potrf;
   std::vector<ReduceOp> reduces;
   int64_t ws_used = 0;
   bool allow_split = true;    // builders whose launches run beside another builder's must not share the split-K workspace
   static bool tma_ok(const GemmOp& op) {
-    return tma_enabled() && op.a_si == 1 && op.b_sj == 1 && op.a_kidx == nullptr && !(op.flags & GF_TRIL_B) &&
+    return op.a_si == 1 && op.b_sj == 1 && op.a_kidx == nullptr && !(op.flags & GF_TRIL_B) &&
            (op.a_sk % 2) == 0 && (op.b_sk % 2) == 0 && op.a_sk > 0 && op.b_sk > 0 && op.K >= 64;
   }
   void push(const GemmOp& op, bool small_tiles) {
@@ -460,9 +445,8 @@ struct PhaseBuilder {
     // lower-masked updates inside a wide front's diagonal block (K = 64 in-block steps, the K = 1024 update of the next
     // block's 1024 x 1024 diagonal part): at most 36 useful 128 x 128 tiles sit on the critical chain with one long K
     // loop each; 64 x 64 tiles put 4x the CTAs on it (0.152 -> ~0.05 ms for the K = 1024 step, 25 -> ~13 us for K = 64)
-    static const bool chain_small = !(getenv("SLMM_CHAIN_SMALL") && getenv("SLMM_CHAIN_SMALL")[0] == '0');
     const bool small_tiles = !force_big && (!(op.M > 64 && op.N > 64) || (!lower && tb < 40 && op.K >= 128) ||
-                                            (chain_small && lower && tb <= 64));
+                                            (lower && tb <= 64));
     const int64_t tiles = small_tiles ? ts : tb;
     if (allow_split && !lower && (op.flags & GF_TRIL_B) && op.K >= 4096 && op.C != op.A && !small_tiles) {
       // L11 * Z of a wide front: the tile of the last 128 columns would run the whole K = ns alone (one CTA, 2.7 ms at
@@ -669,13 +653,10 @@ static void init_kernel_attributes() {
   CUDA_OK(cudaFuncSetAttribute(gemm_tiles_kernel<64, 64, 2, 2, SMALL_STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMALL_SMEM));
   CUDA_OK(cudaFuncSetAttribute(potrf_inv_kernel_v4, cudaFuncAttributeMaxDynamicSharedMemorySize, POTRF4_SMEM));
   CUDA_OK(cudaFuncSetAttribute(gemm_tiles_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TMA_SMEM));
-  CUDA_OK(cudaFuncSetAttribute(skinny_f2_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, SK_F2_KMAX * 12 * 8));
-  CUDA_OK(cudaFuncSetAttribute(skinny_f2_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, SK_F2_KMAX * 16 * 8));
 #define SKD_ATTR(NMT)                                                                                                         \
   CUDA_OK(cudaFuncSetAttribute(skinny_f2_dmma_kernel<NMT>, cudaFuncAttributeMaxDynamicSharedMemorySize, SkDmma<NMT>::SMEM));   \
-  CUDA_OK(cudaFuncSetAttribute(skinny_f1_dmma_kernel<NMT>, cudaFuncAttributeMaxDynamicSharedMemorySize,                       \
-                               8 * NMT * ((NMT <= 4 ? 256 : 128) + 4) * (int)sizeof(double)));
-  SKD_ATTR(1) SKD_ATTR(2) SKD_ATTR(4) SKD_ATTR(8)
+  CUDA_OK(cudaFuncSetAttribute(skinny_f1_dmma_kernel<NMT>, cudaFuncAttributeMaxDynamicSharedMemorySize, SkDmma<NMT>::F1_SMEM));
+  SKD_ATTR(1) SKD_ATTR(2) SKD_ATTR(4)
 #undef SKD_ATTR
   done = true;
 }
@@ -715,31 +696,22 @@ static void launch_one(slmm_chol* h, const Schedule& sch, const Launch& L, const
       const GemmOp* ops = sch.d_gemm + L.off;
       const int32_t* top = sch.d_tile_op + L.tile_off;
       const bool f1 = L.kind == Launch::SKINNY_F1;
-      const bool f2_dmma = skinny_dmma_on(2);
-      const bool f1_dmma = skinny_dmma_on(1);
-#define SKD_CASE(NMT)                                                                                                   \
-  if (f1) skinny_f1_dmma_kernel<NMT><<<L.grid, 256, 8 * NMT * ((NMT <= 4 ? 256 : 128) + 4) * sizeof(double), st>>>(ops, top); \
+#define SKD_CASE(NMT)                                                                          \
+  if (f1) skinny_f1_dmma_kernel<NMT><<<L.grid, 256, SkDmma<NMT>::F1_SMEM, st>>>(ops, top);  \
   else skinny_f2_dmma_kernel<NMT><<<L.grid, 256, SkDmma<NMT>::SMEM, st>>>(ops, top);
-      if (L.child_parity >= 8 && (f1 ? f1_dmma : f2_dmma)) {   // 5..64 right-hand sides: streaming on the tensor pipe
-        if (L.child_parity == 8) { SKD_CASE(1) }
-        else if (L.child_parity <= 16) { SKD_CASE(2) }
-        else if (L.child_parity <= 32) { SKD_CASE(4) }
-        else { SKD_CASE(8) }
-        break;
-      }
-#undef SKD_CASE
-#define SK_CASE(MT)                                                                                          \
-  if (f1) skinny_f1_kernel<MT><<<L.grid, SK_F1_COLS, 0, st>>>(ops, top);                                     \
+#define SK_CASE(MT)                                                                        \
+  if (f1) skinny_f1_kernel<MT><<<L.grid, SK_F1_COLS, 0, st>>>(ops, top);                   \
   else skinny_f2_kernel<MT><<<L.grid, 256, SK_F2_KMAX * MT * sizeof(double), st>>>(ops, top);
       switch (L.child_parity) {
         case 1: SK_CASE(1) break;
         case 2: SK_CASE(2) break;
         case 4: SK_CASE(4) break;
-        case 8: SK_CASE(8) break;
-        case 12: SK_CASE(12) break;
-        default: SK_CASE(16) break;
+        case 8: SKD_CASE(1) break;
+        case 16: SKD_CASE(2) break;
+        default: SKD_CASE(4) break;
       }
 #undef SK_CASE
+#undef SKD_CASE
       break;
     }
     case Launch::INIT_W:
@@ -761,7 +733,7 @@ static bool is_kernel(const Launch& L) { return L.kind != Launch::EV_RECORD && L
 //
 // The lists are static (every kernel argument is fixed once the schedule is uploaded), so each one is captured
 // ONCE into a CUDA graph and replayed: a 12-column solve is a chain of ~1000 tiny launches whose cost was the
-// host's launch rate, not the kernels (SLMM_GRAPHS=0 falls back to launch-by-launch).
+// host's launch rate, not the kernels.
 static void issue_schedule(slmm_chol* h, const Schedule& sch, double* X, double* const* vec_arena,
                            const int64_t* d_vptr, int nrhs, bool two, cudaStream_t one,
                            std::vector<cudaEvent_t>* per_launch = nullptr) {
@@ -778,18 +750,6 @@ static void issue_schedule(slmm_chol* h, const Schedule& sch, double* X, double*
     }
     nk++;
   }
-}
-
-static bool skinny_enabled() {
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("SLMM_SKINNY"); on = (e && e[0] == '0') ? 0 : 1; }
-  return on == 1;
-}
-
-static bool graphs_enabled() {
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("SLMM_GRAPHS"); on = (e && e[0] == '0') ? 0 : 1; }
-  return on == 1;
 }
 
 // Captures the launch list into a graph.  Capture happens on the (non-blocking) priority stream - the legacy
@@ -865,7 +825,7 @@ static void run_schedule(slmm_chol* h, Schedule& sch, double* X, double* const* 
     }
     // graphs for the single-stream lists only: replaying the look-ahead pair from a graph loses the stream priorities
     // the chain relies on (measured: factorization 183 -> 190 ms at the 250K config)
-    const bool use_graph = graphs_enabled() && !two && h->s_main != nullptr && !sch.graph_failed;
+    const bool use_graph = !two && h->s_main != nullptr && !sch.graph_failed;
     if (use_graph && sch.gexec[gi] == nullptr) {
       try {
         sch.gexec[gi] = capture_schedule(h, sch, X, vec_arena, d_vptr, nrhs, two);
@@ -1252,15 +1212,12 @@ static SolvePlan* get_plan(slmm_chol* h, int nrhs) {
   // consecutive diagonal blocks are serialised (same rows), and the late ones have far fewer tiles than SMs: without
   // split-K each still costs one full-K tile latency (170 us at the 250K config whatever its size)
   pb_rest.ws_id = 1;
-  // narrow blocks: HBM-streaming kernels instead of DMMA tiles (skinny_ops.cuh).  Up to 16 columns always; up to
-  // SLMM_SKINNY_MAX (default 32: the local probe block at 4 GPUs) on the tensor-pipe streaming kernels.  Measured at
-  // the 250K config, solve / L*Z in ms, tiles -> streaming: 32 columns 7.7 -> 6.3 / 3.6 -> 2.2; 64 columns
-  // 8.2 -> 9.6 / 3.9 -> 3.7 (16 DMMA per streamed fragment: the tensor pipe, not HBM, bounds the stream there).
-  static const int skinny_max = !(skinny_dmma_on(1) && skinny_dmma_on(2)) ? 16 :
-      getenv("SLMM_SKINNY_MAX") ? std::max(16, std::min(64, atoi(getenv("SLMM_SKINNY_MAX")))) : 32;
-  if (nrhs <= skinny_max && skinny_enabled())
-    pb.skinny_mt = nrhs <= 1 ? 1 : nrhs <= 2 ? 2 : nrhs <= 4 ? 4 : nrhs <= 8 ? 8 : nrhs <= 12 ? 12 : nrhs <= 16 ? 16 : nrhs <= 32 ? 32 : 64;
-  const bool lookahead = nrhs >= 64 && pb.skinny_mt == 0;     // narrow solves are launch-latency chains: nothing to overlap with
+  // narrow blocks, up to 32 columns (the local probe block at 4 GPUs): HBM-streaming kernels instead of DMMA tiles
+  // (skinny_ops.cuh).  Measured at the 250K config, solve / L*Z in ms, tiles -> streaming: 32 columns 7.7 -> 6.3 /
+  // 3.6 -> 2.2; 64 columns 8.2 -> 9.6 / 3.9 -> 3.7 (16 DMMA per streamed fragment: the tensor pipe, not HBM, bounds
+  // the stream there).
+  if (nrhs <= 32) pb.skinny_mt = nrhs <= 1 ? 1 : nrhs <= 2 ? 2 : nrhs <= 4 ? 4 : nrhs <= 8 ? 8 : nrhs <= 16 ? 16 : 32;
+  const bool lookahead = nrhs >= 64;     // narrow solves are launch-latency chains: nothing to overlap with
   int last_bulk_ev = -1;
   // One phase: the chain's launches on the main stream; look-ahead remainders (if any) on the bulk stream, after
   // the diagonal step that produced their operand and before anything that touches the same rows again.

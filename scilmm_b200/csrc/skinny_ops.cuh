@@ -1,29 +1,34 @@
-// Narrow right-hand sides (nrhs <= 16): the supernode-blocked triangular solves and L*Z as HBM-STREAMING kernels.
+// Narrow right-hand sides (nrhs <= 32): the supernode-blocked triangular solves and L*Z as HBM-STREAMING kernels.
 //
 // factor(b) for the c+1 fixed-effect columns, a single phenotype vector, the K and K(K+1)/2 columns of compute_hess
-// (reference scilmm/SparseCholesky.py:30,32,100,149,153) and the per-GPU probe slice at 8 GPUs all have at most 16
-// columns.  There every GemmOp of the solve schedules is  C(M x N) (+/-)= A(M x K) B(N x K)^T  with M = nrhs: 2*M flops
-// per 8 bytes of L - far below the machine balance - so the bound is HBM (each sweep reads L once: 8*nnz(L) bytes),
-// not the tensor pipe.  The DMMA tile kernel wastes a 64-row tile on <= 16 rows, pays a producer/consumer hand-off per
-// 16-wide K slab and reached 1.2 TB/s on the 12-column solve of the 250K config; these kernels keep the M accumulators
-// of one output column in registers, stage the small A operand in shared memory and stream B with many independent
-// coalesced loads per thread.  Same GemmOp descriptors, same schedules, same deterministic split-K reduction.
+// (reference scilmm/SparseCholesky.py:30,32,100,149,153), the K-column forward half-sweep of AI-REML and the per-GPU
+// probe slice at 4 or more GPUs all have at most 32 columns.  There every GemmOp of the solve schedules is
+// C(M x N) (+/-)= A(M x K) B(N x K)^T  with M = nrhs: 2*M flops per 8 bytes of L - far below the machine balance - so
+// the bound is HBM (each sweep reads L once: 8*nnz(L) bytes), not the tensor pipe.  The DMMA tile kernel wastes a
+// 64-row tile on <= 32 rows, pays a producer/consumer hand-off per 16-wide K slab and reached 1.2 TB/s on the 12-column
+// solve of the 250K config; these kernels stage the small A operand in shared memory, stream B from global memory
+// with many independent loads and keep the accumulators in registers.  Same GemmOp descriptors, same schedules, same
+// deterministic split-K reduction.
 //
 // Two flavours, by the memory layout of B (the factor panel or an inverse block):
-//   F1  B(j,k) = B[j + k*b_sk]   consecutive OUTPUT columns j are contiguous (forward sweep, L*Z):
-//       thread <-> output column, loop over k; a warp reads 32 consecutive doubles per k.
-//   F2  B(j,k) = B[j*b_sj + k]   consecutive k are contiguous (backward sweep: L' and gathered rows):
-//       warp <-> output column, lanes stride k; one shuffle reduction per column.
+//   F1  B(j,k) = B[j + k*b_sk]   consecutive OUTPUT columns j are contiguous (forward sweep, L*Z)
+//   F2  B(j,k) = B[j*b_sj + k]   consecutive k are contiguous (backward sweep: L' and gathered rows)
+// 5..32 right-hand sides run on the FP64 tensor pipe (the *_dmma kernels): NMT = row tiles of 8, M <= 8 NMT, NMT in
+// {1, 2, 4}; rows past M are zero-padded in shared memory.
 #pragma once
 #include "dense_tiles.cuh"
 
 namespace slmm {
 
-constexpr int SK_F1_COLS = 128;    // output columns per CTA, flavour 1 (= threads)
-constexpr int SK_F1_KC = 256;      // k chunk staged in shared memory per pass
+constexpr int SK_F1_COLS = 128;    // output columns per CTA, flavour 1
+constexpr int SK_F1_KC = 256;      // register-blocked F1: k chunk staged in shared memory per pass
 constexpr int SK_F2_COLS = 64;     // output columns per CTA, flavour 2 (8 warps x 8 columns)
-constexpr int SK_F2_KMAX = 512;    // an F2 work item holds its whole K range of A in shared memory
+constexpr int SK_F2_KMAX = 512;    // a register-blocked F2 work item holds its whole K range of A in shared memory
 
+// 1..4 right-hand sides, register-blocked: the MT accumulators of one output column in registers, the small operand in
+// shared memory, L streamed with many independent coalesced loads per thread.
+//   F1: thread <-> output column, loop over k; a warp reads 32 consecutive doubles per k.
+//   F2: warp <-> output column, lanes stride k; one shuffle reduction per column.
 template <int MT>
 __global__ void __launch_bounds__(SK_F1_COLS) skinny_f1_kernel(const GemmOp* __restrict__ ops,
                                                                const int32_t* __restrict__ tile_op) {
@@ -197,22 +202,22 @@ __global__ void __launch_bounds__(256, 2) skinny_f2_kernel(const GemmOp* __restr
   }
 }
 
-// Backward-sweep flavour on the FP64 tensor pipe, for 5..16 right-hand sides.  Same tiling and operand staging as
-// skinny_f2_kernel (64 output columns per CTA; A is staged in shared memory chunk by chunk along K, so K is not
-// limited), but the products run as DMMA
-// m8n8k4: a warp owns 8 output columns, its B fragment b[k = t][n = g] = B(j0 + g, kk + t) comes STRAIGHT from global
-// memory (each lane 8 bytes, a quad 32 contiguous bytes of one column of L: whole sectors, 256 bytes per warp load
-// like a coalesced load), the A fragments from shared memory (leading dimension = 4 mod 16: conflict free).  The
-// register-blocked kernel reads 12..16 shared-memory values per pair of streamed values and is bound by that; here it
-// is 2 per streamed value and the FMA work leaves the FP64 pipe.  NMT = row tiles of 8 (M <= 8 NMT; 1, 2, 4, 8).
 template <int NMT> struct SkDmma {
   // k chunk of the staged operand: the copy of A (8 NMT rows) must leave room for 2-3 resident CTAs per SM
-  static constexpr int KC = NMT <= 2 ? 512 : (NMT == 4 ? 256 : 128);
+  static constexpr int KC = NMT <= 2 ? 512 : 256;    // F2
   static constexpr int KP = KC + 4;                  // leading dimension = 4 mod 16: conflict-free fragment reads
   static constexpr int SMEM = 8 * NMT * KP * (int)sizeof(double);
+  static constexpr int F1_KC = 256, F1_KP = F1_KC + 4;
+  static constexpr int F1_SMEM = 8 * NMT * F1_KP * (int)sizeof(double);
   static constexpr int OCC = NMT <= 2 ? 3 : 2;
 };
 
+// Backward-sweep flavour on the tensor pipe (A staged chunk by chunk along K, so unlike skinny_f2_kernel K is not
+// limited): a warp owns 8 output columns, its B fragment b[k = t][n = g] = B(j0 + g, kk + t) comes
+// STRAIGHT from global memory (each lane 8 bytes, a quad 32 contiguous bytes of one column of L: whole sectors, 256
+// bytes per warp load like a coalesced load), the A fragments from shared memory (leading dimension = 4 mod 16:
+// conflict free).  The register-blocked kernel would read 12..16 shared-memory values per pair of streamed values at
+// these widths and be bound by that; here it is 2 per streamed value.
 template <int NMT>
 __global__ void __launch_bounds__(256, SkDmma<NMT>::OCC) skinny_f2_dmma_kernel(const GemmOp* __restrict__ ops,
                                                                               const int32_t* __restrict__ tile_op) {
@@ -294,17 +299,15 @@ __global__ void __launch_bounds__(256, SkDmma<NMT>::OCC) skinny_f2_dmma_kernel(c
   }
 }
 
-// Forward flavour on the FP64 tensor pipe (5..16 right-hand sides): B(j, k) = B[j + k*b_sk], a warp owns 16 output
-// columns (two 8-column DMMA tiles); its B fragment b[k = t][n = g] = B(jb + g, kk + t) comes straight from global
-// memory - for a fixed k the 8 lanes of a g-group read 64 contiguous bytes, the 8 warps of a CTA 1 KB of that k-row.
-// A(M x K) is staged in K chunks of 256 (128 for 64 rows) as [i][chunk + 4] (leading dimension = 4 mod 16:
-// conflict-free fragment reads).
-// Same op lists, tiling (128 columns per CTA) and split-K parts as skinny_f1_kernel.
+// Forward flavour: a warp owns 16 output columns (two 8-column DMMA tiles); its B fragment b[k = t][n = g] =
+// B(jb + g, kk + t) comes straight from global memory - for a fixed k the 8 lanes of a g-group read 64 contiguous
+// bytes, the 8 warps of a CTA 1 KB of that k-row.  A(M x K) is staged in K chunks of F1_KC as [i][F1_KP]
+// (leading dimension = 4 mod 16: conflict-free fragment reads).
 
 template <int NMT>
 __global__ void __launch_bounds__(256, SkDmma<NMT>::OCC) skinny_f1_dmma_kernel(const GemmOp* __restrict__ ops,
                                                                               const int32_t* __restrict__ tile_op) {
-  constexpr int SK_F1D_KC = NMT <= 4 ? 256 : 128, SK_F1D_KCP = SK_F1D_KC + 4;
+  constexpr int SK_F1D_KC = SkDmma<NMT>::F1_KC, SK_F1D_KCP = SkDmma<NMT>::F1_KP;
   extern __shared__ double As[];                       // [8 * NMT][SK_F1D_KCP]
   const int tile = blockIdx.x;
   const GemmOp& op = ops[tile_op[tile]];

@@ -1192,29 +1192,16 @@ int slmm_matset_is_symmetric(slmm_matset_t* ms, int32_t k, int32_t* out) {
   if (c.symmetric < 0) {
     // one streaming pass: hash sums of the entries above / below the diagonal (the test the row-block shards use; a
     // mismatch survives with probability ~2^-64).  The exact kernel (a binary search per entry: 9 ms per matrix at
-    // 1M individuals, a quarter of HE()'s device-side time) stays behind SLMM_EXACT_SYMMETRY=1 and in
-    // slmm_device_csr_is_symmetric.
-    static const bool exact = getenv("SLMM_EXACT_SYMMETRY") && getenv("SLMM_EXACT_SYMMETRY")[0] == '1';
-    if (exact) {
-      int* d_flag = dev_alloc<int>(1);
-      CUDA_OK(cudaMemsetAsync(d_flag, 0, sizeof(int), 0));
-      symmetry_check_kernel<<<he_grid(ms->n), 256>>>(c.indptr, c.indices, c.data, ms->n, d_flag);
-      g_launch_count++;
-      int flag = 1;
-      CUDA_OK(cudaMemcpy(&flag, d_flag, sizeof(int), cudaMemcpyDeviceToHost));
-      dev_free(d_flag);
-      c.symmetric = flag ? 0 : 1;
-    } else {
-      unsigned long long* d = dev_alloc<unsigned long long>(2);
-      CUDA_OK(cudaMemsetAsync(d, 0, 2 * sizeof(unsigned long long), 0));
-      symmetry_hash_kernel<<<he_grid(ms->n), 256>>>(c.indptr, c.indices, c.data, 0, ms->n, d);
-      g_launch_count++;
-      unsigned long long h2[2] = {0, 1};
-      const cudaError_t e = cudaMemcpy(h2, d, sizeof(h2), cudaMemcpyDeviceToHost);
-      dev_free(d);
-      CUDA_OK(e);
-      c.symmetric = h2[0] == h2[1] ? 1 : 0;
-    }
+    // 1M individuals, a quarter of HE()'s device-side time) is slmm_device_csr_is_symmetric.
+    unsigned long long* d = dev_alloc<unsigned long long>(2);
+    CUDA_OK(cudaMemsetAsync(d, 0, 2 * sizeof(unsigned long long), 0));
+    symmetry_hash_kernel<<<he_grid(ms->n), 256>>>(c.indptr, c.indices, c.data, 0, ms->n, d);
+    g_launch_count++;
+    unsigned long long h2[2] = {0, 1};
+    const cudaError_t e = cudaMemcpy(h2, d, sizeof(h2), cudaMemcpyDeviceToHost);
+    dev_free(d);
+    CUDA_OK(e);
+    c.symmetric = h2[0] == h2[1] ? 1 : 0;
   }
   *out = c.symmetric;
   return SLMM_OK;

@@ -520,10 +520,10 @@ def test_device_ibd_builder_known_answers_and_errors():
 
 # ------------------------------------------------------------------------------------------ narrow-RHS kernels
 def test_narrow_rhs_streaming_kernels(slmm, eng):
-    """nrhs <= 64 takes the HBM-streaming kernels (csrc/skinny_ops.cuh): every row template (1, 2, 4 register-blocked;
-    8, 16, 32, 64 rows on the tensor pipe),
-    both flavours, split-K with the triangular bound (L*Z of a 2,500-column front), gathered rows with K > 512
-    (700 coupled rows below the dense front), against LAPACK and bit-reproducible."""
+    """nrhs <= 32 takes the HBM-streaming kernels (csrc/skinny_ops.cuh): every row template (1, 2, 4 register-blocked;
+    8, 16, 32 rows on the tensor pipe; each at its top edge and inside it), both flavours, split-K with the triangular
+    bound (L*Z of a 2,500-column front), gathered rows with K > 512 (700 coupled rows below the dense front); 33, 48
+    and 64 columns take the DMMA tile path.  Against LAPACK and bit-reproducible."""
     rng = np.random.default_rng(12)
     nd, nt, nc = 2500, 900, 700
     B = rng.standard_normal((nd, nd))
@@ -543,7 +543,7 @@ def test_narrow_rhs_streaming_kernels(slmm, eng):
         f = slmm.SparseCholesky(ordering_method=ordering)(Vs)
         P = f.P()
         Lref = la.cholesky(V[P][:, P], lower=True)
-        for k in (1, 2, 3, 5, 9, 12, 13, 16, 17, 24, 32, 33, 48, 64):
+        for k in (1, 2, 3, 4, 5, 8, 9, 12, 13, 16, 17, 24, 32, 33, 48, 64):
             Bm = rng.standard_normal((n, k)) if k > 1 else rng.standard_normal(n)
             X1, X2 = f(Bm), f(Bm)
             assert np.array_equal(X1, X2)
@@ -638,8 +638,8 @@ def test_headline_size_250k_properties(slmm, eng):
     """BASELINE config 1 as simulated for the headline metric (250,000 individuals, K = 3, 10 covariates, wide
     fronts of several thousand columns): size-independent properties of the factor at FULL size - V x = b for every
     RHS-width class of the solve schedules (narrow streaming kernels, DMMA tiles), L*Z undone by the forward sweep,
-    bitwise repeatability of logdet and (LZ)' V^-1 (LZ) = Z'Z.  (scripts/solve_check.py runs the same residuals
-    with SLMM_TMA=0 / SLMM_SKINNY=0 twins.)"""
+    bitwise repeatability of logdet and (LZ)' V^-1 (LZ) = Z'Z.  (scripts/solve_check.py prints the same residuals
+    for a chosen size.)"""
     import torch, bench
     from scilmm_b200 import pedigree as P
     A, _, cov, y, info = bench.make_inputs(250000, 1e-3, 10)
@@ -698,14 +698,3 @@ def test_symmetry_detection_by_hash_sums(golden_c1mini, eng):
     D.data[up[0]], D.data[up[1]] = D.data[up[1]] + 0.25, D.data[up[0]] + 0.25
     ms = eng.MatSet([A, B, C_.tocsr(), D])
     assert ms.is_symmetric(0) and not ms.is_symmetric(1) and not ms.is_symmetric(2) and not ms.is_symmetric(3)
-
-
-def test_narrow_rhs_streaming_kernels_64_row_template():
-    """The 33..64-column streaming templates are off by default (slower than the tile path at 64 columns, see
-    chol.cu): the narrow-RHS test is repeated in a process that enables them (the switch is read once per process)."""
-    import os, subprocess, sys
-    env = dict(os.environ, SLMM_SKINNY_MAX="64")
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-q", "-m", "gpu", "-x", "-k",
-                        "test_narrow_rhs_streaming_kernels and not template"], env=env, capture_output=True, text=True,
-                       timeout=900)
-    assert r.returncode == 0 and "1 passed" in r.stdout, r.stdout[-3000:] + r.stderr[-2000:]
