@@ -302,36 +302,36 @@ struct Schedule {
   std::vector<PotrfOp> potrf;
   std::vector<PullItem> pull;
   std::vector<PullEntry> pull_entries;
-  PullEntry* d_pull_entries = nullptr;
+  DevPtr<PullEntry> d_pull_entries;
   std::vector<ReduceOp> reduce;
   std::vector<CUtensorMap> tmaps; // two per GEMM_TMA op (A, B), in op order
-  CUtensorMap* d_tmaps = nullptr;
+  DevPtr<CUtensorMap> d_tmaps;
   std::vector<int32_t> tile_op;   // per GEMM launch: op index (relative to the launch's first op) of every tile
-  int32_t* d_tile_op = nullptr;
+  DevPtr<int32_t> d_tile_op;
   int nevents = 0;                // events used by EV_RECORD / EV_WAIT
   int64_t ws_size = 0;            // doubles of split-K workspace (max over phases)
   int64_t ws2_size = 0;           // second workspace: split-K of bulk-stream ops running beside the chain's
-  double* d_ws = nullptr;
-  double* d_ws2 = nullptr;
-  ReduceOp* d_reduce = nullptr;
-  GemmOp* d_gemm = nullptr;
-  PotrfOp* d_potrf = nullptr;
-  PullItem* d_pull = nullptr;
+  DevPtr<double> d_ws;
+  DevPtr<double> d_ws2;
+  DevPtr<ReduceOp> d_reduce;
+  DevPtr<GemmOp> d_gemm;
+  DevPtr<PotrfOp> d_potrf;
+  DevPtr<PullItem> d_pull;
   double flops = 0;
   // CUDA graphs of this launch list (built lazily on first use; every kernel argument is fixed per schedule):
   // [0] the look-ahead variant on the priority + bulk stream pair, [1] the serial variant (one stream)
-  cudaGraphExec_t gexec[2] = {nullptr, nullptr};
+  GraphExec gexec[2];
   bool graph_failed = false;
   void upload() {
     if (ws_size > 0 || ws2_size > 0) {              // patch workspace offsets into pointers
       d_ws = dev_alloc<double>(ws_size);
       d_ws2 = dev_alloc<double>(ws2_size);
       for (GemmOp& op : gemm) {
-        if (op.flags & GF_WS) { op.C = d_ws + (int64_t)(intptr_t)op.C; op.flags &= ~GF_WS; }
-        if (op.flags & GF_WS2) { op.C = d_ws2 + (int64_t)(intptr_t)op.C; op.flags &= ~GF_WS2; }
+        if (op.flags & GF_WS) { op.C = d_ws.get() + (int64_t)(intptr_t)op.C; op.flags &= ~GF_WS; }
+        if (op.flags & GF_WS2) { op.C = d_ws2.get() + (int64_t)(intptr_t)op.C; op.flags &= ~GF_WS2; }
       }
       for (ReduceOp& r : reduce) {
-        r.ws = ((r.flags & GF_WS2) ? d_ws2 : d_ws) + (int64_t)(intptr_t)r.ws;
+        r.ws = ((r.flags & GF_WS2) ? d_ws2 : d_ws).get() + (int64_t)(intptr_t)r.ws;
         r.flags &= ~GF_WS2;
       }
     }
@@ -342,14 +342,6 @@ struct Schedule {
     d_tile_op = dev_upload(tile_op.data(), tile_op.size());
     d_tmaps = dev_upload(tmaps.data(), tmaps.size());
     d_pull_entries = dev_upload(pull_entries.data(), pull_entries.size());
-  }
-  void release() {
-    for (int q = 0; q < 2; q++) if (gexec[q]) { cudaGraphExecDestroy(gexec[q]); gexec[q] = nullptr; }
-    dev_free(d_gemm); dev_free(d_potrf); dev_free(d_pull); dev_free(d_ws); dev_free(d_ws2); dev_free(d_reduce); dev_free(d_tile_op); dev_free(d_pull_entries);
-    d_ws2 = nullptr;
-    dev_free(d_tmaps); d_tmaps = nullptr;
-    d_tile_op = nullptr; d_pull_entries = nullptr;
-    d_gemm = nullptr; d_potrf = nullptr; d_pull = nullptr; d_ws = nullptr; d_reduce = nullptr;
   }
   size_t device_bytes() const {
     return gemm.size() * sizeof(GemmOp) + potrf.size() * sizeof(PotrfOp) + pull.size() * sizeof(PullItem) +
@@ -579,18 +571,14 @@ static GemmOp make_op(double* C, int64_t c_si, int64_t c_sj, const double* A, in
 
 struct SolvePlan {
   int nrhs = 0;
-  double *X = nullptr, *X2 = nullptr;
-  double* arena[2] = {nullptr, nullptr};
-  int64_t* d_vptr = nullptr;
+  DevPtr<double> X, X2;
+  DevPtr<double> arena[2];
+  DevPtr<int64_t> d_vptr;
   Schedule fwd, bwd, lmul;
   size_t bytes = 0;
-  void release() {
-    dev_free(X); dev_free(X2); dev_free(arena[0]); dev_free(arena[1]); dev_free(d_vptr);
-    fwd.release(); bwd.release(); lmul.release();
-  }
 };
 
-struct EntryMap { int64_t* d_map = nullptr; int64_t nnz = 0; };
+struct EntryMap { DevPtr<int64_t> d_map; int64_t nnz = 0; };
 
 }  // namespace slmm
 
@@ -599,36 +587,35 @@ using namespace slmm;
 struct slmm_chol {
   Symbolic S;
   // device copies of the symbolic structure
-  int32_t *d_sn_first = nullptr, *d_sn_nrow = nullptr, *d_rows = nullptr, *d_rel = nullptr, *d_child_ptr = nullptr,
-          *d_child_idx = nullptr, *d_col2sn = nullptr, *d_perm = nullptr, *d_iperm = nullptr;
-  int64_t *d_sn_rowptr = nullptr, *d_sn_lptr = nullptr, *d_sn_uptr = nullptr;
+  DevPtr<int32_t> d_sn_first, d_sn_nrow, d_rows, d_rel, d_child_ptr, d_child_idx, d_col2sn, d_perm, d_iperm;
+  DevPtr<int64_t> d_sn_rowptr, d_sn_lptr, d_sn_uptr;
   std::vector<int64_t> uptr, invptr;
   std::vector<int64_t> wptr;          // [nsuper+1] offsets of the wide inverse blocks of each supernode
   std::vector<WBlock> wblocks;
-  WBlock* d_wblocks = nullptr;
-  double* Lx = nullptr;
-  double* inv = nullptr;
-  double* W = nullptr;                // inverses of the NBO-wide diagonal blocks (supernodes wider than NBI)
-  double* wscratch = nullptr;         // wide fronts: products of one recursive-doubling level
+  DevPtr<WBlock> d_wblocks;
+  DevPtr<double> Lx;
+  DevPtr<double> inv;
+  DevPtr<double> W;                   // inverses of the NBO-wide diagonal blocks (supernodes wider than NBI)
+  DevPtr<double> wscratch;            // wide fronts: products of one recursive-doubling level
   std::vector<int64_t> wscratch_off;
-  double* arena[2] = {nullptr, nullptr};
+  DevPtr<double> arena[2];
   int64_t arena_size[2] = {0, 0};
-  int* d_info = nullptr;
-  double* d_partial = nullptr;
+  DevPtr<int> d_info;
+  DevPtr<double> d_partial;
   Schedule fact;
   std::vector<EntryMap> maps;
   std::map<int, std::unique_ptr<SolvePlan>> plans;
-  cudaStream_t s_main = nullptr, s_bulk = nullptr;   // factorization streams (main: highest priority)
-  cudaStream_t s_aux = nullptr;        // auxiliary stream: a second solve running beside the one on stream 0
+  Stream s_main, s_bulk;              // factorization streams (main: highest priority)
+  Stream s_aux;                        // auxiliary stream: a second solve running beside the one on stream 0
   cudaStream_t cur = nullptr;          // stream the single-stream schedules (solves, L*Z) are issued on (0 or s_aux)
-  cudaEvent_t ev_aux = nullptr;
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-  std::vector<cudaEvent_t> events;
+  Event ev_aux;
+  Event ev_fork, ev_join;
+  std::vector<Event> events;
   bool factored = false;
   bool profiling = false;
   bool timeline = false;               // events of the two-stream schedules carry timestamps (eager issue, no graphs)
-  std::vector<cudaEvent_t> tl_events;  // timed twins of `events` + [0] = fork
-  std::vector<cudaEvent_t> tl_launch;  // one timed event after every kernel of the schedule
+  std::vector<Event> tl_events;        // timed twins of `events` + [0] = fork
+  std::vector<Event> tl_launch;        // one timed event after every kernel of the schedule
   int tl_count = 0;
   double prof_ms[16] = {};
   double prof_flops[16] = {};
@@ -639,8 +626,13 @@ struct slmm_chol {
   size_t bytes = 0;
   int64_t exported_nnz = 0;
 
+  // the graph execs, streams and events are destroyed only after the work queued on them has finished (errors
+  // are ignored: teardown also runs at interpreter shutdown)
+  ~slmm_chol() { cudaDeviceSynchronize(); }
+
   DevSym devsym() const {
-    return DevSym{d_sn_first, d_sn_nrow, d_rows, d_rel, d_child_ptr, d_child_idx, d_sn_rowptr, d_sn_lptr, d_sn_uptr};
+    return DevSym{d_sn_first.get(), d_sn_nrow.get(), d_rows.get(), d_rel.get(), d_child_ptr.get(), d_child_idx.get(),
+                  d_sn_rowptr.get(), d_sn_lptr.get(), d_sn_uptr.get()};
   }
 };
 
@@ -662,39 +654,40 @@ static void init_kernel_attributes() {
 }
 
 static void launch_one(slmm_chol* h, const Schedule& sch, const Launch& L, const DevSym& ds, double* X,
-                       double* const* vec_arena, const int64_t* d_vptr, int nrhs, cudaStream_t st) {
+                       const DevPtr<double>* vec_arena, const int64_t* d_vptr, int nrhs, cudaStream_t st) {
   switch (L.kind) {
     case Launch::POTRF:
-      potrf_inv_kernel_v4<<<L.grid, 256, POTRF4_SMEM, st>>>(sch.d_potrf + L.off, h->d_info);
+      potrf_inv_kernel_v4<<<L.grid, 256, POTRF4_SMEM, st>>>(sch.d_potrf.get() + L.off, h->d_info.get());
       break;
     case Launch::GEMM_BIG:
-      gemm_tiles_kernel<128, 128, 2, 4, BIG_STAGES><<<L.grid, BIG_THREADS, BIG_SMEM, st>>>(sch.d_gemm + L.off, sch.d_tile_op + L.tile_off);
+      gemm_tiles_kernel<128, 128, 2, 4, BIG_STAGES><<<L.grid, BIG_THREADS, BIG_SMEM, st>>>(sch.d_gemm.get() + L.off, sch.d_tile_op.get() + L.tile_off);
       break;
     case Launch::GEMM_TMA:
-      gemm_tiles_tma_kernel<<<L.grid, TMA_THREADS, TMA_SMEM, st>>>(sch.d_gemm + L.off, sch.d_tile_op + L.tile_off, sch.d_tmaps + L.aux_off);
+      gemm_tiles_tma_kernel<<<L.grid, TMA_THREADS, TMA_SMEM, st>>>(sch.d_gemm.get() + L.off, sch.d_tile_op.get() + L.tile_off, sch.d_tmaps.get() + L.aux_off);
       break;
     case Launch::GEMM_SMALL:
-      gemm_tiles_kernel<64, 64, 2, 2, SMALL_STAGES><<<L.grid, SMALL_THREADS, SMALL_SMEM, st>>>(sch.d_gemm + L.off, sch.d_tile_op + L.tile_off);
+      gemm_tiles_kernel<64, 64, 2, 2, SMALL_STAGES><<<L.grid, SMALL_THREADS, SMALL_SMEM, st>>>(sch.d_gemm.get() + L.off, sch.d_tile_op.get() + L.tile_off);
       break;
     case Launch::PULL_MAT:
-      extend_add_kernel<32><<<(L.count + 3) / 4, 128, 0, st>>>(sch.d_pull + L.off, L.count, sch.d_pull_entries, ds, h->Lx,
-                                                               h->arena[L.child_parity], h->arena[L.child_parity ^ 1]);
+      extend_add_kernel<32><<<(L.count + 3) / 4, 128, 0, st>>>(sch.d_pull.get() + L.off, L.count, sch.d_pull_entries.get(), ds, h->Lx.get(),
+                                                               h->arena[L.child_parity].get(), h->arena[L.child_parity ^ 1].get());
       break;
     case Launch::PULL_MAT_BIG:
-      extend_add_kernel<256><<<L.count, 256, 0, st>>>(sch.d_pull + L.off, L.count, sch.d_pull_entries, ds, h->Lx,
-                                                      h->arena[L.child_parity], h->arena[L.child_parity ^ 1]);
+      extend_add_kernel<256><<<L.count, 256, 0, st>>>(sch.d_pull.get() + L.off, L.count, sch.d_pull_entries.get(), ds, h->Lx.get(),
+                                                      h->arena[L.child_parity].get(), h->arena[L.child_parity ^ 1].get());
       break;
     case Launch::PULL_VEC:
-      vec_pull_kernel<<<(L.count + 3) / 4, 128, 0, st>>>(sch.d_pull + L.off, L.count, sch.d_pull_entries, ds, X,
-                                                         vec_arena[L.child_parity], vec_arena[L.child_parity ^ 1], d_vptr, nrhs);
+      vec_pull_kernel<<<(L.count + 3) / 4, 128, 0, st>>>(sch.d_pull.get() + L.off, L.count, sch.d_pull_entries.get(), ds, X,
+                                                         vec_arena[L.child_parity].get(),
+                                                         vec_arena[L.child_parity ^ 1].get(), d_vptr, nrhs);
       break;
     case Launch::REDUCE:
-      splitk_reduce_kernel<<<L.grid, 256, 0, st>>>(sch.d_reduce + L.off, L.count);
+      splitk_reduce_kernel<<<L.grid, 256, 0, st>>>(sch.d_reduce.get() + L.off, L.count);
       break;
     case Launch::SKINNY_F1:
     case Launch::SKINNY_F2: {
-      const GemmOp* ops = sch.d_gemm + L.off;
-      const int32_t* top = sch.d_tile_op + L.tile_off;
+      const GemmOp* ops = sch.d_gemm.get() + L.off;
+      const int32_t* top = sch.d_tile_op.get() + L.tile_off;
       const bool f1 = L.kind == Launch::SKINNY_F1;
 #define SKD_CASE(NMT)                                                                          \
   if (f1) skinny_f1_dmma_kernel<NMT><<<L.grid, 256, SkDmma<NMT>::F1_SMEM, st>>>(ops, top);  \
@@ -715,7 +708,7 @@ static void launch_one(slmm_chol* h, const Schedule& sch, const Launch& L, const
       break;
     }
     case Launch::INIT_W:
-      init_identity_kernel<<<L.count, 256, 0, st>>>(h->d_wblocks, h->W);
+      init_identity_kernel<<<L.count, 256, 0, st>>>(h->d_wblocks.get(), h->W.get());
       break;
     default:
       break;
@@ -734,19 +727,19 @@ static bool is_kernel(const Launch& L) { return L.kind != Launch::EV_RECORD && L
 // The lists are static (every kernel argument is fixed once the schedule is uploaded), so each one is captured
 // ONCE into a CUDA graph and replayed: a 12-column solve is a chain of ~1000 tiny launches whose cost was the
 // host's launch rate, not the kernels.
-static void issue_schedule(slmm_chol* h, const Schedule& sch, double* X, double* const* vec_arena,
+static void issue_schedule(slmm_chol* h, const Schedule& sch, double* X, const DevPtr<double>* vec_arena,
                            const int64_t* d_vptr, int nrhs, bool two, cudaStream_t one,
-                           std::vector<cudaEvent_t>* per_launch = nullptr) {
+                           std::vector<Event>* per_launch = nullptr) {
   const DevSym ds = h->devsym();
   size_t nk = 0;
   for (const Launch& L : sch.launches) {
-    cudaStream_t st = two ? (L.stream ? h->s_bulk : h->s_main) : one;
-    if (L.kind == Launch::EV_RECORD) { if (two) CUDA_OK(cudaEventRecord(h->events[L.count], st)); continue; }
-    if (L.kind == Launch::EV_WAIT) { if (two) CUDA_OK(cudaStreamWaitEvent(st, h->events[L.count], 0)); continue; }
+    cudaStream_t st = two ? (L.stream ? h->s_bulk.get() : h->s_main.get()) : one;
+    if (L.kind == Launch::EV_RECORD) { if (two) CUDA_OK(cudaEventRecord(h->events[L.count].get(), st)); continue; }
+    if (L.kind == Launch::EV_WAIT) { if (two) CUDA_OK(cudaStreamWaitEvent(st, h->events[L.count].get(), 0)); continue; }
     launch_one(h, sch, L, ds, X, vec_arena, d_vptr, nrhs, st);
     if (per_launch) {                       // timeline mode: when did this launch finish (on its own stream)?
-      if (nk >= per_launch->size()) { cudaEvent_t e; CUDA_OK(cudaEventCreate(&e)); per_launch->push_back(e); }
-      CUDA_OK(cudaEventRecord((*per_launch)[nk], st));
+      if (nk >= per_launch->size()) per_launch->push_back(make_event(cudaEventDefault));
+      CUDA_OK(cudaEventRecord((*per_launch)[nk].get(), st));
     }
     nk++;
   }
@@ -754,21 +747,21 @@ static void issue_schedule(slmm_chol* h, const Schedule& sch, double* X, double*
 
 // Captures the launch list into a graph.  Capture happens on the (non-blocking) priority stream - the legacy
 // default stream cannot be captured; the bulk stream joins the capture through the fork event.
-static cudaGraphExec_t capture_schedule(slmm_chol* h, const Schedule& sch, double* X, double* const* vec_arena,
+static GraphExec capture_schedule(slmm_chol* h, const Schedule& sch, double* X, const DevPtr<double>* vec_arena,
                                         const int64_t* d_vptr, int nrhs, bool two) {
-  cudaStream_t origin = h->s_main;
+  cudaStream_t origin = h->s_main.get();
   cudaGraph_t graph = nullptr;
   cudaGraphExec_t exec = nullptr;
   CUDA_OK(cudaStreamBeginCapture(origin, cudaStreamCaptureModeRelaxed));
   try {
     if (two) {
-      CUDA_OK(cudaEventRecord(h->ev_fork, origin));
-      CUDA_OK(cudaStreamWaitEvent(h->s_bulk, h->ev_fork, 0));
+      CUDA_OK(cudaEventRecord(h->ev_fork.get(), origin));
+      CUDA_OK(cudaStreamWaitEvent(h->s_bulk.get(), h->ev_fork.get(), 0));
     }
     issue_schedule(h, sch, X, vec_arena, d_vptr, nrhs, two, origin);
     if (two) {
-      CUDA_OK(cudaEventRecord(h->ev_join, h->s_bulk));
-      CUDA_OK(cudaStreamWaitEvent(origin, h->ev_join, 0));
+      CUDA_OK(cudaEventRecord(h->ev_join.get(), h->s_bulk.get()));
+      CUDA_OK(cudaStreamWaitEvent(origin, h->ev_join.get(), 0));
     }
     CUDA_OK(cudaGetLastError());
   } catch (...) {
@@ -781,10 +774,10 @@ static cudaGraphExec_t capture_schedule(slmm_chol* h, const Schedule& sch, doubl
   const cudaError_t e = cudaGraphInstantiate(&exec, graph, 0);
   cudaGraphDestroy(graph);
   CUDA_OK(e);
-  return exec;
+  return GraphExec(exec);
 }
 
-static void run_schedule(slmm_chol* h, Schedule& sch, double* X, double* const* vec_arena, const int64_t* d_vptr,
+static void run_schedule(slmm_chol* h, Schedule& sch, double* X, const DevPtr<double>* vec_arena, const int64_t* d_vptr,
                          int nrhs) {
   int64_t nk = 0;
   for (const Launch& L : sch.launches) nk += is_kernel(L) ? 1 : 0;
@@ -793,32 +786,23 @@ static void run_schedule(slmm_chol* h, Schedule& sch, double* X, double* const* 
     // schedules with events run on the priority + bulk stream pair; inside an auxiliary section (cur != 0) the
     // pair may already be in use by the solve on stream 0, so the list is walked serially (a valid order)
     const bool two = sch.nevents > 0 && h->s_main != nullptr && h->cur == nullptr;
-    while ((int)h->events.size() < sch.nevents) {
-      cudaEvent_t e;
-      CUDA_OK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      h->events.push_back(e);
-    }
+    while ((int)h->events.size() < sch.nevents) h->events.push_back(make_event(cudaEventDisableTiming));
     const int gi = two ? 0 : 1;
     if (h->timeline && two) {
       // timeline mode: the same two-stream issue with TIMED events, so the host can read when each panel / bulk
       // update finished relative to the fork (where is the critical path: the chain or the bulk stream?)
-      while ((int)h->tl_events.size() < sch.nevents + 2) {
-        cudaEvent_t e;
-        CUDA_OK(cudaEventCreate(&e));
-        h->tl_events.push_back(e);
-      }
-      std::vector<cudaEvent_t> saved = h->events;
-      for (int q = 0; q < sch.nevents; q++) h->events[q] = h->tl_events[q + 2];
-      CUDA_OK(cudaEventRecord(h->tl_events[0], 0));
-      CUDA_OK(cudaStreamWaitEvent(h->s_main, h->tl_events[0], 0));
-      CUDA_OK(cudaStreamWaitEvent(h->s_bulk, h->tl_events[0], 0));
+      while ((int)h->tl_events.size() < sch.nevents + 2) h->tl_events.push_back(make_event(cudaEventDefault));
+      for (int q = 0; q < sch.nevents; q++) std::swap(h->events[q], h->tl_events[q + 2]);
+      CUDA_OK(cudaEventRecord(h->tl_events[0].get(), 0));
+      CUDA_OK(cudaStreamWaitEvent(h->s_main.get(), h->tl_events[0].get(), 0));
+      CUDA_OK(cudaStreamWaitEvent(h->s_bulk.get(), h->tl_events[0].get(), 0));
       issue_schedule(h, sch, X, vec_arena, d_vptr, nrhs, true, nullptr, &h->tl_launch);
-      CUDA_OK(cudaEventRecord(h->ev_join, h->s_bulk));
-      CUDA_OK(cudaStreamWaitEvent(h->s_main, h->ev_join, 0));
-      CUDA_OK(cudaEventRecord(h->tl_events[1], h->s_main));
-      CUDA_OK(cudaStreamWaitEvent(0, h->tl_events[1], 0));
-      CUDA_OK(cudaEventSynchronize(h->tl_events[1]));
-      h->events = saved;
+      CUDA_OK(cudaEventRecord(h->ev_join.get(), h->s_bulk.get()));
+      CUDA_OK(cudaStreamWaitEvent(h->s_main.get(), h->ev_join.get(), 0));
+      CUDA_OK(cudaEventRecord(h->tl_events[1].get(), h->s_main.get()));
+      CUDA_OK(cudaStreamWaitEvent(0, h->tl_events[1].get(), 0));
+      CUDA_OK(cudaEventSynchronize(h->tl_events[1].get()));
+      for (int q = 0; q < sch.nevents; q++) std::swap(h->events[q], h->tl_events[q + 2]);
       h->tl_count = sch.nevents + 2;
       g_launch_count += nk;
       return;
@@ -831,26 +815,25 @@ static void run_schedule(slmm_chol* h, Schedule& sch, double* X, double* const* 
         sch.gexec[gi] = capture_schedule(h, sch, X, vec_arena, d_vptr, nrhs, two);
       } catch (const std::exception&) {
         sch.graph_failed = true;      // fall back to launch-by-launch for this schedule
-        sch.gexec[gi] = nullptr;
       }
     }
-    cudaGraphExec_t exec = (use_graph && !sch.graph_failed) ? sch.gexec[gi] : nullptr;
+    cudaGraphExec_t exec = (use_graph && !sch.graph_failed) ? sch.gexec[gi].get() : nullptr;
     if (exec != nullptr && h->cur != nullptr) {
       CUDA_OK(cudaGraphLaunch(exec, h->cur));              // auxiliary section: the whole list on the auxiliary stream
     } else if (exec != nullptr || two) {
       // fork from / join to the legacy default stream around the priority stream (and, inside, the bulk stream)
-      CUDA_OK(cudaEventRecord(h->ev_fork, 0));
-      CUDA_OK(cudaStreamWaitEvent(h->s_main, h->ev_fork, 0));
+      CUDA_OK(cudaEventRecord(h->ev_fork.get(), 0));
+      CUDA_OK(cudaStreamWaitEvent(h->s_main.get(), h->ev_fork.get(), 0));
       if (exec != nullptr) {
-        CUDA_OK(cudaGraphLaunch(exec, h->s_main));
+        CUDA_OK(cudaGraphLaunch(exec, h->s_main.get()));
       } else {
-        CUDA_OK(cudaStreamWaitEvent(h->s_bulk, h->ev_fork, 0));
+        CUDA_OK(cudaStreamWaitEvent(h->s_bulk.get(), h->ev_fork.get(), 0));
         issue_schedule(h, sch, X, vec_arena, d_vptr, nrhs, true, nullptr);
-        CUDA_OK(cudaEventRecord(h->ev_join, h->s_bulk));
-        CUDA_OK(cudaStreamWaitEvent(h->s_main, h->ev_join, 0));
+        CUDA_OK(cudaEventRecord(h->ev_join.get(), h->s_bulk.get()));
+        CUDA_OK(cudaStreamWaitEvent(h->s_main.get(), h->ev_join.get(), 0));
       }
-      CUDA_OK(cudaEventRecord(h->ev_join, h->s_main));
-      CUDA_OK(cudaStreamWaitEvent(0, h->ev_join, 0));
+      CUDA_OK(cudaEventRecord(h->ev_join.get(), h->s_main.get()));
+      CUDA_OK(cudaStreamWaitEvent(0, h->ev_join.get(), 0));
     } else {
       issue_schedule(h, sch, X, vec_arena, d_vptr, nrhs, false, h->cur);
     }
@@ -861,17 +844,17 @@ static void run_schedule(slmm_chol* h, Schedule& sch, double* X, double* const* 
     std::vector<const Launch*> ks;
     for (const Launch& L : sch.launches) if (is_kernel(L)) ks.push_back(&L);
     const size_t nl = ks.size();
-    std::vector<cudaEvent_t> ev(nl + 1);
-    for (auto& e : ev) CUDA_OK(cudaEventCreate(&e));
-    CUDA_OK(cudaEventRecord(ev[0], st));
+    std::vector<Event> ev(nl + 1);
+    for (auto& e : ev) e = make_event(cudaEventDefault);
+    CUDA_OK(cudaEventRecord(ev[0].get(), st));
     for (size_t i = 0; i < nl; i++) {
       launch_one(h, sch, *ks[i], ds, X, vec_arena, d_vptr, nrhs, st);
-      CUDA_OK(cudaEventRecord(ev[i + 1], st));
+      CUDA_OK(cudaEventRecord(ev[i + 1].get(), st));
     }
-    CUDA_OK(cudaEventSynchronize(ev[nl]));
+    CUDA_OK(cudaEventSynchronize(ev[nl].get()));
     for (size_t i = 0; i < nl; i++) {
       float ms = 0;
-      CUDA_OK(cudaEventElapsedTime(&ms, ev[i], ev[i + 1]));
+      CUDA_OK(cudaEventElapsedTime(&ms, ev[i].get(), ev[i + 1].get()));
       const int k = (int)ks[i]->kind;
       h->prof_ms[k] += ms;
       h->prof_flops[k] += ks[i]->flops;
@@ -881,7 +864,6 @@ static void run_schedule(slmm_chol* h, Schedule& sch, double* X, double* const* 
       h->prof_launch_kind.push_back(k);
       h->prof_launch_grid.push_back((ks[i]->kind <= Launch::GEMM_SMALL || ks[i]->kind >= Launch::SKINNY_F1) ? ks[i]->grid : ks[i]->count);
     }
-    for (auto& e : ev) cudaEventDestroy(e);
   }
   g_launch_count += nk;
   CUDA_OK(cudaGetLastError());
@@ -951,12 +933,12 @@ static OuterBlock outer_block(const slmm_chol* h, int s, int ob) {
   b.o0 = ob * NBO;
   b.nbo = std::min(ns, b.o0 + NBO) - b.o0;
   if (b.nbo <= NBI) {
-    b.winv = h->inv + h->invptr[s] + (int64_t)(b.o0 / NBI) * NBI * NBI;
+    b.winv = h->inv.get() + h->invptr[s] + (int64_t)(b.o0 / NBI) * NBI * NBI;
     b.ldw = NBI;
   } else {
     int64_t off = h->wptr[s];
     for (int q = 0; q < ob; q++) off += (int64_t)NBO * NBO;      // every earlier block of s is a full one
-    b.winv = h->W + off;
+    b.winv = h->W.get() + off;
     b.ldw = b.nbo;
   }
   return b;
@@ -1026,13 +1008,13 @@ static void build_factor_schedule(slmm_chol* h) {
         const int s = S.level_sn[S.level_ptr[d] + q];
         const int f = S.sn_first[s], ns = S.sn_first[s + 1] - f, ms = S.sn_nrow[s], rs = ms - ns;
         const bool wide = ns > NBO;
-        double* P = h->Lx + S.sn_lptr[s];
+        double* P = h->Lx.get() + S.sn_lptr[s];
         const int64_t ld = panel_ld(ms);
         if (st.kind == FStep::POTRF || st.kind == FStep::TRSM || st.kind == FStep::UPD) {
           const int ib = st.a, c0 = ib * NBI, c1 = std::min(ns, c0 + NBI), nb = c1 - c0;
           const int ob = c0 / NBO, ob0 = ob * NBO, ob_end = std::min(ns, ob0 + NBO);
           // where the inverse of this 64 x 64 block lives: its private slot, or (wide fronts) the diagonal of W
-          double* inv = h->inv + h->invptr[s] + (int64_t)ib * NBI * NBI;
+          double* inv = h->inv.get() + h->invptr[s] + (int64_t)ib * NBI * NBI;
           int64_t inv_ld = NBI;
           if (wide) {
             const OuterBlock wb = outer_block(h, s, ob);
@@ -1054,7 +1036,7 @@ static void build_factor_schedule(slmm_chol* h) {
           // recursive doubling: inv([A 0; C B]) = [A^-1 0; -B^-1 (C A^-1)  B^-1], pairs of blocks of size m
           const OuterBlock wb = outer_block(h, s, st.a);
           const int m = st.b, o0 = wb.o0;
-          double* T = h->wscratch + h->wscratch_off[s];
+          double* T = h->wscratch.get() + h->wscratch_off[s];
           int pair = 0;
           for (int lo = 0; lo + m < wb.nbo; lo += 2 * m, pair++) {
             const int m2 = std::min(m, wb.nbo - lo - m);
@@ -1097,7 +1079,7 @@ static void build_factor_schedule(slmm_chol* h) {
             pb_rest.add(make_op(P + nx + nx * ld, 1, ld, P + nx + ob0 * ld, 1, ld, P + nx + ob0 * ld, 1, ld, ms - nx,
                                 ns - nx, c1 - ob0, GF_LOWER | GF_ACCUM | GF_NEG));
         } else {                      // SCHUR: panel done, U = -L21 L21'
-          double* U = h->arena[d & 1] + h->uptr[s];
+          double* U = h->arena[d & 1].get() + h->uptr[s];
           pb.add(make_op(U, 1, rs, P + ns, 1, ld, P + ns, 1, ld, rs, rs, ns, GF_LOWER | GF_NEG));
         }
       }
@@ -1150,13 +1132,13 @@ static void build_factor_schedule(slmm_chol* h) {
         for (int s2 = 0; s2 < S.nsuper; s2++) {
           const int ns = S.sn_first[s2 + 1] - S.sn_first[s2];
           if (ns <= NBI || ns > NBO) continue;
-          double* P = h->Lx + S.sn_lptr[s2];
+          double* P = h->Lx.get() + S.sn_lptr[s2];
           const int64_t ldp = panel_ld(S.sn_nrow[s2]);
           for (int ob = 0; ob < num_outer(ns); ob++) {
             const OuterBlock b = outer_block(h, s2, ob);
             if (b.nbo <= NBI || t * NBI >= b.nbo) continue;
             const int r0 = t * NBI, nbt = std::min(NBI, b.nbo - r0), ncols = std::min(b.nbo, r0 + NBI);
-            double* inv64 = h->inv + h->invptr[s2] + (int64_t)((b.o0 + r0) / NBI) * NBI * NBI;
+            double* inv64 = h->inv.get() + h->invptr[s2] + (int64_t)((b.o0 + r0) / NBI) * NBI * NBI;
             if (half == 0) {
               pb.add(make_op(b.winv + r0, 1, b.ldw, inv64, 1, NBI, b.winv + r0, b.ldw, 1, nbt, ncols, nbt, 0));
             } else if (r0 + nbt < b.nbo) {
@@ -1182,7 +1164,6 @@ static SolvePlan* get_plan(slmm_chol* h, int nrhs) {
   // keep a few widths resident (probe block, deterministic RHS, compute_hess stages)
   if (h->plans.size() >= 6) {
     CUDA_OK(cudaDeviceSynchronize());
-    for (auto& kv : h->plans) kv.second->release();
     h->plans.clear();
   }
   const Symbolic& S = h->S;
@@ -1254,13 +1235,13 @@ static SolvePlan* get_plan(slmm_chol* h, int nrhs) {
         const int s = S.level_sn[q];
         const int f = S.sn_first[s], ns = S.sn_first[s + 1] - f, ms = S.sn_nrow[s], rs = ms - ns;
         const int nob = num_outer(ns);
-        double* P = h->Lx + S.sn_lptr[s];
+        double* P = h->Lx.get() + S.sn_lptr[s];
         const int64_t ld = panel_ld(ms);
-        double* Xs = pl->X + (int64_t)f * R;
-        double* Ys = pl->X2 + (int64_t)f * R;
+        double* Xs = pl->X.get() + (int64_t)f * R;
+        double* Ys = pl->X2.get() + (int64_t)f * R;
         if (ph == 2 * nob) {                       // contribution block  u = -L21 y   (rs x nrhs)
           if (rs > 0)
-            pb.add(make_op(pl->arena[d & 1] + vptr[s], 1, R, Ys, 1, R, P + ns, 1, ld, nrhs, rs, ns, GF_NEG));
+            pb.add(make_op(pl->arena[d & 1].get() + vptr[s], 1, R, Ys, 1, R, P + ns, 1, ld, nrhs, rs, ns, GF_NEG));
           continue;
         }
         if (ph > 2 * nob) continue;
@@ -1301,14 +1282,14 @@ static SolvePlan* get_plan(slmm_chol* h, int nrhs) {
         const int s = S.level_sn[q];
         const int f = S.sn_first[s], ns = S.sn_first[s + 1] - f, ms = S.sn_nrow[s], rs = ms - ns;
         const int nob = num_outer(ns);
-        double* P = h->Lx + S.sn_lptr[s];
+        double* P = h->Lx.get() + S.sn_lptr[s];
         const int64_t ld = panel_ld(ms);
-        double* Xs = pl->X + (int64_t)f * R;
-        double* Ys = pl->X2 + (int64_t)f * R;
+        double* Xs = pl->X.get() + (int64_t)f * R;
+        double* Ys = pl->X2.get() + (int64_t)f * R;
         if (ph == 0) {                             // y_top -= L21' x[rows below]   (gathered rows of X)
           if (rs > 0)
-            pb.add(make_op(Ys, 1, R, pl->X, 1, R, P + ns, ld, 1, nrhs, ns, rs, GF_ACCUM | GF_NEG,
-                           h->d_rows + S.sn_rowptr[s] + ns));
+            pb.add(make_op(Ys, 1, R, pl->X.get(), 1, R, P + ns, ld, 1, nrhs, ns, rs, GF_ACCUM | GF_NEG,
+                           h->d_rows.get() + S.sn_rowptr[s] + ns));
           continue;
         }
         const int step = ph - 1, r = step / 2;     // outer blocks in reverse order
@@ -1338,12 +1319,12 @@ static SolvePlan* get_plan(slmm_chol* h, int nrhs) {
     for (int q = S.level_ptr[d]; q < S.level_ptr[d + 1]; q++) {
       const int s = S.level_sn[q];
       const int f = S.sn_first[s], ns = S.sn_first[s + 1] - f, ms = S.sn_nrow[s], rs = ms - ns;
-      double* P = h->Lx + S.sn_lptr[s];
+      double* P = h->Lx.get() + S.sn_lptr[s];
       const int64_t ld = panel_ld(ms);
       // out_top = L11 z_top (upper part of the diagonal block is stored as zeros)
-      pb.add(make_op(pl->X2 + (int64_t)f * R, 1, R, pl->X + (int64_t)f * R, 1, R, P, 1, ld, nrhs, ns, ns, GF_TRIL_B));
+      pb.add(make_op(pl->X2.get() + (int64_t)f * R, 1, R, pl->X.get() + (int64_t)f * R, 1, R, P, 1, ld, nrhs, ns, ns, GF_TRIL_B));
       if (rs > 0)
-        pb.add(make_op(pl->arena[d & 1] + vptr[s], 1, R, pl->X + (int64_t)f * R, 1, R, P + ns, 1, ld, nrhs, rs, ns, 0));
+        pb.add(make_op(pl->arena[d & 1].get() + vptr[s], 1, R, pl->X.get() + (int64_t)f * R, 1, R, P + ns, 1, ld, nrhs, rs, ns, 0));
     }
     pb.flush(pl->lmul);
     add_pull_items(pl->lmul, S, vptr, d, 2, Launch::PULL_VEC, 4);
@@ -1433,7 +1414,7 @@ int slmm_chol_analyze(int32_t n, const int32_t* indptr, const int32_t* indices, 
   h->Lx = dev_alloc<double>(S.lsize);
   h->inv = dev_alloc<double>(h->invptr[S.nsuper]);
   h->W = dev_alloc<double>(h->wptr[S.nsuper]);
-  CUDA_OK(cudaMemset(h->W, 0, std::max<int64_t>(1, h->wptr[S.nsuper]) * sizeof(double)));   // upper blocks of wide fronts' W stay zero
+  CUDA_OK(cudaMemset(h->W.get(), 0, std::max<int64_t>(1, h->wptr[S.nsuper]) * sizeof(double)));   // upper blocks of wide fronts' W stay zero
   h->wscratch = dev_alloc<double>(wscratch_total);
   h->d_wblocks = dev_upload(h->wblocks.data(), h->wblocks.size());
   h->arena[0] = dev_alloc<double>(h->arena_size[0]);
@@ -1443,14 +1424,19 @@ int slmm_chol_analyze(int32_t n, const int32_t* indptr, const int32_t* indices, 
   {
     int least = 0, greatest = 0;
     CUDA_OK(cudaDeviceGetStreamPriorityRange(&least, &greatest));
-    CUDA_OK(cudaStreamCreateWithPriority(&h->s_main, cudaStreamNonBlocking, greatest));
-    CUDA_OK(cudaStreamCreateWithPriority(&h->s_bulk, cudaStreamNonBlocking, least));
-    CUDA_OK(cudaStreamCreateWithPriority(&h->s_aux, cudaStreamNonBlocking, least));
-    CUDA_OK(cudaEventCreateWithFlags(&h->ev_aux, cudaEventDisableTiming));
-    CUDA_OK(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-    CUDA_OK(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
+    auto make_stream = [](int priority) {
+      cudaStream_t s = nullptr;
+      CUDA_OK(cudaStreamCreateWithPriority(&s, cudaStreamNonBlocking, priority));
+      return Stream(s);
+    };
+    h->s_main = make_stream(greatest);
+    h->s_bulk = make_stream(least);
+    h->s_aux = make_stream(least);
+    h->ev_aux = make_event(cudaEventDisableTiming);
+    h->ev_fork = make_event(cudaEventDisableTiming);
+    h->ev_join = make_event(cudaEventDisableTiming);
   }
-  CUDA_OK(cudaMemset(h->Lx, 0, S.lsize * sizeof(double)));
+  CUDA_OK(cudaMemset(h->Lx.get(), 0, S.lsize * sizeof(double)));
   build_factor_schedule(h.get());
   h->bytes = (S.lsize + h->invptr[S.nsuper] + h->wptr[S.nsuper] + h->arena_size[0] + h->arena_size[1]) * 8 +
              (S.rows.size() * 2 + S.sn_first.size() * 8) * 4 + h->fact.device_bytes();
@@ -1461,24 +1447,6 @@ int slmm_chol_analyze(int32_t n, const int32_t* indptr, const int32_t* indices, 
 }
 
 int slmm_chol_destroy(slmm_chol_t* h) {
-  if (!h) return SLMM_OK;
-  dev_free(h->d_sn_first); dev_free(h->d_sn_nrow); dev_free(h->d_rows); dev_free(h->d_rel);
-  dev_free(h->d_child_ptr); dev_free(h->d_child_idx); dev_free(h->d_col2sn); dev_free(h->d_perm); dev_free(h->d_iperm);
-  dev_free(h->d_sn_rowptr); dev_free(h->d_sn_lptr); dev_free(h->d_sn_uptr);
-  dev_free(h->Lx); dev_free(h->inv); dev_free(h->W); dev_free(h->wscratch); dev_free(h->d_wblocks); dev_free(h->arena[0]); dev_free(h->arena[1]);
-  dev_free(h->d_info); dev_free(h->d_partial);
-  for (cudaEvent_t e : h->events) cudaEventDestroy(e);
-  for (cudaEvent_t e : h->tl_events) cudaEventDestroy(e);
-  for (cudaEvent_t e : h->tl_launch) cudaEventDestroy(e);
-  if (h->ev_fork) cudaEventDestroy(h->ev_fork);
-  if (h->ev_join) cudaEventDestroy(h->ev_join);
-  if (h->s_main) cudaStreamDestroy(h->s_main);
-  if (h->s_bulk) cudaStreamDestroy(h->s_bulk);
-  if (h->s_aux) cudaStreamDestroy(h->s_aux);
-  if (h->ev_aux) cudaEventDestroy(h->ev_aux);
-  h->fact.release();
-  for (auto& m : h->maps) dev_free(m.d_map);
-  for (auto& kv : h->plans) kv.second->release();
   delete h;
   return SLMM_OK;
 }
@@ -1511,8 +1479,8 @@ int slmm_chol_perm(const slmm_chol_t* h, int32_t* perm) {
 
 int slmm_chol_device_perm(const slmm_chol_t* h, const int32_t** d_perm, const int32_t** d_iperm) {
   if (!h || !d_perm || !d_iperm) return SLMM_ERR_INVALID;
-  *d_perm = h->d_perm;
-  *d_iperm = h->d_iperm;
+  *d_perm = h->d_perm.get();
+  *d_iperm = h->d_iperm.get();
   return SLMM_OK;
 }
 
@@ -1527,7 +1495,7 @@ int slmm_chol_register_pattern_tri(slmm_chol_t* h, const int32_t* indptr, const 
   m.nnz = nnz;
   m.d_map = dev_upload(tgt.data(), tgt.size());
   CUDA_OK(cudaDeviceSynchronize());
-  h->maps.push_back(m);
+  h->maps.push_back(std::move(m));
   *map_id = (int32_t)h->maps.size() - 1;
   return SLMM_OK;
   SLMM_CATCH
@@ -1544,21 +1512,16 @@ int slmm_chol_register_pattern_device(slmm_chol_t* h, const int32_t* d_indptr, c
   EntryMap m;
   m.nnz = nnz;
   m.d_map = dev_alloc<int64_t>((size_t)nnz);
-  int* d_bad = dev_alloc<int>(1);
-  CUDA_OK(cudaMemsetAsync(d_bad, 0, sizeof(int), 0));
+  DevPtr<int> d_bad = dev_alloc<int>(1);
+  CUDA_OK(cudaMemsetAsync(d_bad.get(), 0, sizeof(int), 0));
   const int n = h->S.n;
-  entry_map_kernel<<<std::max(1, std::min(148 * 8, (n + 7) / 8)), 256>>>(d_indptr, d_indices, n, h->d_iperm, h->d_col2sn,
-                                                                       h->devsym(), tri, m.d_map, d_bad);
+  entry_map_kernel<<<std::max(1, std::min(148 * 8, (n + 7) / 8)), 256>>>(d_indptr, d_indices, n, h->d_iperm.get(), h->d_col2sn.get(),
+                                                                       h->devsym(), tri, m.d_map.get(), d_bad.get());
   g_launch_count++;
   int bad = 0;
-  const cudaError_t e = cudaMemcpy(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost);
-  dev_free(d_bad);
-  if (e != cudaSuccess || bad) {
-    dev_free(m.d_map);
-    CUDA_OK(e);
-    throw std::invalid_argument("matrix entry outside the analysed pattern");
-  }
-  h->maps.push_back(m);
+  CUDA_OK(cudaMemcpy(&bad, d_bad.get(), sizeof(int), cudaMemcpyDeviceToHost));
+  if (bad) throw std::invalid_argument("matrix entry outside the analysed pattern");
+  h->maps.push_back(std::move(m));
   *map_id = (int32_t)h->maps.size() - 1;
   return SLMM_OK;
   SLMM_CATCH
@@ -1567,11 +1530,11 @@ int slmm_chol_register_pattern_device(slmm_chol_t* h, const int32_t* d_indptr, c
 int slmm_chol_add_values(slmm_chol_t* h, int32_t map_id, const double* d_values, double sigma, int32_t first) {
   SLMM_TRY
   if (!h || map_id < 0 || map_id >= (int)h->maps.size()) throw std::invalid_argument("bad map id");
-  if (first) CUDA_OK(cudaMemsetAsync(h->Lx, 0, h->S.lsize * sizeof(double), 0));
+  if (first) CUDA_OK(cudaMemsetAsync(h->Lx.get(), 0, h->S.lsize * sizeof(double), 0));
   const EntryMap& m = h->maps[map_id];
   if (m.nnz > 0) {
     const int grid = (int)std::min<int64_t>((m.nnz + 255) / 256, 148 * 16);
-    scatter_axpy_kernel<<<grid, 256>>>(m.d_map, d_values, sigma, h->Lx, m.nnz);
+    scatter_axpy_kernel<<<grid, 256>>>(m.d_map.get(), d_values, sigma, h->Lx.get(), m.nnz);
     g_launch_count++;
   }
   CUDA_OK(cudaGetLastError());
@@ -1584,11 +1547,11 @@ int slmm_chol_add_values2(slmm_chol_t* h, int32_t map_id, const double* d_values
                           const double* d_values1, double sigma1, int32_t first) {
   SLMM_TRY
   if (!h || map_id < 0 || map_id >= (int)h->maps.size() || !d_values0 || !d_values1) throw std::invalid_argument("bad arguments");
-  if (first) CUDA_OK(cudaMemsetAsync(h->Lx, 0, h->S.lsize * sizeof(double), 0));
+  if (first) CUDA_OK(cudaMemsetAsync(h->Lx.get(), 0, h->S.lsize * sizeof(double), 0));
   const EntryMap& m = h->maps[map_id];
   if (m.nnz > 0) {
     const int grid = (int)std::min<int64_t>((m.nnz + 255) / 256, 148 * 16);
-    scatter_axpy2_kernel<<<grid, 256>>>(m.d_map, d_values0, sigma0, d_values1, sigma1, h->Lx, m.nnz);
+    scatter_axpy2_kernel<<<grid, 256>>>(m.d_map.get(), d_values0, sigma0, d_values1, sigma1, h->Lx.get(), m.nnz);
     g_launch_count++;
   }
   CUDA_OK(cudaGetLastError());
@@ -1601,10 +1564,10 @@ int slmm_chol_factorize(slmm_chol_t* h, int32_t* fail_col) {
   SLMM_TRY
   if (!h) throw std::invalid_argument("null handle");
   const int big = 0x7fffffff;
-  CUDA_OK(cudaMemcpyAsync(h->d_info, &big, sizeof(int), cudaMemcpyHostToDevice, 0));
+  CUDA_OK(cudaMemcpyAsync(h->d_info.get(), &big, sizeof(int), cudaMemcpyHostToDevice, 0));
   run_schedule(h, h->fact, nullptr, nullptr, nullptr, 0);
   int info = 0;
-  CUDA_OK(cudaMemcpy(&info, h->d_info, sizeof(int), cudaMemcpyDeviceToHost));
+  CUDA_OK(cudaMemcpy(&info, h->d_info.get(), sizeof(int), cudaMemcpyDeviceToHost));
   if (info != big) {
     if (fail_col) *fail_col = info - 1;
     set_last_error("matrix is not positive definite (non-positive pivot at permuted column " + std::to_string(info - 1) + ")");
@@ -1621,10 +1584,10 @@ int slmm_chol_logdet(slmm_chol_t* h, double* out) {
   if (!h || !out) throw std::invalid_argument("null argument");
   if (!h->factored) throw std::invalid_argument("factorize first");
   const int grid = std::min(1024, (h->S.n + 255) / 256);
-  logdet_kernel<<<grid, 256>>>(h->Lx, h->d_col2sn, h->d_sn_first, h->d_sn_nrow, h->d_sn_lptr, h->S.n, h->d_partial);
+  logdet_kernel<<<grid, 256>>>(h->Lx.get(), h->d_col2sn.get(), h->d_sn_first.get(), h->d_sn_nrow.get(), h->d_sn_lptr.get(), h->S.n, h->d_partial.get());
   g_launch_count++;
   std::vector<double> part(grid);
-  CUDA_OK(cudaMemcpy(part.data(), h->d_partial, grid * sizeof(double), cudaMemcpyDeviceToHost));
+  CUDA_OK(cudaMemcpy(part.data(), h->d_partial.get(), grid * sizeof(double), cudaMemcpyDeviceToHost));
   double s = 0;
   for (double v : part) s += v;
   *out = 2.0 * s;
@@ -1641,10 +1604,10 @@ int slmm_chol_solve(slmm_chol_t* h, double* d_B, int32_t nrhs, int32_t mode) {
   const int64_t total = (int64_t)n * nrhs;
   const int grid = (int)std::min<int64_t>((total + 255) / 256, 148 * 32);
   // forward consumes X and leaves y in X2; backward consumes X2 and leaves x in X
-  gather_rows_kernel<<<grid, 256, 0, h->cur>>>(d_B, mode == 2 ? pl->X2 : pl->X, h->d_perm, n, nrhs, 0);
-  if (mode == 0 || mode == 1) run_schedule(h, pl->fwd, pl->X, pl->arena, pl->d_vptr, nrhs);
-  if (mode == 0 || mode == 2) run_schedule(h, pl->bwd, pl->X, pl->arena, pl->d_vptr, nrhs);
-  gather_rows_kernel<<<grid, 256, 0, h->cur>>>(mode == 1 ? pl->X2 : pl->X, d_B, h->d_perm, n, nrhs, 1);
+  gather_rows_kernel<<<grid, 256, 0, h->cur>>>(d_B, mode == 2 ? pl->X2.get() : pl->X.get(), h->d_perm.get(), n, nrhs, 0);
+  if (mode == 0 || mode == 1) run_schedule(h, pl->fwd, pl->X.get(), pl->arena, pl->d_vptr.get(), nrhs);
+  if (mode == 0 || mode == 2) run_schedule(h, pl->bwd, pl->X.get(), pl->arena, pl->d_vptr.get(), nrhs);
+  gather_rows_kernel<<<grid, 256, 0, h->cur>>>(mode == 1 ? pl->X2.get() : pl->X.get(), d_B, h->d_perm.get(), n, nrhs, 1);
   g_launch_count += 2;
   CUDA_OK(cudaGetLastError());
   return SLMM_OK;
@@ -1658,10 +1621,10 @@ int slmm_chol_lmul(slmm_chol_t* h, const double* d_Z, double* d_out, int32_t nrh
   SolvePlan* pl = get_plan(h, nrhs);
   const int n = h->S.n;
   const int64_t total = (int64_t)n * nrhs;
-  CUDA_OK(cudaMemcpyAsync(pl->X, d_Z, total * sizeof(double), cudaMemcpyDeviceToDevice, h->cur));
-  run_schedule(h, pl->lmul, pl->X2, pl->arena, pl->d_vptr, nrhs);
+  CUDA_OK(cudaMemcpyAsync(pl->X.get(), d_Z, total * sizeof(double), cudaMemcpyDeviceToDevice, h->cur));
+  run_schedule(h, pl->lmul, pl->X2.get(), pl->arena, pl->d_vptr.get(), nrhs);
   const int grid = (int)std::min<int64_t>((total + 255) / 256, 148 * 32);
-  gather_rows_kernel<<<grid, 256, 0, h->cur>>>(pl->X2, d_out, h->d_perm, n, nrhs, 1);
+  gather_rows_kernel<<<grid, 256, 0, h->cur>>>(pl->X2.get(), d_out, h->d_perm.get(), n, nrhs, 1);
   g_launch_count++;
   CUDA_OK(cudaGetLastError());
   return SLMM_OK;
@@ -1686,7 +1649,7 @@ int slmm_chol_export_L(slmm_chol_t* h, int64_t* colptr, int32_t* rowidx, double*
   if (!h->factored) throw std::invalid_argument("factorize first");
   const Symbolic& S = h->S;
   std::vector<double> Lh(S.lsize);
-  CUDA_OK(cudaMemcpy(Lh.data(), h->Lx, S.lsize * sizeof(double), cudaMemcpyDeviceToHost));
+  CUDA_OK(cudaMemcpy(Lh.data(), h->Lx.get(), S.lsize * sizeof(double), cudaMemcpyDeviceToHost));
   int64_t q = 0;
   for (int s = 0; s < S.nsuper; s++) {
     const int f = S.sn_first[s], ns = S.sn_first[s + 1] - f, ms = S.sn_nrow[s];
@@ -1706,9 +1669,9 @@ int slmm_chol_aux_begin(slmm_chol_t* h) {
   SLMM_TRY
   if (!h || !h->s_aux) throw std::invalid_argument("null handle");
   if (h->cur != nullptr) throw std::invalid_argument("auxiliary section already open");
-  CUDA_OK(cudaEventRecord(h->ev_aux, 0));               // everything issued so far (the factorization) comes first
-  CUDA_OK(cudaStreamWaitEvent(h->s_aux, h->ev_aux, 0));
-  h->cur = h->s_aux;
+  CUDA_OK(cudaEventRecord(h->ev_aux.get(), 0));         // everything issued so far (the factorization) comes first
+  CUDA_OK(cudaStreamWaitEvent(h->s_aux.get(), h->ev_aux.get(), 0));
+  h->cur = h->s_aux.get();
   return SLMM_OK;
   SLMM_CATCH
 }
@@ -1722,8 +1685,8 @@ int slmm_chol_aux_end(slmm_chol_t* h) {
 int slmm_chol_aux_join(slmm_chol_t* h) {
   SLMM_TRY
   if (!h || !h->s_aux) throw std::invalid_argument("null handle");
-  CUDA_OK(cudaEventRecord(h->ev_aux, h->s_aux));
-  CUDA_OK(cudaStreamWaitEvent(0, h->ev_aux, 0));
+  CUDA_OK(cudaEventRecord(h->ev_aux.get(), h->s_aux.get()));
+  CUDA_OK(cudaStreamWaitEvent(0, h->ev_aux.get(), 0));
   return SLMM_OK;
   SLMM_CATCH
 }
@@ -1731,7 +1694,7 @@ int slmm_chol_aux_join(slmm_chol_t* h) {
 int slmm_chol_copy_panels(slmm_chol_t* h, double* host_out) {
   SLMM_TRY
   if (!h || !host_out) throw std::invalid_argument("null argument");
-  CUDA_OK(cudaMemcpy(host_out, h->Lx, h->S.lsize * sizeof(double), cudaMemcpyDeviceToHost));
+  CUDA_OK(cudaMemcpy(host_out, h->Lx.get(), h->S.lsize * sizeof(double), cudaMemcpyDeviceToHost));
   return SLMM_OK;
   SLMM_CATCH
 }
@@ -1769,7 +1732,7 @@ int slmm_chol_get_timeline(slmm_chol_t* h, int32_t max_n, int32_t* n_out, float*
       if (L.kind == Launch::EV_RECORD && L.count + 2 < n) rec_stream[L.count] = L.stream;
     for (int q = 0; q < n && q < max_n; q++) {
       float v = 0.f;
-      if (q > 0) CUDA_OK(cudaEventElapsedTime(&v, h->tl_events[0], h->tl_events[q]));
+      if (q > 0) CUDA_OK(cudaEventElapsedTime(&v, h->tl_events[0].get(), h->tl_events[q].get()));
       ms[q] = v;
       if (stream) stream[q] = q >= 2 ? rec_stream[q - 2] : 0;
     }
@@ -1787,7 +1750,7 @@ int slmm_chol_get_launch_timeline(slmm_chol_t* h, int32_t max_n, int32_t* n_out,
   const int n = (int)std::min(ks.size(), h->tl_launch.size());
   *n_out = n;
   for (int q = 0; q < n && q < max_n; q++) {
-    if (end_ms) { float v = 0.f; CUDA_OK(cudaEventElapsedTime(&v, h->tl_events[0], h->tl_launch[q])); end_ms[q] = v; }
+    if (end_ms) { float v = 0.f; CUDA_OK(cudaEventElapsedTime(&v, h->tl_events[0].get(), h->tl_launch[q].get())); end_ms[q] = v; }
     if (stream) stream[q] = ks[q]->stream;
     if (kind) kind[q] = (int)ks[q]->kind;
     if (grid) grid[q] = (ks[q]->kind <= Launch::GEMM_SMALL || ks[q]->kind >= Launch::SKINNY_F1) ? ks[q]->grid : ks[q]->count;
@@ -1905,7 +1868,6 @@ int slmm_gemm_selftest_ex(int32_t M, int32_t N, int32_t K, const double* d_A, in
   slmm_chol dummy;
   run_schedule(&dummy, sch, nullptr, nullptr, nullptr, 0);
   CUDA_OK(cudaDeviceSynchronize());
-  sch.release();
   return SLMM_OK;
   SLMM_CATCH
 }
@@ -1919,21 +1881,16 @@ int slmm_gemm_selftest(int32_t M, int32_t N, int32_t K, const double* d_A, const
   pb.add(make_op(d_C, 1, M, d_A, 1, M, d_B, 1, N, M, N, K, lower ? GF_LOWER : 0));
   pb.flush(sch);
   sch.upload();
-  cudaEvent_t e0, e1;
-  CUDA_OK(cudaEventCreate(&e0));
-  CUDA_OK(cudaEventCreate(&e1));
+  const Event e0 = make_event(cudaEventDefault), e1 = make_event(cudaEventDefault);
   slmm_chol dummy;
   run_schedule(&dummy, sch, nullptr, nullptr, nullptr, 0);
-  CUDA_OK(cudaEventRecord(e0, 0));
+  CUDA_OK(cudaEventRecord(e0.get(), 0));
   for (int r = 0; r < reps; r++) run_schedule(&dummy, sch, nullptr, nullptr, nullptr, 0);
-  CUDA_OK(cudaEventRecord(e1, 0));
-  CUDA_OK(cudaEventSynchronize(e1));
+  CUDA_OK(cudaEventRecord(e1.get(), 0));
+  CUDA_OK(cudaEventSynchronize(e1.get()));
   float ms = 0;
-  CUDA_OK(cudaEventElapsedTime(&ms, e0, e1));
+  CUDA_OK(cudaEventElapsedTime(&ms, e0.get(), e1.get()));
   if (ms_out) *ms_out = reps > 0 ? ms / reps : 0.f;
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
-  sch.release();
   return SLMM_OK;
   SLMM_CATCH
 }

@@ -6,6 +6,7 @@
 
 #include <cstdint>
 #include <cstdio>
+#include <memory>
 #include <stdexcept>
 #include <string>
 
@@ -27,23 +28,36 @@ inline void cuda_check(cudaError_t e, const char* what, const char* file, int li
 }
 #define CUDA_OK(x) ::slmm::cuda_check((x), #x, __FILE__, __LINE__)
 
+// Owning handles: device memory, streams, events and graph execs are freed when their owner goes away, on error
+// paths too.  Raw pointers taken with .get() are views.
+struct CudaFree { void operator()(void* p) const noexcept { cudaFree(p); } };
+struct StreamDestroy { void operator()(cudaStream_t s) const noexcept { cudaStreamDestroy(s); } };
+struct EventDestroy { void operator()(cudaEvent_t e) const noexcept { cudaEventDestroy(e); } };
+struct GraphExecDestroy { void operator()(cudaGraphExec_t g) const noexcept { cudaGraphExecDestroy(g); } };
+template <class T> using DevPtr = std::unique_ptr<T[], CudaFree>;
+using Stream = std::unique_ptr<CUstream_st, StreamDestroy>;
+using Event = std::unique_ptr<CUevent_st, EventDestroy>;
+using GraphExec = std::unique_ptr<CUgraphExec_st, GraphExecDestroy>;
+
 template <typename T>
-T* dev_alloc(size_t count) {
+DevPtr<T> dev_alloc(size_t count) {
   T* p = nullptr;
   if (count == 0) count = 1;
   CUDA_OK(cudaMalloc((void**)&p, count * sizeof(T)));
-  return p;
+  return DevPtr<T>(p);
 }
 
 template <typename T>
-T* dev_upload(const T* host, size_t count, cudaStream_t st = 0) {
-  T* p = dev_alloc<T>(count);
-  if (count) CUDA_OK(cudaMemcpyAsync(p, host, count * sizeof(T), cudaMemcpyHostToDevice, st));
+DevPtr<T> dev_upload(const T* host, size_t count, cudaStream_t st = 0) {
+  DevPtr<T> p = dev_alloc<T>(count);
+  if (count) CUDA_OK(cudaMemcpyAsync(p.get(), host, count * sizeof(T), cudaMemcpyHostToDevice, st));
   return p;
 }
 
-inline void dev_free(void* p) {
-  if (p) cudaFree(p);
+inline Event make_event(unsigned flags) {
+  cudaEvent_t e = nullptr;
+  CUDA_OK(cudaEventCreateWithFlags(&e, flags));
+  return Event(e);
 }
 
 }  // namespace slmm

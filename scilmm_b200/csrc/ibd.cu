@@ -212,9 +212,9 @@ struct slmm_ibd {
   int n = 0;
   int64_t nnzL = 0, nnzA = 0;
   int nlevels = 0;
-  int64_t *d_lptr = nullptr, *d_aptr = nullptr;
-  int32_t *d_lidx = nullptr, *d_aidx = nullptr;
-  double *d_lval = nullptr, *d_aval = nullptr, *d_D = nullptr, *d_F = nullptr;
+  DevPtr<int64_t> d_lptr, d_aptr;
+  DevPtr<int32_t> d_lidx, d_aidx;
+  DevPtr<double> d_lval, d_aval, d_D, d_F;
   std::vector<int64_t> lptr, aptr;
 };
 
@@ -235,30 +235,29 @@ int slmm_ibd_build(int32_t n, const int32_t* h_rel_indptr, const int32_t* h_rel_
   std::unique_ptr<slmm_ibd> h(new slmm_ibd());
   h->n = n;
   const int64_t nrel = h_rel_indptr[n];
-  int32_t* rp = dev_upload(h_rel_indptr, (size_t)n + 1);
-  int32_t* ri = dev_upload(h_rel_indices, (size_t)nrel);
-  int* d_flag = dev_alloc<int>(1);
+  DevPtr<int32_t> rp_own = dev_upload(h_rel_indptr, (size_t)n + 1), ri_own = dev_upload(h_rel_indices, (size_t)nrel);
+  const int32_t *rp = rp_own.get(), *ri = ri_own.get();
+  DevPtr<int> d_flag = dev_alloc<int>(1);
   const int g1 = std::max(1, std::min(148 * 8, (n + 255) / 256));
-  CUDA_OK(cudaMemset(d_flag, 0, sizeof(int)));
-  ibd_check_kernel<<<g1, 256>>>(rp, ri, n, d_flag);
+  CUDA_OK(cudaMemset(d_flag.get(), 0, sizeof(int)));
+  ibd_check_kernel<<<g1, 256>>>(rp, ri, n, d_flag.get());
   int flag = 0;
-  CUDA_OK(cudaMemcpy(&flag, d_flag, sizeof(int), cudaMemcpyDeviceToHost));
+  CUDA_OK(cudaMemcpy(&flag, d_flag.get(), sizeof(int), cudaMemcpyDeviceToHost));
   if (flag) {
-    dev_free(rp); dev_free(ri); dev_free(d_flag);
     throw std::invalid_argument(flag == 1 ? "an individual has more than two parents"
                                           : flag == 2 ? "parents must precede their children (topological order)"
                                                       : "duplicate parent");
   }
   // ---- levels
-  int32_t* d_depth = dev_alloc<int32_t>(n);
-  CUDA_OK(cudaMemset(d_depth, 0, sizeof(int32_t) * n));
+  DevPtr<int32_t> d_depth = dev_alloc<int32_t>(n);
+  CUDA_OK(cudaMemset(d_depth.get(), 0, sizeof(int32_t) * n));
   for (int sweep = 0; sweep < n + 1; sweep++) {
-    CUDA_OK(cudaMemset(d_flag, 0, sizeof(int)));
-    ibd_depth_kernel<<<g1, 256>>>(rp, ri, n, d_depth, d_flag);
-    CUDA_OK(cudaMemcpy(&flag, d_flag, sizeof(int), cudaMemcpyDeviceToHost));
+    CUDA_OK(cudaMemset(d_flag.get(), 0, sizeof(int)));
+    ibd_depth_kernel<<<g1, 256>>>(rp, ri, n, d_depth.get(), d_flag.get());
+    CUDA_OK(cudaMemcpy(&flag, d_flag.get(), sizeof(int), cudaMemcpyDeviceToHost));
     if (!flag) break;
   }
-  std::vector<int32_t> depth = to_host(d_depth, n);
+  std::vector<int32_t> depth = to_host(d_depth.get(), n);
   int maxd = 0;
   for (int i = 0; i < n; i++) maxd = std::max(maxd, depth[i]);
   h->nlevels = maxd + 1;
@@ -269,23 +268,24 @@ int slmm_ibd_build(int32_t n, const int32_t* h_rel_indptr, const int32_t* h_rel_
     std::vector<int32_t> fill(level_ptr.begin(), level_ptr.end() - 1);
     for (int i = 0; i < n; i++) level_rows[fill[depth[i]]++] = i;
   }
-  int32_t* d_level_rows = dev_upload(level_rows.data(), (size_t)n);
+  DevPtr<int32_t> d_level_rows = dev_upload(level_rows.data(), (size_t)n);
   // ---- T (the reference's L), level by level into a level-ordered pool
-  int32_t* d_tlen = dev_alloc<int32_t>(n);
-  int64_t* d_tptr = dev_alloc<int64_t>(n);
+  DevPtr<int32_t> d_tlen = dev_alloc<int32_t>(n);
+  DevPtr<int64_t> d_tptr = dev_alloc<int64_t>(n);
   std::vector<int64_t> tptr(n, 0);
   std::vector<int32_t> tlen(n, 0);
   int64_t pool = 0, cap = std::max<int64_t>(1024, 8LL * n);
-  int32_t* d_tidx = dev_alloc<int32_t>((size_t)cap);
-  double* d_tval = dev_alloc<double>((size_t)cap);
+  DevPtr<int32_t> d_tidx = dev_alloc<int32_t>((size_t)cap);
+  DevPtr<double> d_tval = dev_alloc<double>((size_t)cap);
   h->d_D = dev_alloc<double>(n);
   h->d_F = dev_alloc<double>(n);
   for (int d = 0; d <= maxd; d++) {
     const int r0 = level_ptr[d], nr = level_ptr[d + 1] - r0;
     if (nr == 0) continue;
     const int grid = (nr + 127) / 128;
-    ibd_trow_kernel<<<grid, 128>>>(d_level_rows + r0, nr, rp, ri, d_tptr, d_tlen, d_tidx, d_tval, d_tlen, false);
-    std::vector<int32_t> len_all = to_host(d_tlen, n);          // small: 4n bytes per level
+    ibd_trow_kernel<<<grid, 128>>>(d_level_rows.get() + r0, nr, rp, ri, d_tptr.get(), d_tlen.get(), d_tidx.get(), d_tval.get(),
+                                   d_tlen.get(), false);
+    std::vector<int32_t> len_all = to_host(d_tlen.get(), n);          // small: 4n bytes per level
     for (int q = 0; q < nr; q++) {
       const int i = level_rows[r0 + q];
       tlen[i] = len_all[i];
@@ -294,17 +294,18 @@ int slmm_ibd_build(int32_t n, const int32_t* h_rel_indptr, const int32_t* h_rel_
     }
     if (pool > cap) {                                           // grow the pool (contents copied device to device)
       int64_t ncap = std::max(pool, cap * 2);
-      int32_t* ni = dev_alloc<int32_t>((size_t)ncap);
-      double* nv = dev_alloc<double>((size_t)ncap);
+      DevPtr<int32_t> ni = dev_alloc<int32_t>((size_t)ncap);
+      DevPtr<double> nv = dev_alloc<double>((size_t)ncap);
       const int64_t used = tptr[level_rows[r0]];
-      CUDA_OK(cudaMemcpy(ni, d_tidx, used * sizeof(int32_t), cudaMemcpyDeviceToDevice));
-      CUDA_OK(cudaMemcpy(nv, d_tval, used * sizeof(double), cudaMemcpyDeviceToDevice));
-      dev_free(d_tidx); dev_free(d_tval);
-      d_tidx = ni; d_tval = nv; cap = ncap;
+      CUDA_OK(cudaMemcpy(ni.get(), d_tidx.get(), used * sizeof(int32_t), cudaMemcpyDeviceToDevice));
+      CUDA_OK(cudaMemcpy(nv.get(), d_tval.get(), used * sizeof(double), cudaMemcpyDeviceToDevice));
+      d_tidx = std::move(ni); d_tval = std::move(nv); cap = ncap;
     }
-    CUDA_OK(cudaMemcpy(d_tptr, tptr.data(), sizeof(int64_t) * n, cudaMemcpyHostToDevice));
-    ibd_trow_kernel<<<grid, 128>>>(d_level_rows + r0, nr, rp, ri, d_tptr, d_tlen, d_tidx, d_tval, nullptr, true);
-    ibd_df_kernel<<<grid, 128>>>(d_level_rows + r0, nr, rp, ri, d_tptr, d_tlen, d_tidx, d_tval, h->d_D, h->d_F);
+    CUDA_OK(cudaMemcpy(d_tptr.get(), tptr.data(), sizeof(int64_t) * n, cudaMemcpyHostToDevice));
+    ibd_trow_kernel<<<grid, 128>>>(d_level_rows.get() + r0, nr, rp, ri, d_tptr.get(), d_tlen.get(), d_tidx.get(), d_tval.get(),
+                                   nullptr, true);
+    ibd_df_kernel<<<grid, 128>>>(d_level_rows.get() + r0, nr, rp, ri, d_tptr.get(), d_tlen.get(), d_tidx.get(), d_tval.get(),
+                                 h->d_D.get(), h->d_F.get());
     g_launch_count += 3;
   }
   CUDA_OK(cudaGetLastError());
@@ -315,47 +316,49 @@ int slmm_ibd_build(int32_t n, const int32_t* h_rel_indptr, const int32_t* h_rel_
   h->d_lptr = dev_upload(h->lptr.data(), (size_t)n + 1);
   h->d_lidx = dev_alloc<int32_t>((size_t)pool);
   h->d_lval = dev_alloc<double>((size_t)pool);
-  uint64_t* d_keys = dev_alloc<uint64_t>((size_t)pool);
-  ibd_compact_kernel<<<std::max(1, std::min(148 * 8, (n + 7) / 8)), 256>>>(n, d_tptr, d_tlen, d_tidx, d_tval, h->d_lptr,
-                                                                         h->d_lidx, h->d_lval, d_keys);
+  DevPtr<uint64_t> d_keys = dev_alloc<uint64_t>((size_t)pool);
+  ibd_compact_kernel<<<std::max(1, std::min(148 * 8, (n + 7) / 8)), 256>>>(n, d_tptr.get(), d_tlen.get(), d_tidx.get(), d_tval.get(),
+                                                                         h->d_lptr.get(), h->d_lidx.get(), h->d_lval.get(), d_keys.get());
   g_launch_count++;
   CUDA_OK(cudaDeviceSynchronize());
-  dev_free(d_tidx); dev_free(d_tval); dev_free(d_tptr); dev_free(d_tlen); dev_free(d_level_rows); dev_free(d_depth);
+  d_tidx.reset(); d_tval.reset(); d_tptr.reset(); d_tlen.reset(); d_level_rows.reset(); d_depth.reset();
   // ---- L' as CSR (columns of L with ascending rows): stable radix sort of (column, row) keys
-  uint64_t* d_keys2 = dev_alloc<uint64_t>((size_t)pool);
-  double* d_cval = dev_alloc<double>((size_t)pool);
+  DevPtr<uint64_t> d_keys2 = dev_alloc<uint64_t>((size_t)pool);
+  DevPtr<double> d_cval = dev_alloc<double>((size_t)pool);
   {
     size_t tmp_bytes = 0;
     int bits = 32;
     while ((1LL << (bits - 32)) < n && bits < 64) bits++;
-    CUDA_OK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, d_keys, d_keys2, h->d_lval, d_cval, (int64_t)pool, 0, bits));
-    void* tmp = dev_alloc<char>(tmp_bytes);
-    CUDA_OK(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, d_keys, d_keys2, h->d_lval, d_cval, (int64_t)pool, 0, bits));
+    CUDA_OK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, d_keys.get(), d_keys2.get(), h->d_lval.get(), d_cval.get(),
+                                            (int64_t)pool, 0, bits));
+    DevPtr<char> tmp = dev_alloc<char>(tmp_bytes);
+    CUDA_OK(cub::DeviceRadixSort::SortPairs(tmp.get(), tmp_bytes, d_keys.get(), d_keys2.get(), h->d_lval.get(), d_cval.get(),
+                                            (int64_t)pool, 0, bits));
     CUDA_OK(cudaDeviceSynchronize());
-    dev_free(tmp);
   }
-  dev_free(d_keys);
-  int32_t* d_ccount = dev_alloc<int32_t>(n);
-  CUDA_OK(cudaMemset(d_ccount, 0, sizeof(int32_t) * n));
-  ibd_colcount_kernel<<<(int)std::min<int64_t>((pool + 255) / 256, 148 * 16), 256>>>(d_keys2, pool, d_ccount);
-  std::vector<int32_t> ccount = to_host(d_ccount, n);
-  dev_free(d_ccount);
+  d_keys.reset();
+  DevPtr<int32_t> d_ccount = dev_alloc<int32_t>(n);
+  CUDA_OK(cudaMemset(d_ccount.get(), 0, sizeof(int32_t) * n));
+  ibd_colcount_kernel<<<(int)std::min<int64_t>((pool + 255) / 256, 148 * 16), 256>>>(d_keys2.get(), pool, d_ccount.get());
+  std::vector<int32_t> ccount = to_host(d_ccount.get(), n);
+  d_ccount.reset();
   std::vector<int64_t> cptr((size_t)n + 1, 0);
   for (int j = 0; j < n; j++) cptr[j + 1] = cptr[j] + ccount[j];
-  int64_t* d_cptr = dev_upload(cptr.data(), (size_t)n + 1);
+  DevPtr<int64_t> d_cptr = dev_upload(cptr.data(), (size_t)n + 1);
   // ---- A = (L D) L'
   const int words = (n + 31) / 32;
   int warps = 148 * 8;
   const int64_t scratch_cap = (int64_t)6 << 30;                  // at most 6 GB of dense accumulators
   warps = (int)std::max<int64_t>(8, std::min<int64_t>(warps, scratch_cap / (8LL * n)));
   warps = (warps / 8) * 8;
-  uint32_t* d_bm = dev_alloc<uint32_t>((size_t)warps * words);
-  CUDA_OK(cudaMemset(d_bm, 0, sizeof(uint32_t) * (size_t)warps * words));
-  int32_t* d_alen = dev_alloc<int32_t>(n);
-  ibd_numerator_kernel<<<warps / 8, 256>>>(n, h->d_lptr, h->d_lidx, h->d_lval, d_cptr, d_keys2, d_cval, h->d_D, d_bm, nullptr,
-                                           words, nullptr, nullptr, nullptr, d_alen, false);
-  std::vector<int32_t> alen = to_host(d_alen, n);
-  dev_free(d_alen);
+  DevPtr<uint32_t> d_bm = dev_alloc<uint32_t>((size_t)warps * words);
+  CUDA_OK(cudaMemset(d_bm.get(), 0, sizeof(uint32_t) * (size_t)warps * words));
+  DevPtr<int32_t> d_alen = dev_alloc<int32_t>(n);
+  ibd_numerator_kernel<<<warps / 8, 256>>>(n, h->d_lptr.get(), h->d_lidx.get(), h->d_lval.get(), d_cptr.get(), d_keys2.get(),
+                                           d_cval.get(), h->d_D.get(), d_bm.get(), nullptr, words, nullptr, nullptr, nullptr,
+                                           d_alen.get(), false);
+  std::vector<int32_t> alen = to_host(d_alen.get(), n);
+  d_alen.reset();
   h->aptr.assign((size_t)n + 1, 0);
   for (int i = 0; i < n; i++) h->aptr[i + 1] = h->aptr[i] + alen[i];
   h->nnzA = h->aptr[n];
@@ -363,15 +366,14 @@ int slmm_ibd_build(int32_t n, const int32_t* h_rel_indptr, const int32_t* h_rel_
   h->d_aptr = dev_upload(h->aptr.data(), (size_t)n + 1);
   h->d_aidx = dev_alloc<int32_t>((size_t)h->nnzA);
   h->d_aval = dev_alloc<double>((size_t)h->nnzA);
-  double* d_acc = dev_alloc<double>((size_t)warps * n);
-  CUDA_OK(cudaMemset(d_acc, 0, sizeof(double) * (size_t)warps * n));
-  ibd_numerator_kernel<<<warps / 8, 256>>>(n, h->d_lptr, h->d_lidx, h->d_lval, d_cptr, d_keys2, d_cval, h->d_D, d_bm, d_acc,
-                                           words, h->d_aptr, h->d_aidx, h->d_aval, nullptr, true);
+  DevPtr<double> d_acc = dev_alloc<double>((size_t)warps * n);
+  CUDA_OK(cudaMemset(d_acc.get(), 0, sizeof(double) * (size_t)warps * n));
+  ibd_numerator_kernel<<<warps / 8, 256>>>(n, h->d_lptr.get(), h->d_lidx.get(), h->d_lval.get(), d_cptr.get(), d_keys2.get(),
+                                           d_cval.get(), h->d_D.get(), d_bm.get(), d_acc.get(), words, h->d_aptr.get(),
+                                           h->d_aidx.get(), h->d_aval.get(), nullptr, true);
   g_launch_count += 3;
   CUDA_OK(cudaDeviceSynchronize());
   CUDA_OK(cudaGetLastError());
-  dev_free(d_acc); dev_free(d_bm); dev_free(d_cptr); dev_free(d_keys2); dev_free(d_cval);
-  dev_free(rp); dev_free(ri); dev_free(d_flag);
   *out = h.release();
   return SLMM_OK;
   SLMM_CATCH
@@ -396,7 +398,7 @@ int slmm_ibd_copy_L(const slmm_ibd_t* h, int32_t* h_indptr, int32_t* h_indices, 
   SLMM_TRY
   if (!h || !h_indptr || !h_indices || !h_data) throw std::invalid_argument("null argument");
   if (h->nnzL > 0x7fffffffLL) throw std::invalid_argument("L has more than 2^31-1 entries");
-  copy_csr(h->n, h->lptr, h->d_lidx, h->d_lval, h_indptr, h_indices, h_data);
+  copy_csr(h->n, h->lptr, h->d_lidx.get(), h->d_lval.get(), h_indptr, h_indices, h_data);
   return SLMM_OK;
   SLMM_CATCH
 }
@@ -404,7 +406,7 @@ int slmm_ibd_copy_L(const slmm_ibd_t* h, int32_t* h_indptr, int32_t* h_indices, 
 int slmm_ibd_copy_A(const slmm_ibd_t* h, int32_t* h_indptr, int32_t* h_indices, double* h_data) {
   SLMM_TRY
   if (!h || !h_indptr || !h_indices || !h_data) throw std::invalid_argument("null argument");
-  copy_csr(h->n, h->aptr, h->d_aidx, h->d_aval, h_indptr, h_indices, h_data);
+  copy_csr(h->n, h->aptr, h->d_aidx.get(), h->d_aval.get(), h_indptr, h_indices, h_data);
   return SLMM_OK;
   SLMM_CATCH
 }
@@ -412,16 +414,13 @@ int slmm_ibd_copy_A(const slmm_ibd_t* h, int32_t* h_indptr, int32_t* h_indices, 
 int slmm_ibd_copy_DF(const slmm_ibd_t* h, double* h_D, double* h_F) {
   SLMM_TRY
   if (!h) throw std::invalid_argument("null argument");
-  if (h_D) CUDA_OK(cudaMemcpy(h_D, h->d_D, sizeof(double) * h->n, cudaMemcpyDeviceToHost));
-  if (h_F) CUDA_OK(cudaMemcpy(h_F, h->d_F, sizeof(double) * h->n, cudaMemcpyDeviceToHost));
+  if (h_D) CUDA_OK(cudaMemcpy(h_D, h->d_D.get(), sizeof(double) * h->n, cudaMemcpyDeviceToHost));
+  if (h_F) CUDA_OK(cudaMemcpy(h_F, h->d_F.get(), sizeof(double) * h->n, cudaMemcpyDeviceToHost));
   return SLMM_OK;
   SLMM_CATCH
 }
 
 int slmm_ibd_destroy(slmm_ibd_t* h) {
-  if (!h) return SLMM_OK;
-  dev_free(h->d_lptr); dev_free(h->d_aptr); dev_free(h->d_lidx); dev_free(h->d_aidx);
-  dev_free(h->d_lval); dev_free(h->d_aval); dev_free(h->d_D); dev_free(h->d_F);
   delete h;
   return SLMM_OK;
 }

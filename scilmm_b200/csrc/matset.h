@@ -14,17 +14,19 @@ namespace slmm {
 constexpr int MAXK = 8;
 
 struct CsrDev {
+  // views: the owned buffers below, the pattern leader's arrays, or device arrays bound by the caller
   const int32_t* indptr = nullptr;
   const int32_t* indices = nullptr;
   const double* data = nullptr;
+  DevPtr<int32_t> own_indptr, own_indices;
+  DevPtr<double> own_data;
   int64_t nnz = 0;
   int pattern = -1;       // index of the first matrix with this pattern
-  bool owned_pattern = false, owned_data = false;
   std::vector<int32_t> h_indptr;   // kept for pattern comparison (uploaded matrices only)
   uint64_t idx_hash = 0;
   int symmetric = -1;      // -1 unknown, 0 no, 1 yes (checked on the device on first use)
   int32_t* rend = nullptr; // per row: one past the last entry with col <= row (pattern leaders only, built lazily)
-  int32_t* rend_base = nullptr;   // allocation behind rend (rend is shifted by -r0 for row-block shards)
+  DevPtr<int32_t> rend_base;   // allocation behind rend (rend is shifted by -r0 for row-block shards)
 };
 
 
@@ -34,34 +36,25 @@ struct RedDesc { int64_t off; int32_t stride, nblocks, dst, pad; };
 struct QuadTiles {
   int ntiles = 0, nrb = 0, ncta = 0;
   int64_t nentries = 0, ndistinct = 0;
-  int64_t* tile_ptr = nullptr;      // [ntiles+1] entry range of every tile
-  int32_t* tile_rb = nullptr;       // [ntiles] row block (64 permuted rows) of the tile
-  int32_t* tile_dc0 = nullptr;      // [ntiles] first entry of the tile's column list in dcols
-  int32_t* tile_nc = nullptr;       // [ntiles] columns in the tile (<= 64)
-  uint16_t* rowptr = nullptr;       // [ntiles*65] row starts inside the tile
-  uint16_t* rc = nullptr;           // [nentries] local column << 1 | diagonal flag
-  uint8_t* roword = nullptr;        // [ntiles*64] rows of a tile by decreasing length, dealt to the 8 warps in snake order (0xFF: none)
-  uint32_t* pos = nullptr;          // [nentries] position of the entry in the matrix' own CSR arrays
-  int32_t* dcols = nullptr;         // [ndistinct] ORIGINAL row id of the gathered block for every tile column
-  int32_t* rowid = nullptr;         // [nrb*64] original row id of every permuted row (-1 past n)
-  int32_t* cta_begin = nullptr;     // [ncta+1] contiguous tile ranges of equal cost
-  int32_t* pair_base = nullptr;     // [ncta+1] first (CTA, row block) pair of every CTA
-  int32_t* pair_rb = nullptr;       // [npairs] row block of every pair
-  double* hpairs = nullptr;         // [npairs][64][2][16] narrow-block row products, one block per pair
+  DevPtr<int64_t> tile_ptr;         // [ntiles+1] entry range of every tile
+  DevPtr<int32_t> tile_rb;          // [ntiles] row block (64 permuted rows) of the tile
+  DevPtr<int32_t> tile_dc0;         // [ntiles] first entry of the tile's column list in dcols
+  DevPtr<int32_t> tile_nc;          // [ntiles] columns in the tile (<= 64)
+  DevPtr<uint16_t> rowptr;          // [ntiles*65] row starts inside the tile
+  DevPtr<uint16_t> rc;              // [nentries] local column << 1 | diagonal flag
+  DevPtr<uint8_t> roword;           // [ntiles*64] rows of a tile by decreasing length, dealt to the 8 warps in snake order (0xFF: none)
+  DevPtr<uint32_t> pos;             // [nentries] position of the entry in the matrix' own CSR arrays
+  DevPtr<int32_t> dcols;            // [ndistinct] ORIGINAL row id of the gathered block for every tile column
+  DevPtr<int32_t> rowid;            // [nrb*64] original row id of every permuted row (-1 past n)
+  DevPtr<int32_t> cta_begin;        // [ncta+1] contiguous tile ranges of equal cost
+  DevPtr<int32_t> pair_base;        // [ncta+1] first (CTA, row block) pair of every CTA
+  DevPtr<int32_t> pair_rb;          // [npairs] row block of every pair
+  DevPtr<double> hpairs;            // [npairs][64][2][16] narrow-block row products, one block per pair
   int npairs = 0;
   std::vector<int64_t> cta_stats;    // [ncta][3] tiles, non-empty rows, entries of every CTA's range (host copy)
-  long long* cta_cycles = nullptr;   // [ncta] clock64 span of every CTA in the last pass (developer profile)
-  std::vector<double*> vals;        // per matrix of the set sharing this pattern: weighted values in tile order
+  DevPtr<long long> cta_cycles;      // [ncta] clock64 span of every CTA in the last pass (developer profile)
+  std::vector<DevPtr<double>> vals;  // per matrix of the set sharing this pattern: weighted values in tile order
   std::vector<int> vals_of;         // which matrix each vals[] belongs to
-  void release() {
-    dev_free(tile_ptr); dev_free(tile_rb); dev_free(tile_dc0); dev_free(tile_nc); dev_free(rowptr); dev_free(rc); dev_free(roword); roword = nullptr;
-    dev_free(pos); dev_free(dcols); dev_free(rowid); dev_free(cta_begin); dev_free(pair_base); dev_free(pair_rb); dev_free(hpairs); dev_free(cta_cycles); cta_cycles = nullptr;
-    pair_base = pair_rb = nullptr; hpairs = nullptr; npairs = 0;
-    for (double* v : vals) dev_free(v);
-    vals.clear(); vals_of.clear();
-    tile_ptr = nullptr; tile_rb = tile_dc0 = tile_nc = dcols = rowid = cta_begin = nullptr; rowptr = rc = nullptr; pos = nullptr;
-    ntiles = 0;
-  }
 };
 
 }  // namespace slmm
@@ -71,36 +64,38 @@ struct slmm_matset {
   int r0 = 0, r1 = 0;      // rows held by this set (a row-block shard of the HE path holds [r0, r1) only)
   bool sharded() const { return r0 != 0 || r1 != n; }
   std::vector<slmm::CsrDev> m;
-  std::map<std::pair<int, int>, int64_t*> cross_maps;   // (probe pattern, target pattern) -> position map (device)
+  std::map<std::pair<int, int>, slmm::DevPtr<int64_t>> cross_maps;   // (probe pattern, target pattern) -> position map (device)
   std::map<int, slmm::QuadTiles> tiles;                  // pattern leader -> tiled lower triangle (built on request)
-  double* d_partial = nullptr;
+  slmm::DevPtr<double> d_partial;
   size_t partial_cap = 0;
-  double* d_y = nullptr;
-  double* d_out = nullptr;
-  int32_t* d_dst = nullptr;
+  slmm::DevPtr<double> d_y;
+  slmm::DevPtr<double> d_out;
+  slmm::DevPtr<int32_t> d_dst;
   // HE calls: one partial arena for all passes + the cached reduction table
-  double* he_arena = nullptr;
+  slmm::DevPtr<double> he_arena;
   size_t he_used = 0;
   static constexpr size_t HE_ARENA = (size_t)148 * 8 * 1024;
   std::vector<slmm::RedDesc> he_desc, he_desc_cached;
-  slmm::RedDesc* d_he_desc = nullptr;
+  slmm::DevPtr<slmm::RedDesc> d_he_desc;
   double* he_part(size_t count) {
     if (!he_arena) he_arena = slmm::dev_alloc<double>(HE_ARENA);
     if (he_used + count > HE_ARENA) throw std::runtime_error("HE partial arena exhausted");
-    double* p = he_arena + he_used;
+    double* p = he_arena.get() + he_used;
     he_used += count;
     return p;
   }
   void he_add(const double* part, int nblocks, int nv, const int32_t* dst) {
-    for (int k = 0; k < nv; k++) he_desc.push_back({(int64_t)(part - he_arena) + k, nv, nblocks, dst[k], 0});
+    for (int k = 0; k < nv; k++) he_desc.push_back({(int64_t)(part - he_arena.get()) + k, nv, nblocks, dst[k], 0});
   }
   double* partial(size_t count) {
     if (count > partial_cap) {
-      slmm::dev_free(d_partial);
+      // free before allocating: the old and the new buffer are never held together
+      d_partial.reset();
+      partial_cap = 0;
       d_partial = slmm::dev_alloc<double>(count);
       partial_cap = count;
     }
-    return d_partial;
+    return d_partial.get();
   }
 };
 

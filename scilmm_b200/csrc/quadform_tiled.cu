@@ -410,7 +410,7 @@ static void qt_launch(const QuadTiles& T, const QtArgs& a, const double* d_X, in
   g_launch_count += 2;
   if (nb > 0) {
     const int gf = std::max(1, std::min(T.npairs, 148 * 4));
-    qt_gram_finish_kernel<G><<<gf, 256>>>(T.hpairs, T.pair_rb, T.npairs, T.rowid, d_X, ncx, nb, part_gram);
+    qt_gram_finish_kernel<G><<<gf, 256>>>(T.hpairs.get(), T.pair_rb.get(), T.npairs, T.rowid.get(), d_X, ncx, nb, part_gram);
     qt_reduce_kernel<<<G * nb * nb, 256>>>(part_gram, gf, G * nb * nb, d_gram);
     g_launch_count += 2;
   }
@@ -441,31 +441,29 @@ int slmm_matset_build_tiles(slmm_matset_t* ms, int32_t k, const int32_t* d_perm,
   if (T.ntiles == 0) {
     const int64_t nnz = c.nnz;
     const int nrb = (n + QT_RB - 1) / QT_RB;
-    uint64_t *keys = dev_alloc<uint64_t>(nnz), *keys_s = dev_alloc<uint64_t>(nnz);
-    uint32_t *pos = dev_alloc<uint32_t>(nnz), *pos_s = dev_alloc<uint32_t>(nnz);
-    unsigned long long* d_cnt = dev_alloc<unsigned long long>(1);
-    CUDA_OK(cudaMemset(d_cnt, 0, sizeof(unsigned long long)));
+    DevPtr<uint64_t> keys = dev_alloc<uint64_t>(nnz), keys_s = dev_alloc<uint64_t>(nnz);
+    DevPtr<uint32_t> pos = dev_alloc<uint32_t>(nnz), pos_s = dev_alloc<uint32_t>(nnz);
+    DevPtr<unsigned long long> d_cnt = dev_alloc<unsigned long long>(1);
+    CUDA_OK(cudaMemset(d_cnt.get(), 0, sizeof(unsigned long long)));
     const int gw = std::max(1, std::min(148 * 8, (n + 7) / 8));
-    qt_keys_kernel<<<gw, 256>>>(c.indptr, c.indices, n, d_iperm, keys, pos, d_cnt);
+    qt_keys_kernel<<<gw, 256>>>(c.indptr, c.indices, n, d_iperm, keys.get(), pos.get(), d_cnt.get());
     unsigned long long cnt = 0;
-    CUDA_OK(cudaMemcpy(&cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost));
-    dev_free(d_cnt);
+    CUDA_OK(cudaMemcpy(&cnt, d_cnt.get(), sizeof(cnt), cudaMemcpyDeviceToHost));
     const int64_t m = (int64_t)cnt;
     if (m <= 0 || m >= (int64_t)0x7fffffff) throw std::invalid_argument("tile build: empty matrix or too many entries");
     size_t tmp_bytes = 0, tb2 = 0;
-    CUDA_OK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, keys, keys_s, pos, pos_s, nnz, 0, 64));
-    int32_t *head = dev_alloc<int32_t>(m), *gidx = dev_alloc<int32_t>(m);
-    CUDA_OK(cub::DeviceScan::InclusiveSum(nullptr, tb2, head, gidx, m));
-    void* tmp = dev_alloc<char>(std::max(tmp_bytes, tb2));
-    CUDA_OK(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys, keys_s, pos, pos_s, nnz, 0, 64));
+    CUDA_OK(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, keys.get(), keys_s.get(), pos.get(), pos_s.get(), nnz, 0, 64));
+    DevPtr<int32_t> head = dev_alloc<int32_t>(m), gidx = dev_alloc<int32_t>(m);
+    CUDA_OK(cub::DeviceScan::InclusiveSum(nullptr, tb2, head.get(), gidx.get(), m));
+    DevPtr<char> tmp = dev_alloc<char>(std::max(tmp_bytes, tb2));
+    CUDA_OK(cub::DeviceRadixSort::SortPairs(tmp.get(), tmp_bytes, keys.get(), keys_s.get(), pos.get(), pos_s.get(), nnz, 0, 64));
     const int ge = (int)std::min<int64_t>((m + 255) / 256, 148 * 16);
-    qt_heads_kernel<<<ge, 256>>>(keys_s, m, head);
-    CUDA_OK(cub::DeviceScan::InclusiveSum(tmp, tb2, head, gidx, m));
-    int64_t* d_rbstart = dev_alloc<int64_t>(nrb + 1);
-    qt_rbstart_kernel<<<(nrb + 256) / 256, 256>>>(keys_s, m, nrb, d_rbstart);
-    std::vector<int64_t> rbstart = qt_to_host(d_rbstart, (size_t)nrb + 1);
-    dev_free(d_rbstart);
-    dev_free(head);
+    qt_heads_kernel<<<ge, 256>>>(keys_s.get(), m, head.get());
+    CUDA_OK(cub::DeviceScan::InclusiveSum(tmp.get(), tb2, head.get(), gidx.get(), m));
+    DevPtr<int64_t> d_rbstart = dev_alloc<int64_t>(nrb + 1);
+    qt_rbstart_kernel<<<(nrb + 256) / 256, 256>>>(keys_s.get(), m, nrb, d_rbstart.get());
+    std::vector<int64_t> rbstart = qt_to_host(d_rbstart.get(), (size_t)nrb + 1);
+    head.reset();
     // distinct columns per row block -> tiles
     std::vector<int32_t> gfirst(nrb, 0), glast(nrb, 0);
     {
@@ -473,11 +471,10 @@ int slmm_matset_build_tiles(slmm_matset_t* ms, int32_t k, const int32_t* d_perm,
       std::vector<int64_t> want;
       for (int rb = 0; rb < nrb; rb++)
         if (rbstart[rb + 1] > rbstart[rb]) { want.push_back(rbstart[rb]); want.push_back(rbstart[rb + 1] - 1); }
-      int64_t* d_want = dev_upload(want.data(), want.size());
-      int32_t* d_got = dev_alloc<int32_t>(want.size());
-      qt_gather_kernel<<<std::max<int>(1, (int)((want.size() + 255) / 256)), 256>>>(gidx, d_want, (int)want.size(), d_got);
-      std::vector<int32_t> got = qt_to_host(d_got, want.size());
-      dev_free(d_want); dev_free(d_got);
+      DevPtr<int64_t> d_want = dev_upload(want.data(), want.size());
+      DevPtr<int32_t> d_got = dev_alloc<int32_t>(want.size());
+      qt_gather_kernel<<<std::max<int>(1, (int)((want.size() + 255) / 256)), 256>>>(gidx.get(), d_want.get(), (int)want.size(), d_got.get());
+      std::vector<int32_t> got = qt_to_host(d_got.get(), want.size());
       size_t q = 0;
       for (int rb = 0; rb < nrb; rb++)
         if (rbstart[rb + 1] > rbstart[rb]) { gfirst[rb] = got[q++]; glast[rb] = got[q++]; }
@@ -497,25 +494,24 @@ int slmm_matset_build_tiles(slmm_matset_t* ms, int32_t k, const int32_t* d_perm,
       ndist = glast[rb];
     }
     const int ntiles = (int)tile_rb.size();
-    int32_t *d_dcol_base = dev_upload(dcol_base.data(), dcol_base.size()), *d_tile_base = dev_upload(tile_base.data(), tile_base.size());
+    DevPtr<int32_t> d_dcol_base = dev_upload(dcol_base.data(), dcol_base.size()), d_tile_base = dev_upload(tile_base.data(), tile_base.size());
     T.dcols = dev_alloc<int32_t>((size_t)ndist);
-    uint64_t* keys2 = keys;                           // reuse the unsorted key buffer
-    qt_keys2_kernel<<<ge, 256>>>(keys_s, pos_s, gidx, m, d_dcol_base, d_tile_base, c.indices, keys2, T.dcols);
-    dev_free(gidx);
-    dev_free(d_dcol_base); dev_free(d_tile_base);
+    uint64_t* keys2 = keys.get();                     // reuse the unsorted key buffer
+    qt_keys2_kernel<<<ge, 256>>>(keys_s.get(), pos_s.get(), gidx.get(), m, d_dcol_base.get(), d_tile_base.get(), c.indices, keys2, T.dcols.get());
+    gidx.reset();
     int bits = 13;
     while ((1LL << (bits - 13)) < ntiles + 1 && bits < 64) bits++;
     T.pos = dev_alloc<uint32_t>((size_t)m);
-    CUDA_OK(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys2, keys_s, pos_s, T.pos, m, 0, bits));
+    CUDA_OK(cub::DeviceRadixSort::SortPairs(tmp.get(), tmp_bytes, keys2, keys_s.get(), pos_s.get(), T.pos.get(), m, 0, bits));
     T.tile_ptr = dev_alloc<int64_t>((size_t)ntiles + 1);
     T.rowptr = dev_alloc<uint16_t>((size_t)ntiles * (QT_RB + 1));
     const int64_t tot = (int64_t)ntiles * (QT_RB + 1) + 1;
-    qt_tileptr_kernel<<<(int)std::min<int64_t>((tot + 255) / 256, 148 * 32), 256>>>(keys_s, m, ntiles, T.tile_ptr, T.rowptr);
+    qt_tileptr_kernel<<<(int)std::min<int64_t>((tot + 255) / 256, 148 * 32), 256>>>(keys_s.get(), m, ntiles, T.tile_ptr.get(), T.rowptr.get());
     T.rc = dev_alloc<uint16_t>((size_t)m);
-    qt_pack_kernel<<<ge, 256>>>(keys_s, m, T.rc);
+    qt_pack_kernel<<<ge, 256>>>(keys_s.get(), m, T.rc.get());
     g_launch_count += 7;
     CUDA_OK(cudaDeviceSynchronize());
-    dev_free(tmp); dev_free(keys); dev_free(keys_s); dev_free(pos); dev_free(pos_s);
+    tmp.reset(); keys.reset(); keys_s.reset(); pos.reset(); pos_s.reset();
     T.tile_rb = dev_upload(tile_rb.data(), tile_rb.size());
     T.tile_dc0 = dev_upload(tile_dc0.data(), tile_dc0.size());
     T.tile_nc = dev_upload(tile_nc.data(), tile_nc.size());
@@ -527,8 +523,8 @@ int slmm_matset_build_tiles(slmm_matset_t* ms, int32_t k, const int32_t* d_perm,
     // entries + 6 per non-empty row
     // + 430 per tile (staging round trips, barriers).  Entries alone left one CTA with
     // 25 646 row segments against a mean of 4 632 (the pass took as long as that CTA: 5 of the 6 ms).
-    std::vector<int64_t> tptr = qt_to_host(T.tile_ptr, (size_t)ntiles + 1);
-    std::vector<uint16_t> rptr = qt_to_host(T.rowptr, (size_t)ntiles * (QT_RB + 1));
+    std::vector<int64_t> tptr = qt_to_host(T.tile_ptr.get(), (size_t)ntiles + 1);
+    std::vector<uint16_t> rptr = qt_to_host(T.rowptr.get(), (size_t)ntiles * (QT_RB + 1));
     const int ncta = std::max(1, std::min(148 * 2, ntiles));
     std::vector<int32_t> cta_begin(ncta + 1, ntiles);
     {
@@ -577,7 +573,7 @@ int slmm_matset_build_tiles(slmm_matset_t* ms, int32_t k, const int32_t* d_perm,
     }
     T.cta_begin = dev_upload(cta_begin.data(), cta_begin.size());
     T.cta_cycles = dev_alloc<long long>((size_t)ncta);
-    CUDA_OK(cudaMemset(T.cta_cycles, 0, (size_t)ncta * sizeof(long long)));
+    CUDA_OK(cudaMemset(T.cta_cycles.get(), 0, (size_t)ncta * sizeof(long long)));
     // (CTA, row block) pairs: where each CTA parks the narrow-block row products of the row blocks it touches
     std::vector<int32_t> pair_base(ncta + 1, 0), pair_rb;
     for (int c2 = 0; c2 < ncta; c2++) {
@@ -597,11 +593,11 @@ int slmm_matset_build_tiles(slmm_matset_t* ms, int32_t k, const int32_t* d_perm,
   bool have = false;
   for (int q : T.vals_of) have = have || q == k;
   if (!have) {
-    double* v = dev_alloc<double>((size_t)T.nentries);
-    qt_values_kernel<<<(int)std::min<int64_t>((T.nentries + 255) / 256, 148 * 16), 256>>>(T.rc, T.pos, ms->m[k].data, T.nentries, ms->m[k].nnz, v);
+    DevPtr<double> v = dev_alloc<double>((size_t)T.nentries);
+    qt_values_kernel<<<(int)std::min<int64_t>((T.nentries + 255) / 256, 148 * 16), 256>>>(T.rc.get(), T.pos.get(), ms->m[k].data, T.nentries, ms->m[k].nnz, v.get());
     CUDA_OK(cudaDeviceSynchronize());
     g_launch_count++;
-    T.vals.push_back(v);
+    T.vals.push_back(std::move(v));
     T.vals_of.push_back(k);
   }
   CUDA_OK(cudaGetLastError());
@@ -624,7 +620,7 @@ int slmm_matset_tile_cta_profile(const slmm_matset_t* ms, int32_t k, int64_t* ou
   if (it == ms->tiles.end() || ncta != it->second.ncta) throw std::invalid_argument("no tiles / wrong CTA count");
   const QuadTiles& T = it->second;
   CUDA_OK(cudaDeviceSynchronize());
-  std::vector<long long> cyc = qt_to_host(T.cta_cycles, (size_t)ncta);
+  std::vector<long long> cyc = qt_to_host(T.cta_cycles.get(), (size_t)ncta);
   for (int c = 0; c < ncta; c++) {
     for (int q = 0; q < 3; q++) out[(size_t)c * 4 + q] = T.cta_stats[(size_t)c * 3 + q];
     out[(size_t)c * 4 + 3] = cyc[c];
@@ -644,13 +640,13 @@ int slmm_quadform_tiled(slmm_matset_t* ms, int32_t nk, const int32_t* ks, const 
   QuadTiles& T = it->second;
   QtArgs a;
   a.nentries = T.nentries; a.ndistinct = T.ndistinct; a.ntiles = T.ntiles; a.nrb = T.nrb; a.n = ms->n; a.pad = 0;
-  a.tile_ptr = T.tile_ptr; a.tile_rb = T.tile_rb; a.tile_dc0 = T.tile_dc0; a.tile_nc = T.tile_nc; a.dcols = T.dcols;
-  a.rowid = T.rowid; a.cta_begin = T.cta_begin; a.rowptr = T.rowptr; a.rc = T.rc; a.roword = T.roword;
-  a.pair_base = T.pair_base; a.hpairs = T.hpairs; a.cta_cycles = T.cta_cycles;
+  a.tile_ptr = T.tile_ptr.get(); a.tile_rb = T.tile_rb.get(); a.tile_dc0 = T.tile_dc0.get(); a.tile_nc = T.tile_nc.get();
+  a.dcols = T.dcols.get(); a.rowid = T.rowid.get(); a.cta_begin = T.cta_begin.get(); a.rowptr = T.rowptr.get(); a.rc = T.rc.get();
+  a.roword = T.roword.get(); a.pair_base = T.pair_base.get(); a.hpairs = T.hpairs.get(); a.cta_cycles = T.cta_cycles.get();
   for (int g = 0; g < nk; g++) {
     a.vals[g] = nullptr;
     for (size_t q = 0; q < T.vals_of.size(); q++)
-      if (T.vals_of[q] == ks[g]) a.vals[g] = T.vals[q];
+      if (T.vals_of[q] == ks[g]) a.vals[g] = T.vals[q].get();
     if (!a.vals[g]) throw std::invalid_argument("matrix has no tiled values (slmm_matset_build_tiles per matrix)");
   }
   if (nk == 1) a.vals[1] = a.vals[0];

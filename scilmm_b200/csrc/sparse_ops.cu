@@ -835,16 +835,6 @@ int slmm_matset_create(int32_t n, int32_t K, slmm_matset_t** out) {
 }
 
 int slmm_matset_destroy(slmm_matset_t* ms) {
-  if (!ms) return SLMM_OK;
-  for (auto& c : ms->m) {
-    if (c.owned_pattern) { dev_free((void*)c.indptr); dev_free((void*)c.indices); }
-    if (c.owned_data) dev_free((void*)c.data);
-    dev_free(c.rend_base);
-  }
-  dev_free(ms->d_partial); dev_free(ms->d_y); dev_free(ms->d_out); dev_free(ms->d_dst);
-  dev_free(ms->he_arena); dev_free(ms->d_he_desc);
-  for (auto& kv : ms->cross_maps) dev_free(kv.second);
-  for (auto& kv : ms->tiles) kv.second.release();
   delete ms;
   return SLMM_OK;
 }
@@ -853,12 +843,7 @@ int slmm_matset_upload(slmm_matset_t* ms, int32_t k, const int32_t* indptr, cons
   SLMM_TRY
   if (!ms || k < 0 || k >= ms->K || !indptr || !indices || !data) throw std::invalid_argument("bad arguments");
   CsrDev& c = ms->m[k];
-  if (c.owned_pattern) { dev_free((void*)c.indptr); dev_free((void*)c.indices); }
-  if (c.owned_data) dev_free((void*)c.data);
-  dev_free(c.rend_base);
-  for (auto& kv : ms->cross_maps) dev_free(kv.second);
   ms->cross_maps.clear();
-  for (auto& kv : ms->tiles) kv.second.release();
   ms->tiles.clear();
   c = CsrDev();
   if (ms->sharded()) throw std::invalid_argument("slmm_matset_upload takes whole matrices (row-block shards bind device arrays)");
@@ -873,15 +858,16 @@ int slmm_matset_upload(slmm_matset_t* ms, int32_t k, const int32_t* indptr, cons
     if (memcmp(o.h_indptr.data(), indptr, sizeof(int32_t) * (n + 1)) == 0) { c.pattern = j; break; }
   }
   if (c.pattern == k) {
-    c.indptr = dev_upload(indptr, n + 1);
-    c.indices = dev_upload(indices, c.nnz);
-    c.owned_pattern = true;
+    c.own_indptr = dev_upload(indptr, n + 1);
+    c.own_indices = dev_upload(indices, c.nnz);
+    c.indptr = c.own_indptr.get();
+    c.indices = c.own_indices.get();
   } else {
     c.indptr = ms->m[c.pattern].indptr;
     c.indices = ms->m[c.pattern].indices;
   }
-  c.data = dev_upload(data, c.nnz);
-  c.owned_data = true;
+  c.own_data = dev_upload(data, c.nnz);
+  c.data = c.own_data.get();
   CUDA_OK(cudaStreamSynchronize(0));
   return SLMM_OK;
   SLMM_CATCH
@@ -893,12 +879,7 @@ int slmm_matset_bind_device(slmm_matset_t* ms, int32_t k, const int32_t* d_indpt
   if (!ms || k < 0 || k >= ms->K || !d_indptr || !d_indices || !d_data) throw std::invalid_argument("bad arguments");
   if (same_as >= ms->K || same_as == k) throw std::invalid_argument("bad same_as");
   CsrDev& c = ms->m[k];
-  if (c.owned_pattern) { dev_free((void*)c.indptr); dev_free((void*)c.indices); }
-  if (c.owned_data) dev_free((void*)c.data);
-  dev_free(c.rend_base);
-  for (auto& kv : ms->cross_maps) dev_free(kv.second);
   ms->cross_maps.clear();
-  for (auto& kv : ms->tiles) kv.second.release();
   ms->tiles.clear();
   c = CsrDev();
   // row-block shards: d_indptr has r1 - r0 + 1 entries counting from 0; the kernels index rows globally
@@ -945,7 +926,7 @@ int slmm_he_moments(slmm_matset_t* ms, const double* d_y, int32_t r0, int32_t r1
     if (!lead.rend) {
       const int rows = ms->r1 - ms->r0;
       lead.rend_base = dev_alloc<int32_t>(rows);
-      lead.rend = lead.rend_base - ms->r0;
+      lead.rend = lead.rend_base.get() - ms->r0;
       row_end_kernel<<<std::max(1, std::min(148 * 8, (rows + 255) / 256)), 256>>>(lead.indptr, lead.indices, ms->r0, ms->r1, lead.rend);
       g_launch_count++;
     }
@@ -1014,13 +995,14 @@ int slmm_he_moments(slmm_matset_t* ms, const double* d_y, int32_t r0, int32_t r1
         const std::vector<int>& T = (&P == &chunks[a]) ? chunks[b] : chunks[a];
         const int gp = (int)P.size(), gt = (int)T.size(), nv = gp * gt * 2;
         const int lp = ms->m[P[0]].pattern, lt = ms->m[T[0]].pattern;
-        int64_t*& map = ms->cross_maps[std::make_pair(lp, lt)];
-        if (!map) {             // once per pattern pair: where every probe entry sits in the target
-          map = dev_alloc<int64_t>(ms->m[lp].nnz);
+        DevPtr<int64_t>& owned_map = ms->cross_maps[std::make_pair(lp, lt)];
+        if (!owned_map) {       // once per pattern pair: where every probe entry sits in the target
+          owned_map = dev_alloc<int64_t>(ms->m[lp].nnz);
           cross_map_kernel<<<he_grid(ms->r1 - ms->r0), 256>>>(ms->m[lp].indptr, ms->m[lp].indices, ms->m[lt].indptr,
-                                                              ms->m[lt].indices, ms->r0, ms->r1, sym_all ? 1 : 0, map);
+                                                              ms->m[lt].indices, ms->r0, ms->r1, sym_all ? 1 : 0, owned_map.get());
           g_launch_count++;
         }
+        const int64_t* map = owned_map.get();
         const int64_t pn = ms->m[lp].nnz;
         const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(148 * 8, (pn + 255) / 256));
         double* part = ms->he_part((size_t)grid * nv);
@@ -1052,13 +1034,13 @@ int slmm_he_moments(slmm_matset_t* ms, const double* d_y, int32_t r0, int32_t r1
   // one reduction for every moment of the call; the table is uploaded only when it changed (first call)
   if (!ms->he_desc.empty()) {
     const size_t nd = ms->he_desc.size();
-    if (ms->he_desc_cached.size() != nd ||
+    if (!ms->d_he_desc || ms->he_desc_cached.size() != nd ||
         memcmp(ms->he_desc_cached.data(), ms->he_desc.data(), nd * sizeof(RedDesc)) != 0) {
-      dev_free(ms->d_he_desc);
+      ms->d_he_desc.reset();
       ms->d_he_desc = dev_upload(ms->he_desc.data(), nd);
       ms->he_desc_cached = ms->he_desc;
     }
-    reduce_all_kernel<<<(int)nd, 256>>>(ms->he_arena, ms->d_he_desc, d_out);
+    reduce_all_kernel<<<(int)nd, 256>>>(ms->he_arena.get(), ms->d_he_desc.get(), d_out);
     g_launch_count++;
   }
   CUDA_OK(cudaGetLastError());
@@ -1069,10 +1051,10 @@ int slmm_he_moments(slmm_matset_t* ms, const double* d_y, int32_t r0, int32_t r1
 int slmm_he_moments_host(slmm_matset_t* ms, const double* h_y, double* h_out) {
   SLMM_TRY
   if (!ms || !h_y || !h_out) throw std::invalid_argument("null argument");
-  CUDA_OK(cudaMemcpyAsync(ms->d_y, h_y, sizeof(double) * ms->n, cudaMemcpyHostToDevice, 0));
-  int rc = slmm_he_moments(ms, ms->d_y, 0, ms->n, ms->d_out);
+  CUDA_OK(cudaMemcpyAsync(ms->d_y.get(), h_y, sizeof(double) * ms->n, cudaMemcpyHostToDevice, 0));
+  int rc = slmm_he_moments(ms, ms->d_y.get(), 0, ms->n, ms->d_out.get());
   if (rc != SLMM_OK) return rc;
-  CUDA_OK(cudaMemcpy(h_out, ms->d_out, sizeof(double) * (2 * ms->K + 2 * ms->K * ms->K), cudaMemcpyDeviceToHost));
+  CUDA_OK(cudaMemcpy(h_out, ms->d_out.get(), sizeof(double) * (2 * ms->K + 2 * ms->K * ms->K), cudaMemcpyDeviceToHost));
   return SLMM_OK;
   SLMM_CATCH
 }
@@ -1154,13 +1136,12 @@ int slmm_matset_validate(slmm_matset_t* ms, int32_t k, int32_t* flags_out) {
   SLMM_TRY
   if (!ms || k < 0 || k >= ms->K || !flags_out || !ms->m[k].data) throw std::invalid_argument("bad arguments");
   const CsrDev& c = ms->m[k];
-  int* d_flag = dev_alloc<int>(1);
-  CUDA_OK(cudaMemsetAsync(d_flag, 0, sizeof(int), 0));
-  csr_validate_kernel<<<he_grid(ms->r1 - ms->r0), 256>>>(c.indptr, c.indices, ms->r0, ms->r1, ms->n, c.nnz, d_flag);
+  DevPtr<int> d_flag = dev_alloc<int>(1);
+  CUDA_OK(cudaMemsetAsync(d_flag.get(), 0, sizeof(int), 0));
+  csr_validate_kernel<<<he_grid(ms->r1 - ms->r0), 256>>>(c.indptr, c.indices, ms->r0, ms->r1, ms->n, c.nnz, d_flag.get());
   g_launch_count++;
   int flag = 0;
-  CUDA_OK(cudaMemcpy(&flag, d_flag, sizeof(int), cudaMemcpyDeviceToHost));
-  dev_free(d_flag);
+  CUDA_OK(cudaMemcpy(&flag, d_flag.get(), sizeof(int), cudaMemcpyDeviceToHost));
   *flags_out = flag;
   return SLMM_OK;
   SLMM_CATCH
@@ -1169,16 +1150,15 @@ int slmm_matset_validate(slmm_matset_t* ms, int32_t k, int32_t* flags_out) {
 int slmm_device_arrays_equal_i32(const int32_t* d_a, const int32_t* d_b, int64_t count, int32_t* out) {
   SLMM_TRY
   if (!d_a || !d_b || !out || count < 0) throw std::invalid_argument("bad arguments");
-  int* d_flag = dev_alloc<int>(1);
-  CUDA_OK(cudaMemsetAsync(d_flag, 0, sizeof(int), 0));
+  DevPtr<int> d_flag = dev_alloc<int>(1);
+  CUDA_OK(cudaMemsetAsync(d_flag.get(), 0, sizeof(int), 0));
   if (count > 0) {
     const int grid = (int)std::min<int64_t>((count + 255) / 256, 148 * 16);
-    arrays_differ_kernel<<<grid, 256>>>(d_a, d_b, count, d_flag);
+    arrays_differ_kernel<<<grid, 256>>>(d_a, d_b, count, d_flag.get());
     g_launch_count++;
   }
   int flag = 1;
-  CUDA_OK(cudaMemcpy(&flag, d_flag, sizeof(int), cudaMemcpyDeviceToHost));
-  dev_free(d_flag);
+  CUDA_OK(cudaMemcpy(&flag, d_flag.get(), sizeof(int), cudaMemcpyDeviceToHost));
   *out = flag ? 0 : 1;
   return SLMM_OK;
   SLMM_CATCH
@@ -1193,14 +1173,12 @@ int slmm_matset_is_symmetric(slmm_matset_t* ms, int32_t k, int32_t* out) {
     // one streaming pass: hash sums of the entries above / below the diagonal (the test the row-block shards use; a
     // mismatch survives with probability ~2^-64).  The exact kernel (a binary search per entry: 9 ms per matrix at
     // 1M individuals, a quarter of HE()'s device-side time) is slmm_device_csr_is_symmetric.
-    unsigned long long* d = dev_alloc<unsigned long long>(2);
-    CUDA_OK(cudaMemsetAsync(d, 0, 2 * sizeof(unsigned long long), 0));
-    symmetry_hash_kernel<<<he_grid(ms->n), 256>>>(c.indptr, c.indices, c.data, 0, ms->n, d);
+    DevPtr<unsigned long long> d = dev_alloc<unsigned long long>(2);
+    CUDA_OK(cudaMemsetAsync(d.get(), 0, 2 * sizeof(unsigned long long), 0));
+    symmetry_hash_kernel<<<he_grid(ms->n), 256>>>(c.indptr, c.indices, c.data, 0, ms->n, d.get());
     g_launch_count++;
     unsigned long long h2[2] = {0, 1};
-    const cudaError_t e = cudaMemcpy(h2, d, sizeof(h2), cudaMemcpyDeviceToHost);
-    dev_free(d);
-    CUDA_OK(e);
+    CUDA_OK(cudaMemcpy(h2, d.get(), sizeof(h2), cudaMemcpyDeviceToHost));
     c.symmetric = h2[0] == h2[1] ? 1 : 0;
   }
   *out = c.symmetric;
@@ -1277,14 +1255,12 @@ int slmm_device_csr_is_symmetric(const int32_t* d_indptr, const int32_t* d_indic
                                  int32_t* out) {
   SLMM_TRY
   if (!d_indptr || !d_indices || !d_data || !out || n <= 0) throw std::invalid_argument("bad arguments");
-  int* d_flag = dev_alloc<int>(1);
-  CUDA_OK(cudaMemsetAsync(d_flag, 0, sizeof(int), 0));
-  symmetry_check_kernel<<<he_grid(n), 256>>>(d_indptr, d_indices, d_data, n, d_flag);
+  DevPtr<int> d_flag = dev_alloc<int>(1);
+  CUDA_OK(cudaMemsetAsync(d_flag.get(), 0, sizeof(int), 0));
+  symmetry_check_kernel<<<he_grid(n), 256>>>(d_indptr, d_indices, d_data, n, d_flag.get());
   g_launch_count++;
   int flag = 1;
-  const cudaError_t e = cudaMemcpy(&flag, d_flag, sizeof(int), cudaMemcpyDeviceToHost);
-  dev_free(d_flag);
-  CUDA_OK(e);
+  CUDA_OK(cudaMemcpy(&flag, d_flag.get(), sizeof(int), cudaMemcpyDeviceToHost));
   *out = flag ? 0 : 1;
   return SLMM_OK;
   SLMM_CATCH
@@ -1294,14 +1270,12 @@ int slmm_device_pattern_subset(const int32_t* d_ap, const int32_t* d_ai, const i
                                int32_t n, int32_t* out) {
   SLMM_TRY
   if (!d_ap || !d_ai || !d_bp || !d_bi || !out || n <= 0) throw std::invalid_argument("bad arguments");
-  int* d_flag = dev_alloc<int>(1);
-  CUDA_OK(cudaMemsetAsync(d_flag, 0, sizeof(int), 0));
-  pattern_subset_kernel<<<he_grid(n), 256>>>(d_ap, d_ai, d_bp, d_bi, n, d_flag);
+  DevPtr<int> d_flag = dev_alloc<int>(1);
+  CUDA_OK(cudaMemsetAsync(d_flag.get(), 0, sizeof(int), 0));
+  pattern_subset_kernel<<<he_grid(n), 256>>>(d_ap, d_ai, d_bp, d_bi, n, d_flag.get());
   g_launch_count++;
   int flag = 1;
-  const cudaError_t e = cudaMemcpy(&flag, d_flag, sizeof(int), cudaMemcpyDeviceToHost);
-  dev_free(d_flag);
-  CUDA_OK(e);
+  CUDA_OK(cudaMemcpy(&flag, d_flag.get(), sizeof(int), cudaMemcpyDeviceToHost));
   *out = flag ? 0 : 1;
   return SLMM_OK;
   SLMM_CATCH
@@ -1322,13 +1296,11 @@ int slmm_matset_symmetry_hash(slmm_matset_t* ms, int32_t k, uint64_t* h_out2) {
   SLMM_TRY
   if (!ms || k < 0 || k >= ms->K || !h_out2 || !ms->m[k].data) throw std::invalid_argument("bad arguments");
   const CsrDev& c = ms->m[k];
-  unsigned long long* d = dev_alloc<unsigned long long>(2);
-  CUDA_OK(cudaMemsetAsync(d, 0, 2 * sizeof(unsigned long long), 0));
-  symmetry_hash_kernel<<<he_grid(ms->r1 - ms->r0), 256>>>(c.indptr, c.indices, c.data, ms->r0, ms->r1, d);
+  DevPtr<unsigned long long> d = dev_alloc<unsigned long long>(2);
+  CUDA_OK(cudaMemsetAsync(d.get(), 0, 2 * sizeof(unsigned long long), 0));
+  symmetry_hash_kernel<<<he_grid(ms->r1 - ms->r0), 256>>>(c.indptr, c.indices, c.data, ms->r0, ms->r1, d.get());
   g_launch_count++;
-  const cudaError_t e = cudaMemcpy(h_out2, d, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
-  dev_free(d);
-  CUDA_OK(e);
+  CUDA_OK(cudaMemcpy(h_out2, d.get(), 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
   return SLMM_OK;
   SLMM_CATCH
 }
