@@ -190,7 +190,10 @@ int slmm_chol_factorize(slmm_chol_t* h, int32_t* fail_col);
 /* factor.logdet() (SparseCholesky.py:40) */
 int slmm_chol_logdet(slmm_chol_t* h, double* h_out);
 /* factor(b) = solve_A (SparseCholesky.py:30,32,52,100,149,153): in-place on a C-ordered n x nrhs device block,
- * original ordering.  mode 0: V^-1 b;  1: forward half only (L^-1 P b, permuted order);  2: backward half only. */
+ * original ordering.  mode 0: V^-1 b;  1: forward half only (L^-1 P b, permuted order);  2: backward half only;
+ * 3: backward half from the factor's row order (P' L^-T b: b is taken in permuted order, the result comes back in
+ * original order).  With Z in permuted order, mode 3 on Z gives V^-1 (slmm_chol_lmul of Z), the probe block of
+ * simulate_vector, without forming L Z.  Any other mode is SLMM_ERR_INVALID. */
 int slmm_chol_solve(slmm_chol_t* h, double* d_B, int32_t nrhs, int32_t mode);
 /* (factor.L().dot(Z))[argsort(P)]  (SparseCholesky.py:50-51): d_out in original ordering, C-ordered n x nrhs */
 int slmm_chol_lmul(slmm_chol_t* h, const double* d_Z, double* d_out, int32_t nrhs);

@@ -313,8 +313,8 @@ class RemlSession(object):
                 Z = self.functor.probe_source(self.n, sim_num)
             else:
                 return None
-        if torch.is_tensor(Z) and Z.is_cuda:
-            return Z[:, col_begin:col_end].contiguous(), None
+        if torch.is_tensor(Z) and Z.is_cuda:               # a copy: the probe solve works in place
+            return Z[:, col_begin:col_end].clone(memory_format=torch.contiguous_format), None
         sliced = bool(col_begin or col_end != Z.shape[1])
         if torch.is_tensor(Z) and not sliced and Z.dtype == torch.float64 and Z.is_contiguous():
             if getattr(self, "_copy_stream", None) is None:
@@ -335,16 +335,17 @@ class RemlSession(object):
 
     def probes(self, sim_num, Z=None, col_begin=0, col_end=None, pre=None, probe_stream=None):
         """W = V^-1 (L Z)[argsort P]   (reference :49-52) for the probe columns [col_begin, col_end) of the
-        n x sim_num block Z.  rng == 'device' draws ONLY those columns, from the counter-based stream keyed by
-        (functor.seed, evaluation index or probe_stream, row, global column): the same values for any number of GPUs.
-        pre: what prefetch_probes returned for the same arguments."""
+        n x sim_num block Z, computed as P' L^-T Z: with P V P' = L L', V^-1 P' L Z = P' L^-T L^-1 L Z, so one
+        backward half-sweep on Z (solve mode 3) replaces L Z and the full solve.  rng == 'device' draws ONLY those
+        columns, from the counter-based stream keyed by (functor.seed, evaluation index or probe_stream, row, global
+        column): the same values for any number of GPUs.  pre: what prefetch_probes returned for the same arguments."""
         torch = self.torch
         col_end = sim_num if col_end is None else col_end
         if pre is not None:
             Zd, ev = pre
             if ev is not None:
                 torch.cuda.current_stream().wait_event(ev)
-            return self.eng.solve_(self.eng.lmul(Zd))
+            return self.eng.solve_(Zd, mode=3)
         if Z is None:
             if self.functor.rng == 'numpy':               # the reference's global stream: the whole block is drawn
                 Z = np.random.randn(self.n, sim_num)
@@ -353,7 +354,7 @@ class RemlSession(object):
             else:
                 stream = self.n_eval if probe_stream is None else probe_stream
                 Z = self.eng.probe_normals(self.n, col_end - col_begin, col_begin, self.functor.seed, stream)
-                col_begin, col_end = 0, Z.shape[1]
+                return self.eng.solve_(Z, mode=3)
         sliced = bool(col_begin or col_end != Z.shape[1])
         if not torch.is_tensor(Z):
             Z = np.ascontiguousarray(Z, dtype=np.float64)
@@ -364,10 +365,9 @@ class RemlSession(object):
                 Z = _eng.upload_columns(Z, col_begin, col_end, torch)
             else:
                 Z = (Z[:, col_begin:col_end] if sliced else Z).contiguous().to("cuda", non_blocking=True)
-        else:
-            Z = (Z[:, col_begin:col_end] if sliced else Z).contiguous()
-        U = self.eng.lmul(Z)
-        return self.eng.solve_(U)
+        else:                                          # a copy: the caller's block is not overwritten
+            Z = Z[:, col_begin:col_end].clone(memory_format=torch.contiguous_format)
+        return self.eng.solve_(Z, mode=3)
 
     def _is_identity(self, k):
         m = self.mats_host[k]
@@ -524,12 +524,13 @@ def negative_log_likelihood(factor, y, invV_y, mu, L_CT_invV_C, reml):
 
 
 def simulate_vector(factor, n, sim_num, p_inv=None):
-    """reference :49-52: V^-1 (L Z)[argsort P] with Z from the global numpy stream; stays on the device
-    until the final copy.  p_inv is accepted for signature compatibility (the engine applies P itself)."""
+    """reference :49-52: V^-1 (L Z)[argsort P] with Z from the global numpy stream, computed as P' L^-T Z by one
+    backward half-sweep (RemlSession.probes); stays on the device until the final copy.  p_inv is accepted for
+    signature compatibility (the engine applies P itself)."""
     torch = _eng.require_cuda()
+    factor._check()
     Z = _eng.to_device(np.random.randn(n, sim_num), torch)
-    U = factor.lmul(Z)
-    return factor._chol.solve_(U).cpu().numpy()
+    return factor._chol.solve_(Z, mode=3).cpu().numpy()
 
 
 def compute_gradients(sig2g_array, mats, sim_vec, invV_y, reml, invV_C, L_CT_invV_C):
@@ -910,7 +911,7 @@ def MINQUE(cholesky_func, mat_list, cov, y, compute_stderr=False, verbose=False,
         else:
             factor = functor(H)
             Z = _eng.to_device(np.random.randn(n, sim_num), torch)
-            invH_simy = factor._chol.solve_(factor.lmul(Z))
+            invH_simy = factor._chol.solve_(Z, mode=3)       # H^-1 (L Z)[argsort P] = P' L^-T Z
             invH_y = factor._chol.solve_(y_dev.clone())
             for i in range(K):
                 q[i] = float(invH_y @ ms.spmm(i, invH_y)) - yy

@@ -1598,17 +1598,24 @@ int slmm_chol_logdet(slmm_chol_t* h, double* out) {
 int slmm_chol_solve(slmm_chol_t* h, double* d_B, int32_t nrhs, int32_t mode) {
   SLMM_TRY
   if (!h || !d_B || nrhs <= 0) throw std::invalid_argument("bad arguments");
+  if (mode < 0 || mode > 3) throw std::invalid_argument("slmm_chol_solve: mode must be 0, 1, 2 or 3");
   if (!h->factored) throw std::invalid_argument("factorize first");
   SolvePlan* pl = get_plan(h, nrhs);
   const int n = h->S.n;
   const int64_t total = (int64_t)n * nrhs;
   const int grid = (int)std::min<int64_t>((total + 255) / 256, 148 * 32);
-  // forward consumes X and leaves y in X2; backward consumes X2 and leaves x in X
-  gather_rows_kernel<<<grid, 256, 0, h->cur>>>(d_B, mode == 2 ? pl->X2.get() : pl->X.get(), h->d_perm.get(), n, nrhs, 0);
+  // forward consumes X and leaves y in X2; backward consumes X2 and leaves x in X.  Mode 3 takes B in the factor's
+  // row order, so it goes into X2 as it is.
+  if (mode == 3) {
+    CUDA_OK(cudaMemcpyAsync(pl->X2.get(), d_B, total * sizeof(double), cudaMemcpyDeviceToDevice, h->cur));
+  } else {
+    gather_rows_kernel<<<grid, 256, 0, h->cur>>>(d_B, mode == 2 ? pl->X2.get() : pl->X.get(), h->d_perm.get(), n, nrhs, 0);
+    g_launch_count++;
+  }
   if (mode == 0 || mode == 1) run_schedule(h, pl->fwd, pl->X.get(), pl->arena, pl->d_vptr.get(), nrhs);
-  if (mode == 0 || mode == 2) run_schedule(h, pl->bwd, pl->X.get(), pl->arena, pl->d_vptr.get(), nrhs);
+  if (mode != 1) run_schedule(h, pl->bwd, pl->X.get(), pl->arena, pl->d_vptr.get(), nrhs);
   gather_rows_kernel<<<grid, 256, 0, h->cur>>>(mode == 1 ? pl->X2.get() : pl->X.get(), d_B, h->d_perm.get(), n, nrhs, 1);
-  g_launch_count += 2;
+  g_launch_count++;
   CUDA_OK(cudaGetLastError());
   return SLMM_OK;
   SLMM_CATCH

@@ -523,7 +523,10 @@ class CholEngine(object):
         return v.value
 
     def solve_(self, B, mode=0):
-        """In-place V^-1 B on a contiguous CUDA float64 tensor of shape (n,) or (n, k)."""
+        """In-place V^-1 B on a contiguous CUDA float64 tensor of shape (n,) or (n, k).
+        mode 0: V^-1 B;  1: forward half only, L^-1 P B (result in the factor's row order);  2: backward half only,
+        P' L^-T P B;  3: backward half from the factor's row order, P' L^-T B.  Mode 3 on Z equals mode 0 on lmul(Z)
+        up to rounding (V^-1 P' L Z = P' L^-T Z), so it gives the probe block without L Z or the forward sweep."""
         if not B.is_contiguous():
             raise ValueError("solve_ needs a contiguous tensor")
         nrhs = 1 if B.dim() == 1 else B.shape[1]

@@ -3,7 +3,7 @@
 The path shards in exactly two places (SURVEY.md §8e); everything else is replicated:
   * REML probe / RHS columns: every rank assembles and factors V itself (inputs are replicated, recomputing
     is cheaper than broadcasting the factor), takes a contiguous slice of the sim_num probe columns through
-    L*Z, the solves and the fused SpMM reductions, and the K partial trace sums are combined with ONE
+    the backward half-sweep and the fused SpMM reductions, and the K partial trace sums are combined with ONE
     all-reduce of K doubles per evaluation.
   * HE row blocks: contiguous row ranges balanced by nonzeros; ONE all-reduce of 2K + 2K^2 doubles.
 The helpers work on CPU tensors with the gloo backend as well, which is how the host logic is tested.
