@@ -69,6 +69,11 @@ int slmm_upload_h2d(void* d_dst, const void* h_src, int64_t nbytes, int32_t thre
  * on the host.  Pinned or pageable source; returns when the copy is done. */
 int slmm_upload_h2d_2d(void* d_dst, int64_t dst_pitch, const void* h_src, int64_t src_pitch, int64_t width_bytes,
                        int64_t rows);
+/* The same two uploads issued on `stream` (a cudaStream_t; NULL = the legacy default stream) instead of the default
+ * stream: the genotype blocks of the association scan go up on a copy stream while the previous block is swept. */
+int slmm_upload_h2d_on(void* d_dst, const void* h_src, int64_t nbytes, int32_t threads, void* stream);
+int slmm_upload_h2d_2d_on(void* d_dst, int64_t dst_pitch, const void* h_src, int64_t src_pitch, int64_t width_bytes,
+                          int64_t rows, void* stream);
 int slmm_matset_nnz(const slmm_matset_t* ms, int32_t k, int64_t* out);
 int slmm_matset_values(const slmm_matset_t* ms, int32_t k, const double** d_data_out);
 
@@ -258,6 +263,22 @@ int slmm_symbolic_entry_map(const slmm_symbolic_t* s, const int32_t* h_indptr, c
                             int64_t* h_target);
 int slmm_symbolic_entry_map_tri(const slmm_symbolic_t* s, const int32_t* h_indptr, const int32_t* h_indices,
                                 int32_t tri, int64_t* h_target);
+
+/* ------------------------------------------------------------------ association scan ------------------ */
+/* Mixed-model association test of genotyped variants at fixed variance components (GCTA --mlma, EMMAX).  The
+ * reference has no counterpart: its users loop over variants with one sparse solve each.  Per block of b variants:
+ *   slmm_assoc_genotypes: int8 allele counts d_G (0, 1, 2; negative = missing) of n individuals x b variants, element
+ *     (i, j) at d_G[i*row_stride + j*col_stride] (one stride 1: C- or Fortran-ordered host blocks).  Writes the
+ *     per-variant non-missing count d_nobs[b] and allele sum d_sum[b], x~ = x - mean (0 where missing) as the
+ *     C-ordered n x b block d_X (original row order, ready for slmm_chol_solve mode 1), and d_proj[k*b + j] =
+ *     P[:,k]' x~_j for the C-ordered n x np block P = [V^-1 C | V^-1 r] (np <= 32).  Any other entry value returns
+ *     SLMM_ERR_INVALID (checked on the device; nothing faults).
+ *   slmm_assoc_colsumsq: d_out[j] = sum_i F[i,j]^2 of a C-ordered n x b block (after the forward half-sweep, F = L^-1
+ *     P x~, so d_out[j] = x~_j' V^-1 x~_j; any row order).
+ * Reductions run over fixed row chunks: a variant's results do not depend on b or on the memory order. */
+int slmm_assoc_genotypes(const int8_t* d_G, int64_t n, int32_t b, int64_t row_stride, int64_t col_stride,
+                         const double* d_P, int32_t np, double* d_X, double* d_proj, int64_t* d_nobs, int64_t* d_sum);
+int slmm_assoc_colsumsq(const double* d_F, int64_t n, int32_t b, double* d_out);
 
 /* ------------------------------------------------------------------ IBD matrix construction ----------- */
 /* The step before the path (SURVEY 8f-1): numerator relationship matrix from a child -> parents matrix, replacing

@@ -19,6 +19,7 @@ import numpy as np
 import scipy.linalg as la
 import scipy.optimize as optimize
 import scipy.sparse as sparse
+import scipy.special as special
 
 from . import engine as _eng
 from . import sharding as _shard
@@ -368,6 +369,110 @@ class RemlSession(object):
         else:                                          # a copy: the caller's block is not overwritten
             Z = Z[:, col_begin:col_end].clone(memory_format=torch.contiguous_format)
         return self.eng.solve_(Z, mode=3)
+
+    def association(self, sigmas, G, block, col_begin=0, col_end=None, timing=None):
+        """Mixed-model association test of the variants (columns) [col_begin, col_end) of the host (n, m) int8 genotype
+        matrix G at the variance components `sigmas` (see association() for the statistic), in blocks of `block`
+        variants.  Per block: int8 upload on a copy stream (the next block goes up while this one is swept), one
+        decode / centre / project kernel, one forward half-sweep F = L^-1 P x~ (solve mode 1), one column sum of
+        squares, and the c x c finalisation on the host.  Returns a dict of arrays of length col_end - col_begin in the
+        units of the standardised y: beta, se, chi2, p, af, n_obs.  timing: a list that receives, per block, five
+        timing events recorded on the compute stream around the upload wait, the genotype kernel, the sweep and the
+        sum of squares (scripts/assoc_scan.py)."""
+        torch = self.torch
+        n = self.n
+        if self.C.shape[1] > ASSOC_MAX_COVARIATES:
+            raise ValueError("the association scan takes at most %d covariates, got %d"
+                             % (ASSOC_MAX_COVARIATES, self.C.shape[1]))
+        col_end = G.shape[1] if col_end is None else int(col_end)
+        m_loc = max(col_end - col_begin, 0)
+        out = {k: np.full(m_loc, np.nan) for k in ("beta", "se", "chi2", "p", "af")}
+        out["n_obs"] = np.zeros(m_loc, dtype=np.int64)
+        if m_loc == 0:
+            return out
+        self.factor_at(sigmas)
+        ViC, chol, beta, Viy = self.fixed_effects()
+        Vir = Viy - ViC @ torch.from_numpy(beta).to("cuda")
+        P = torch.cat([ViC, Vir.unsqueeze(1)], dim=1).contiguous()       # n x (c + 1)
+        c1 = P.shape[1]
+        block = max(1, min(int(block), m_loc))
+        starts = list(range(col_begin, col_end, block))
+        # one int8 buffer: the upload of block i + 1 is issued after assoc_genotypes has returned for block i, and that
+        # call waits for its kernels (device-side input check), so nothing still reads the buffer
+        g8 = torch.empty(n * block, dtype=torch.int8, device="cuda")
+        X = torch.empty(n * block, dtype=torch.float64, device="cuda")
+        small = [dict(proj=torch.empty(c1 * block, dtype=torch.float64, device="cuda"),
+                      nobs=torch.empty(block, dtype=torch.int64, device="cuda"),
+                      gsum=torch.empty(block, dtype=torch.int64, device="cuda"),
+                      ss=torch.empty(block, dtype=torch.float64, device="cuda")) for _ in range(2)]
+        if getattr(self, "_copy_stream", None) is None:
+            self._copy_stream = torch.cuda.Stream()
+        copy, main = self._copy_stream, torch.cuda.current_stream()
+        uploaded = torch.cuda.Event()
+        strides = [None]
+
+        def upload(i):
+            j0 = starts[i]
+            strides[0] = _eng.upload_genotype_block(G, j0, min(j0 + block, col_end), g8, copy)
+            uploaded.record(copy)
+
+        def finish(i):
+            """Statistics of block i, whose kernels have completed.  The small outputs come back on the copy stream, so
+            the host does not wait behind the sweep of block i + 1 queued on the compute stream."""
+            j0 = starts[i]
+            w = min(j0 + block, col_end) - j0
+            s = small[i % 2]
+            with torch.cuda.stream(copy):
+                proj = s["proj"][:c1 * w].view(c1, w).cpu().numpy()
+                ss = s["ss"][:w].cpu().numpy()
+                nobs, gsum = s["nobs"][:w].cpu().numpy(), s["gsum"][:w].cpu().numpy()
+            q, t = proj[:c1 - 1], proj[c1 - 1]
+            xPx = ss - np.sum(q * la.cho_solve(chol, q), axis=0)
+            ok = xPx > 1e-10 * ss                      # monomorphic (ss = 0) or in the span of C: NaN
+            sl = slice(j0 - col_begin, j0 - col_begin + w)
+            with np.errstate(invalid="ignore", divide="ignore"):
+                xPx = np.where(ok, xPx, np.nan)
+                out["beta"][sl] = t / xPx
+                out["se"][sl] = 1.0 / np.sqrt(xPx)
+                out["chi2"][sl] = t * t / xPx
+                out["p"][sl] = special.chdtrc(1, out["chi2"][sl])
+                out["af"][sl] = gsum / nobs / 2.0
+            out["n_obs"][sl] = nobs
+
+        def mark(marks):
+            if marks is not None:
+                marks.append(torch.cuda.Event(enable_timing=True))
+                marks[-1].record(main)
+
+        upload(0)
+        try:
+            for i, j0 in enumerate(starts):
+                w = min(j0 + block, col_end) - j0
+                s = small[i % 2]
+                Xb = X[:n * w].view(n, w)
+                marks = None if timing is None else []
+                mark(marks)
+                main.wait_event(uploaded)
+                mark(marks)
+                # returns once the kernels are done (device-side input check): block i - 1 is swept and reduced by then
+                _eng.assoc_genotypes(g8, n, w, strides[0], P, Xb, s["proj"], s["nobs"], s["gsum"])
+                mark(marks)
+                self.eng.solve_(Xb, mode=1)
+                mark(marks)
+                _eng.assoc_colsumsq(Xb, s["ss"])
+                mark(marks)
+                if timing is not None:
+                    timing.append(marks)
+                # while the device sweeps block i: statistics of block i - 1, then the host stages block i + 1
+                if i > 0:
+                    finish(i - 1)
+                if i + 1 < len(starts):
+                    upload(i + 1)
+            main.synchronize()
+            finish(len(starts) - 1)
+        finally:
+            torch.cuda.synchronize()                   # no copy may still target the buffers when they are freed
+        return out
 
     def _is_identity(self, k):
         m = self.mats_host[k]
@@ -756,6 +861,78 @@ def REML(cholesky_func, mats, covariates, y, reml=True, sim_num=100, verbose=Fal
     if aireml:
         out["aireml"] = ai_info
     return out
+
+
+# ------------------------------------------------------------------------------------------- association scan
+ASSOC_BLOCK = 512         # variants per block of the public scan: the fastest width measured (DESIGN.md 6c)
+ASSOC_MAX_COVARIATES = 31   # [V^-1 C | V^-1 r] is projected in registers, c + 1 <= 32 (csrc/assoc.cu)
+# device bytes a block holds per (individual, variant): x~, the solve plan of its width, int8 and small buffers.  Measured
+# 40.7 / 41.9 / 49.3 at widths 512 / 256 / 128 (profiles/r05_assoc_scan.json).  The width is chosen so that these fit
+# in half the free memory; the other half covers the plan of a narrower tail block, which is no larger.
+ASSOC_BYTES_PER_ENTRY = 50
+
+
+def _scan_session(functor, mats, covariates, y):
+    """The session REML() left for the same inputs, or a new one.  REML() appends its own identity and divides y by
+    its std into a new array, so those two are matched by content; the caller's matrices and covariates by the
+    session key (object and content fingerprint)."""
+    for ses in list(functor._sessions.values()):
+        m_s, _, y_s = ses._refs
+        if len(m_s) == len(mats) + 1 and ses._ident[-1] and m_s[-1].shape[0] == y.shape[0] \
+                and np.array_equal(y_s, y):
+            return functor._session(list(mats) + [m_s[-1]], covariates, y_s)
+    return functor._session(list(mats) + [sparse.eye(y.shape[0]).tocsr()], covariates, y)
+
+
+def association(cholesky_func, mats, covariates, y, sigmas, G):
+    """Mixed-model association scan (GCTA --mlma, EMMAX) of the variants in G at the variance components `sigmas`.
+
+    Arguments as for REML(): `mats` without the identity, `sigmas` = REML()['covariance coefficients'] (K + 1 values,
+    the residual last); V = sum_k sigma_k A_k + sigma_e I on y / y.std().  At most 31 covariates (columns of C).  A call after REML() on the same functor
+    reuses its device session.  G: (n, m) int8 ndarray in C or Fortran order, rows in y's order, entries 0 / 1 / 2
+    allele counts and negative values for missing (any other value raises SlmmError).
+
+    Per variant x: mean imputation and centring (x~), q = (V^-1 C)' x~, t = (V^-1 r)' x~ with r = y - C beta,
+    xPx = x~'V^-1 x~ - q' (C'V^-1 C)^-1 q, beta = t / xPx, se = xPx^-1/2, chi2 = t^2 / xPx, p its chi^2_1 survival
+    function: the coefficient of x~ and its standard error in the GLS fit of [C | x~] under the same V.  beta and se
+    are in the units of y.  Monomorphic variants and those in the span of C (xPx <= 1e-10 x~'V^-1 x~) get NaN.
+
+    Returns a dict of length-m arrays: beta, se, chi2, p, af (allele frequency of the non-missing entries), n_obs.
+    With torch.distributed initialised every rank scans a contiguous slice of the variants and one all-reduce gives
+    every rank the whole result."""
+    functor = _need_functor(cholesky_func)
+    torch = _eng.require_cuda()
+    G = np.asarray(G)
+    if G.ndim != 2 or G.dtype != np.int8:
+        raise ValueError("G must be a 2-D int8 array of allele counts (negative = missing)")
+    if G.shape[0] != y.shape[0]:
+        raise ValueError("G has %d rows for %d individuals" % (G.shape[0], y.shape[0]))
+    if not (G.flags.c_contiguous or G.flags.f_contiguous):
+        G = np.ascontiguousarray(G)
+    if np.shape(covariates)[1] > ASSOC_MAX_COVARIATES:
+        raise ValueError("the association scan takes at most %d covariates, got %d"
+                         % (ASSOC_MAX_COVARIATES, np.shape(covariates)[1]))
+    sigmas = np.asarray(sigmas, dtype=float)
+    if sigmas.shape != (len(mats) + 1,):
+        raise ValueError("need %d variance components (the residual last), got %d" % (len(mats) + 1, sigmas.size))
+    scale = y.std()
+    ses = _scan_session(functor, mats, covariates, y / scale)
+    n, m = G.shape
+    free = torch.cuda.mem_get_info()[0]
+    block = int(max(8, min(ASSOC_BLOCK, free // 2 // (ASSOC_BYTES_PER_ENTRY * n))))
+    rank, world = _shard.rank_world()
+    lo, hi = _shard.column_block(m, rank, world)
+    part = ses.association(sigmas, G, block, lo, hi)
+    keys = ("beta", "se", "chi2", "p", "af", "n_obs")
+    if world > 1:
+        full = torch.zeros(len(keys), m, dtype=torch.float64, device="cuda")
+        full[:, lo:hi] = torch.from_numpy(np.stack([part[k].astype(np.float64) for k in keys]))
+        full = _shard.allreduce_sum_(full).cpu().numpy()
+        part = {k: full[i] for i, k in enumerate(keys)}
+        part["n_obs"] = part["n_obs"].astype(np.int64)
+    part["beta"] = part["beta"] * scale
+    part["se"] = part["se"] * scale
+    return {k: part[k] for k in keys}
 
 
 # ------------------------------------------------------------------------------------------- Haseman-Elston

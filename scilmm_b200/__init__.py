@@ -3,7 +3,7 @@
 Mirrors the reference package facade (scilmm/__init__.py:1-2 star-imports SparseCholesky), so
 `from scilmm_b200 import HE, REML, SparseCholesky, run_estimates` works like `from scilmm import ...`.
 """
-from .SparseCholesky import (HE, MINQUE, REML, B200Factor, NotPositiveDefiniteError, SlmmError,  # noqa: F401
+from .SparseCholesky import (HE, MINQUE, REML, B200Factor, association, NotPositiveDefiniteError, SlmmError,  # noqa: F401
                              SparseCholesky, bolt_gradient_estimation, compute_gradients, compute_hess,
                              compute_varcomp_stderr, estimate_fixed_effects, estimate_var_comps,
                              matrices_weighted_sum, negative_log_likelihood, run_estimates,

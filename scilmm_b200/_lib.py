@@ -46,6 +46,10 @@ SIGNATURES = {
     "slmm_matset_set_symmetric": (C.c_int, [vp, i32, i32]),
     "slmm_upload_h2d": (C.c_int, [vp, vp, i64, i32]),
     "slmm_upload_h2d_2d": (C.c_int, [vp, i64, vp, i64, i64, i64]),
+    "slmm_upload_h2d_on": (C.c_int, [vp, vp, i64, i32, vp]),
+    "slmm_upload_h2d_2d_on": (C.c_int, [vp, i64, vp, i64, i64, i64, vp]),
+    "slmm_assoc_genotypes": (C.c_int, [vp, i64, i32, i64, i64, vp, i32, vp, vp, vp, vp]),
+    "slmm_assoc_colsumsq": (C.c_int, [vp, i64, i32, vp]),
     "slmm_matset_nnz": (C.c_int, [vp, i32, C.POINTER(i64)]),
     "slmm_matset_values": (C.c_int, [vp, i32, pp]),
     "slmm_he_moments": (C.c_int, [vp, vp, i32, i32, vp]),

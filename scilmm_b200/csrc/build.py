@@ -9,7 +9,7 @@ LIB = os.path.join(PKG, "libscilmm_b200.so")
 CUDA_HOME = os.environ.get("CUDA_HOME", "/usr/local/cuda")
 NVCC = os.path.join(CUDA_HOME, "bin", "nvcc")
 METIS = os.path.join(CUDA_HOME, "lib64", "libmetis_static.a")
-SOURCES_CU = ["chol.cu", "sparse_ops.cu", "ibd.cu", "quadform_tiled.cu"]
+SOURCES_CU = ["chol.cu", "sparse_ops.cu", "ibd.cu", "quadform_tiled.cu", "assoc.cu"]
 SOURCES_CPP = ["symbolic.cpp"]
 HEADERS = ["common.h", "dense_tiles.cuh", "potrf_block.cuh", "symbolic.h", "skinny_ops.cuh", "matset.h", "dense_tiles_tma.cuh"]
 

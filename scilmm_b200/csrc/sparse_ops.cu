@@ -1347,11 +1347,16 @@ Stager g_stager;
 }  // namespace
 
 int slmm_upload_h2d(void* d_dst, const void* h_src, int64_t nbytes, int32_t threads) {
+  return slmm_upload_h2d_on(d_dst, h_src, nbytes, threads, nullptr);
+}
+
+int slmm_upload_h2d_on(void* d_dst, const void* h_src, int64_t nbytes, int32_t threads, void* stream) {
   SLMM_TRY
   if (!d_dst || !h_src || nbytes < 0) throw std::invalid_argument("bad arguments");
   if (nbytes == 0) return SLMM_OK;
+  cudaStream_t on = (cudaStream_t)stream;
   if (nbytes < (int64_t)(4 << 20)) {            // small arrays: the driver's own staging is as good
-    CUDA_OK(cudaMemcpyAsync(d_dst, h_src, (size_t)nbytes, cudaMemcpyHostToDevice, 0));
+    CUDA_OK(cudaMemcpyAsync(d_dst, h_src, (size_t)nbytes, cudaMemcpyHostToDevice, on));
     return SLMM_OK;
   }
   Stager& S = g_stager;
@@ -1359,8 +1364,8 @@ int slmm_upload_h2d(void* d_dst, const void* h_src, int64_t nbytes, int32_t thre
   S.init(T);
   const int64_t nchunks = (nbytes + (int64_t)Stager::CHUNK - 1) / (int64_t)Stager::CHUNK;
   int dev = S.device;
-  // the destination may be recycled memory with work still queued on the default stream
-  CUDA_OK(cudaEventRecord(S.ev_in, 0));
+  // the destination may be recycled memory with work still queued on the calling stream
+  CUDA_OK(cudaEventRecord(S.ev_in, on));
   CUDA_OK(cudaStreamWaitEvent(S.st, S.ev_in, 0));
   std::vector<cudaError_t> err(T, cudaSuccess);
   auto work = [&](int t) {
@@ -1383,7 +1388,7 @@ int slmm_upload_h2d(void* d_dst, const void* h_src, int64_t nbytes, int32_t thre
   for (auto& th : pool) th.join();
   for (int t = 0; t < T; t++) CUDA_OK(err[t]);
   CUDA_OK(cudaEventRecord(S.ev_out, S.st));
-  CUDA_OK(cudaStreamWaitEvent(0, S.ev_out, 0));
+  CUDA_OK(cudaStreamWaitEvent(on, S.ev_out, 0));
   // the staging buffers are reused by the next call: its first writes must not overtake this call's last DMAs
   CUDA_OK(cudaEventSynchronize(S.ev_out));
   return SLMM_OK;
@@ -1392,14 +1397,20 @@ int slmm_upload_h2d(void* d_dst, const void* h_src, int64_t nbytes, int32_t thre
 
 int slmm_upload_h2d_2d(void* d_dst, int64_t dst_pitch, const void* h_src, int64_t src_pitch, int64_t width_bytes,
                        int64_t rows) {
+  return slmm_upload_h2d_2d_on(d_dst, dst_pitch, h_src, src_pitch, width_bytes, rows, nullptr);
+}
+
+int slmm_upload_h2d_2d_on(void* d_dst, int64_t dst_pitch, const void* h_src, int64_t src_pitch, int64_t width_bytes,
+                          int64_t rows, void* stream) {
   SLMM_TRY
+  cudaStream_t on = (cudaStream_t)stream;
   if (!d_dst || !h_src || width_bytes < 0 || rows < 0 || dst_pitch < width_bytes || src_pitch < width_bytes)
     throw std::invalid_argument("bad arguments");
   if (width_bytes == 0 || rows == 0) return SLMM_OK;
   // the DMA engine walks the pitched source: no host-side packing of the column slice
   CUDA_OK(cudaMemcpy2DAsync(d_dst, (size_t)dst_pitch, h_src, (size_t)src_pitch, (size_t)width_bytes, (size_t)rows,
-                            cudaMemcpyHostToDevice, 0));
-  CUDA_OK(cudaStreamSynchronize(0));            // the host block may be reused by the caller right away
+                            cudaMemcpyHostToDevice, on));
+  CUDA_OK(cudaStreamSynchronize(on));           // the host block may be reused by the caller right away
   return SLMM_OK;
   SLMM_CATCH
 }

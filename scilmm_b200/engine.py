@@ -66,25 +66,59 @@ def to_device(a, torch=None):
     return out
 
 
-def upload_columns(Z, col_begin, col_end, torch=None):
-    """Columns [col_begin, col_end) of a C-ordered host float64 block (ndarray or CPU tensor, pinned or not) as a
-    contiguous CUDA tensor: one pitched DMA, no host-side packing of the slice (slmm_upload_h2d_2d)."""
+def upload_columns(Z, col_begin, col_end, torch=None, out=None, stream=None):
+    """Columns [col_begin, col_end) of a C-ordered host float64 block (ndarray or CPU tensor, pinned or not) or int8
+    genotype ndarray as a contiguous CUDA tensor: one pitched DMA, no host-side packing of the slice
+    (slmm_upload_h2d_2d).  out: a device buffer of at least n * width elements of that dtype to fill instead of a new
+    tensor; stream: a torch CUDA stream to issue the copy on instead of the default stream."""
     torch = torch or require_cuda()
     n, s = int(Z.shape[0]), int(Z.shape[1])
     if torch.is_tensor(Z):
         if Z.dtype != torch.float64 or not Z.is_contiguous() or Z.is_cuda:
             raise ValueError("upload_columns needs a contiguous float64 host block")
-        src, itemsize = Z.data_ptr(), 8
+        src, itemsize, dtype = Z.data_ptr(), 8, torch.float64
     else:
-        if Z.dtype != np.float64 or not Z.flags.c_contiguous:
-            raise ValueError("upload_columns needs a C-ordered float64 host block")
-        src, itemsize = Z.ctypes.data, 8
+        if Z.dtype not in (np.float64, np.int8) or not Z.flags.c_contiguous:
+            raise ValueError("upload_columns needs a C-ordered float64 or int8 host block")
+        src, itemsize = Z.ctypes.data, Z.itemsize
+        dtype = torch.float64 if Z.dtype == np.float64 else torch.int8
     w = int(col_end) - int(col_begin)
-    out = torch.empty(n, w, dtype=torch.float64, device="cuda")
+    out = torch.empty(n, w, dtype=dtype, device="cuda") if out is None else out[:n * max(w, 0)].view(n, max(w, 0))
     if n == 0 or w <= 0:
         return out
-    check(lib().slmm_upload_h2d_2d(out.data_ptr(), w * itemsize, src + int(col_begin) * itemsize, s * itemsize,
-                                   w * itemsize, n))
+    check(lib().slmm_upload_h2d_2d_on(out.data_ptr(), w * itemsize, src + int(col_begin) * itemsize, s * itemsize,
+                                      w * itemsize, n, None if stream is None else stream.cuda_stream))
+    return out
+
+
+def upload_genotype_block(G, col_begin, col_end, out, stream=None):
+    """Columns [col_begin, col_end) of a host (n, m) int8 genotype matrix into the flat device int8 buffer `out` (at
+    least n * width entries) on `stream`.  Returns (row_stride, col_stride) of the block in `out`: a C-ordered matrix
+    goes up as n rows of width bytes by one pitched DMA (strides (width, 1)); in a Fortran-ordered one the columns are
+    one contiguous span, staged through the ring of pinned buffers (strides (1, n))."""
+    n, w = int(G.shape[0]), int(col_end) - int(col_begin)
+    if G.flags.c_contiguous:
+        upload_columns(G, col_begin, col_end, out=out, stream=stream)
+        return w, 1
+    if not G.flags.f_contiguous or G.dtype != np.int8:
+        raise ValueError("upload_genotype_block needs a C- or Fortran-ordered int8 host matrix")
+    check(lib().slmm_upload_h2d_on(out.data_ptr(), G.ctypes.data + int(col_begin) * n, n * w, int(UPLOAD_THREADS),
+                                   None if stream is None else stream.cuda_stream))
+    return 1, n
+
+
+def assoc_genotypes(Gd, n, width, strides, P, X, proj, nobs, gsum):
+    """Association scan, device side of one genotype block (slmm_assoc_genotypes): decodes the int8 block Gd (element
+    (i, j) at i * strides[0] + j * strides[1]) into X = centred allele counts (n x width, missing = 0), nobs / gsum =
+    per-variant non-missing counts and allele sums (int64), proj = P' X for P = [V^-1 C | V^-1 r] (np x width).  An
+    entry outside {0, 1, 2, negative} raises SlmmError."""
+    check(lib().slmm_assoc_genotypes(Gd.data_ptr(), int(n), int(width), int(strides[0]), int(strides[1]), P.data_ptr(),
+                                     int(P.shape[1]), X.data_ptr(), proj.data_ptr(), nobs.data_ptr(), gsum.data_ptr()))
+
+
+def assoc_colsumsq(F, out):
+    """out[j] = sum_i F[i, j]^2 of a contiguous n x width CUDA float64 block (slmm_assoc_colsumsq)."""
+    check(lib().slmm_assoc_colsumsq(F.data_ptr(), int(F.shape[0]), int(F.shape[1]), out.data_ptr()))
     return out
 
 
