@@ -251,19 +251,27 @@ __global__ void logdet_kernel(const double* __restrict__ Lx, const int32_t* __re
 
 // ---------------------------------------------------------------------------------------------------------
 struct Launch {
-  // EV_RECORD / EV_WAIT carry no kernel: `count` is an event id, recorded on / awaited by the launch's stream
+  // EV_RECORD / EV_WAIT carry no kernel: the launch's stream records / waits for event event()
   enum Kind { POTRF, GEMM_BIG, GEMM_SMALL, PULL_MAT, PULL_VEC, PULL_MAT_BIG, INIT_W, REDUCE, EV_RECORD, EV_WAIT,
-              SKINNY_F1, SKINNY_F2 /* narrow-RHS streaming kernels; child_parity holds the row template MT */,
+              SKINNY_F1, SKINNY_F2 /* narrow-RHS streaming kernels */,
               GEMM_TMA /* 128 x 128 DMMA tiles with TMA-staged operands (dense_tiles_tma.cuh); aux_off = first tensor map */ } kind;
   int64_t off;      // offset into the matching op array
-  int32_t count;    // ops / items
+  int32_t count;    // ops / items; the event id of EV_RECORD / EV_WAIT
   int32_t grid;     // CTAs
-  int32_t child_parity;
+  int32_t variant;  // PULL_*: parity of the children's arena;  SKINNY_*: row template MT
   double flops;     // dense flops issued by this launch (0 for pulls)
   int64_t tile_off; // GEMM launches: offset of this launch's tile -> op table
   int32_t stream;   // 0: main (high priority) stream   1: bulk stream (look-ahead trailing updates)
   int64_t aux_off = 0;
+  int event() const { return count; }
+  int child_parity() const { return variant; }
+  int row_mt() const { return variant; }
 };
+
+// work size the profiles report per launch: tiles / blocks of the GEMM-type kernels, ops / items of the others
+static int32_t work_size(const Launch& L) {
+  return (L.kind <= Launch::GEMM_SMALL || L.kind >= Launch::SKINNY_F1) ? L.grid : L.count;
+}
 
 // cuTensorMapEncodeTiled through the runtime's driver entry point (the library does not link libcuda: it must load
 // on machines without a driver for the host-only analysis).  2-D FP64 tensor: dim 0 = rows (contiguous), dim 1 = k
@@ -318,10 +326,20 @@ struct Schedule {
   DevPtr<PotrfOp> d_potrf;
   DevPtr<PullItem> d_pull;
   double flops = 0;
-  // CUDA graphs of this launch list (built lazily on first use; every kernel argument is fixed per schedule):
-  // [0] the look-ahead variant on the priority + bulk stream pair, [1] the serial variant (one stream)
-  GraphExec gexec[2];
+  // CUDA graph of the serial walk of this launch list (built lazily on first use; every kernel argument is fixed
+  // per schedule)
+  GraphExec gexec;
   bool graph_failed = false;
+  Launch& add(Launch::Kind kind, int64_t off, int32_t count, int32_t grid, double flops, int stream) {
+    launches.push_back(Launch{kind, off, count, grid, 0, flops, 0, stream});
+    return launches.back();
+  }
+  int record(int stream) {
+    const int ev = nevents++;
+    add(Launch::EV_RECORD, 0, ev, 0, 0.0, stream);
+    return ev;
+  }
+  void wait(int ev, int stream) { add(Launch::EV_WAIT, 0, ev, 0, 0.0, stream); }
   void upload() {
     if (ws_size > 0 || ws2_size > 0) {              // patch workspace offsets into pointers
       d_ws = dev_alloc<double>(ws_size);
@@ -461,37 +479,44 @@ struct PhaseBuilder {
     }
     push(op, small_tiles);
   }
+  static double op_flops(const GemmOp& op) {
+    if (op.flags & GF_LOWER) {       // entries on/below the diagonal of an M x N region (M >= N)
+      const double nn = std::min(op.M, op.N);
+      return 2.0 * op.K * ((double)op.M * op.N - nn * (nn - 1) / 2.0);
+    }
+    if (op.flags & GF_TRIL_B) return (double)op.M * op.N * op.K;      // about half of K per output column
+    return 2.0 * op.M * op.N * op.K;
+  }
   void flush(Schedule& sch, int stream = 0) {
-    const size_t first_launch = sch.launches.size();
     if (!potrf.empty()) {
       double pf = 0;
       for (const PotrfOp& o : potrf) pf += 2.0 * o.nb * o.nb * o.nb / 3.0;
-      sch.launches.push_back({Launch::POTRF, (int64_t)sch.potrf.size(), (int32_t)potrf.size(), (int32_t)potrf.size(), 0, pf});
+      sch.add(Launch::POTRF, (int64_t)sch.potrf.size(), (int32_t)potrf.size(), (int32_t)potrf.size(), pf, stream);
       sch.potrf.insert(sch.potrf.end(), potrf.begin(), potrf.end());
     }
-    for (int pass = 0; pass < 3; pass++) {
-      std::vector<GemmOp>& v = pass == 0 ? tma : pass == 1 ? big : small;
+    // one launch per op list; a tile is tm x tn outputs.  The streaming kernels take all M <= skinny_mt rows of a block
+    // of output columns in one CTA.
+    const struct { std::vector<GemmOp>& ops; Launch::Kind kind; int tm, tn; } lists[] = {
+        {tma, Launch::GEMM_TMA, 128, 128}, {big, Launch::GEMM_BIG, 128, 128}, {small, Launch::GEMM_SMALL, 64, 64},
+        {sk1, Launch::SKINNY_F1, skinny_mt, SK_F1_COLS}, {sk2, Launch::SKINNY_F2, skinny_mt, SK_F2_COLS}};
+    for (const auto& l : lists) {
+      std::vector<GemmOp>& v = l.ops;
       if (v.empty()) continue;
-      const int T = pass == 2 ? 64 : 128;
+      const bool is_tma = l.kind == Launch::GEMM_TMA;
       int64_t tiles = 0;
       double lf = 0;
       for (GemmOp& op : v) {
         int em = 0, en = 0;
-        if (pass == 0) {      // TMA operands that start on an odd element: map based one element early, tile grid shifted
+        if (is_tma) {      // TMA operands that start on an odd element: map based one element early, tile grid shifted
           em = (int)(((uintptr_t)op.A >> 3) & 1);
           en = (int)(((uintptr_t)op.B >> 3) & 1);
           op.pad = em | (en << 1);
         }
-        op.tiles_m = (op.M + em + T - 1) / T;
-        op.tiles_n = (op.N + en + T - 1) / T;
+        op.tiles_m = (op.M + em + l.tm - 1) / l.tm;
+        op.tiles_n = (op.N + en + l.tn - 1) / l.tn;
         op.tile_start = (int32_t)tiles;
         tiles += (int64_t)op.tiles_m * op.tiles_n;
-        double f = 2.0 * op.M * op.N * op.K;
-        if (op.flags & GF_TRIL_B) f = (double)op.M * op.N * op.K;      // about half of K per output column
-        if (op.flags & GF_LOWER) {       // entries on/below the diagonal of an M x N region (M >= N)
-          const double nn = std::min(op.M, op.N);
-          f = 2.0 * op.K * ((double)op.M * op.N - nn * (nn - 1) / 2.0);
-        }
+        const double f = op_flops(op);
         sch.flops += f;
         lf += f;
       }
@@ -501,7 +526,7 @@ struct PhaseBuilder {
       for (size_t q = 0; q < v.size(); q++)
         std::fill(sch.tile_op.begin() + tile_off + v[q].tile_start,
                   sch.tile_op.begin() + tile_off + v[q].tile_start + (int64_t)v[q].tiles_m * v[q].tiles_n, (int32_t)q);
-      if (pass == 0) {
+      if (is_tma) {
         // tensor maps of the two operands: base rounded down to 16 bytes (op.pad bit 0 / 1 = the operand starts one
         // element after its map's base), extents = the op's own M / N x K so that ragged edges are zero-filled
         for (GemmOp& op : v) {
@@ -510,35 +535,10 @@ struct PhaseBuilder {
           sch.tmaps.push_back(encode_tmap(op.B - sb, (uint64_t)op.N + sb, (uint64_t)op.K, (uint64_t)op.b_sk));
         }
       }
-      Launch L{pass == 0 ? Launch::GEMM_TMA : pass == 1 ? Launch::GEMM_BIG : Launch::GEMM_SMALL, (int64_t)sch.gemm.size(),
-               (int32_t)v.size(), (int32_t)tiles, 0, lf, tile_off};
-      if (pass == 0) L.aux_off = (int64_t)sch.tmaps.size() - 2 * (int64_t)v.size();
-      sch.launches.push_back(L);
-      sch.gemm.insert(sch.gemm.end(), v.begin(), v.end());
-    }
-    for (int pass = 0; pass < 2; pass++) {      // narrow-RHS streaming flavours: one CTA per block of output columns
-      std::vector<GemmOp>& v = pass == 0 ? sk1 : sk2;
-      if (v.empty()) continue;
-      const int T = pass == 0 ? SK_F1_COLS : SK_F2_COLS;
-      int64_t tiles = 0;
-      double lf = 0;
-      for (GemmOp& op : v) {
-        op.tiles_m = 1;
-        op.tiles_n = (op.N + T - 1) / T;
-        op.tile_start = (int32_t)tiles;
-        tiles += op.tiles_n;
-        const double f = (op.flags & GF_TRIL_B) ? (double)op.M * op.N * op.K : 2.0 * op.M * op.N * op.K;
-        sch.flops += f;
-        lf += f;
-      }
-      if (tiles > 2000000000LL) throw std::runtime_error("too many tiles in one phase");
-      const int64_t tile_off = (int64_t)sch.tile_op.size();
-      sch.tile_op.resize(tile_off + tiles);
-      for (size_t q = 0; q < v.size(); q++)
-        std::fill(sch.tile_op.begin() + tile_off + v[q].tile_start,
-                  sch.tile_op.begin() + tile_off + v[q].tile_start + v[q].tiles_n, (int32_t)q);
-      sch.launches.push_back({pass == 0 ? Launch::SKINNY_F1 : Launch::SKINNY_F2, (int64_t)sch.gemm.size(),
-                              (int32_t)v.size(), (int32_t)tiles, skinny_mt, lf, tile_off});
+      Launch& L = sch.add(l.kind, (int64_t)sch.gemm.size(), (int32_t)v.size(), (int32_t)tiles, lf, stream);
+      L.tile_off = tile_off;
+      if (is_tma) L.aux_off = (int64_t)sch.tmaps.size() - 2 * (int64_t)v.size();
+      if (l.kind == Launch::SKINNY_F1 || l.kind == Launch::SKINNY_F2) L.variant = skinny_mt;
       sch.gemm.insert(sch.gemm.end(), v.begin(), v.end());
     }
     if (!reduces.empty()) {
@@ -547,11 +547,10 @@ struct PhaseBuilder {
         r.block_start = (int32_t)blocks;
         blocks += ((int64_t)r.M * r.N + 255) / 256;
       }
-      sch.launches.push_back({Launch::REDUCE, (int64_t)sch.reduce.size(), (int32_t)reduces.size(), (int32_t)blocks, 0, 0.0});
+      sch.add(Launch::REDUCE, (int64_t)sch.reduce.size(), (int32_t)reduces.size(), (int32_t)blocks, 0.0, stream);
       sch.reduce.insert(sch.reduce.end(), reduces.begin(), reduces.end());
       if (ws_id) sch.ws2_size = std::max(sch.ws2_size, ws_used); else sch.ws_size = std::max(sch.ws_size, ws_used);
     }
-    for (size_t q = first_launch; q < sch.launches.size(); q++) sch.launches[q].stream = stream;
     big.clear(); small.clear(); tma.clear(); sk1.clear(); sk2.clear(); potrf.clear(); reduces.clear();
     ws_used = 0;
   }
@@ -614,7 +613,8 @@ struct slmm_chol {
   bool factored = false;
   bool profiling = false;
   bool timeline = false;               // events of the two-stream schedules carry timestamps (eager issue, no graphs)
-  std::vector<Event> tl_events;        // timed twins of `events` + [0] = fork
+  Event tl_fork, tl_join;              // timed twins of ev_fork / ev_join
+  std::vector<Event> tl_events;        // timed twins of `events`
   std::vector<Event> tl_launch;        // one timed event after every kernel of the schedule
   int tl_count = 0;
   double prof_ms[16] = {};
@@ -670,16 +670,16 @@ static void launch_one(slmm_chol* h, const Schedule& sch, const Launch& L, const
       break;
     case Launch::PULL_MAT:
       extend_add_kernel<32><<<(L.count + 3) / 4, 128, 0, st>>>(sch.d_pull.get() + L.off, L.count, sch.d_pull_entries.get(), ds, h->Lx.get(),
-                                                               h->arena[L.child_parity].get(), h->arena[L.child_parity ^ 1].get());
+                                                               h->arena[L.child_parity()].get(), h->arena[L.child_parity() ^ 1].get());
       break;
     case Launch::PULL_MAT_BIG:
       extend_add_kernel<256><<<L.count, 256, 0, st>>>(sch.d_pull.get() + L.off, L.count, sch.d_pull_entries.get(), ds, h->Lx.get(),
-                                                      h->arena[L.child_parity].get(), h->arena[L.child_parity ^ 1].get());
+                                                      h->arena[L.child_parity()].get(), h->arena[L.child_parity() ^ 1].get());
       break;
     case Launch::PULL_VEC:
       vec_pull_kernel<<<(L.count + 3) / 4, 128, 0, st>>>(sch.d_pull.get() + L.off, L.count, sch.d_pull_entries.get(), ds, X,
-                                                         vec_arena[L.child_parity].get(),
-                                                         vec_arena[L.child_parity ^ 1].get(), d_vptr, nrhs);
+                                                         vec_arena[L.child_parity()].get(),
+                                                         vec_arena[L.child_parity() ^ 1].get(), d_vptr, nrhs);
       break;
     case Launch::REDUCE:
       splitk_reduce_kernel<<<L.grid, 256, 0, st>>>(sch.d_reduce.get() + L.off, L.count);
@@ -695,7 +695,7 @@ static void launch_one(slmm_chol* h, const Schedule& sch, const Launch& L, const
 #define SK_CASE(MT)                                                                        \
   if (f1) skinny_f1_kernel<MT><<<L.grid, SK_F1_COLS, 0, st>>>(ops, top);                   \
   else skinny_f2_kernel<MT><<<L.grid, 256, SK_F2_KMAX * MT * sizeof(double), st>>>(ops, top);
-      switch (L.child_parity) {
+      switch (L.row_mt()) {
         case 1: SK_CASE(1) break;
         case 2: SK_CASE(2) break;
         case 4: SK_CASE(4) break;
@@ -717,27 +717,21 @@ static void launch_one(slmm_chol* h, const Schedule& sch, const Launch& L, const
 
 static bool is_kernel(const Launch& L) { return L.kind != Launch::EV_RECORD && L.kind != Launch::EV_WAIT; }
 
-// Walks a launch list.  Single-stream schedules (solves, L*Z) run on the legacy default stream like every other
-// call of the library.  The factorization schedule names two streams: its critical chain (diagonal-block
-// factorizations, panel solves, next-panel updates) runs on a highest-priority stream, the look-ahead trailing
-// updates on a second one, ordered by events; both are forked from / joined to the default stream, so callers see
-// plain stream-0 semantics.  The list order is a valid topological order: the profiling mode simply runs it
-// serially on one stream with an event pair around every kernel.
-//
-// The lists are static (every kernel argument is fixed once the schedule is uploaded), so each one is captured
-// ONCE into a CUDA graph and replayed: a 12-column solve is a chain of ~1000 tiny launches whose cost was the
-// host's launch rate, not the kernels.
+// Issues a launch list.  With `two`, every launch goes to the stream it names, the priority stream (critical chain)
+// or the bulk stream (look-ahead trailing updates), ordered through `events`; otherwise all of them go to `one` in
+// list order, which is a valid topological order.  `per_launch` (optional) gets an event recorded after every kernel
+// on that kernel's stream.
 static void issue_schedule(slmm_chol* h, const Schedule& sch, double* X, const DevPtr<double>* vec_arena,
                            const int64_t* d_vptr, int nrhs, bool two, cudaStream_t one,
-                           std::vector<Event>* per_launch = nullptr) {
+                           const std::vector<Event>& events, std::vector<Event>* per_launch = nullptr) {
   const DevSym ds = h->devsym();
   size_t nk = 0;
   for (const Launch& L : sch.launches) {
     cudaStream_t st = two ? (L.stream ? h->s_bulk.get() : h->s_main.get()) : one;
-    if (L.kind == Launch::EV_RECORD) { if (two) CUDA_OK(cudaEventRecord(h->events[L.count].get(), st)); continue; }
-    if (L.kind == Launch::EV_WAIT) { if (two) CUDA_OK(cudaStreamWaitEvent(st, h->events[L.count].get(), 0)); continue; }
+    if (L.kind == Launch::EV_RECORD) { if (two) CUDA_OK(cudaEventRecord(events[L.event()].get(), st)); continue; }
+    if (L.kind == Launch::EV_WAIT) { if (two) CUDA_OK(cudaStreamWaitEvent(st, events[L.event()].get(), 0)); continue; }
     launch_one(h, sch, L, ds, X, vec_arena, d_vptr, nrhs, st);
-    if (per_launch) {                       // timeline mode: when did this launch finish (on its own stream)?
+    if (per_launch) {
       if (nk >= per_launch->size()) per_launch->push_back(make_event(cudaEventDefault));
       CUDA_OK(cudaEventRecord((*per_launch)[nk].get(), st));
     }
@@ -745,24 +739,32 @@ static void issue_schedule(slmm_chol* h, const Schedule& sch, double* X, const D
   }
 }
 
-// Captures the launch list into a graph.  Capture happens on the (non-blocking) priority stream - the legacy
-// default stream cannot be captured; the bulk stream joins the capture through the fork event.
+// Runs `body` on the priority stream (with `two`, on the bulk stream too) between a fork from the legacy default
+// stream (event `fork`) and a join back to it (event `join`), so that callers see plain stream-0 semantics.
+template <typename Body>
+static void forked(slmm_chol* h, bool two, cudaEvent_t fork, cudaEvent_t join, Body body) {
+  CUDA_OK(cudaEventRecord(fork, 0));
+  CUDA_OK(cudaStreamWaitEvent(h->s_main.get(), fork, 0));
+  if (two) CUDA_OK(cudaStreamWaitEvent(h->s_bulk.get(), fork, 0));
+  body();
+  if (two) {
+    CUDA_OK(cudaEventRecord(h->ev_join.get(), h->s_bulk.get()));
+    CUDA_OK(cudaStreamWaitEvent(h->s_main.get(), h->ev_join.get(), 0));
+  }
+  CUDA_OK(cudaEventRecord(join, h->s_main.get()));
+  CUDA_OK(cudaStreamWaitEvent(0, join, 0));
+}
+
+// Captures the serial walk of a launch list into a graph.  Capture happens on the (non-blocking) priority stream:
+// the legacy default stream cannot be captured.
 static GraphExec capture_schedule(slmm_chol* h, const Schedule& sch, double* X, const DevPtr<double>* vec_arena,
-                                        const int64_t* d_vptr, int nrhs, bool two) {
+                                  const int64_t* d_vptr, int nrhs) {
   cudaStream_t origin = h->s_main.get();
   cudaGraph_t graph = nullptr;
   cudaGraphExec_t exec = nullptr;
   CUDA_OK(cudaStreamBeginCapture(origin, cudaStreamCaptureModeRelaxed));
   try {
-    if (two) {
-      CUDA_OK(cudaEventRecord(h->ev_fork.get(), origin));
-      CUDA_OK(cudaStreamWaitEvent(h->s_bulk.get(), h->ev_fork.get(), 0));
-    }
-    issue_schedule(h, sch, X, vec_arena, d_vptr, nrhs, two, origin);
-    if (two) {
-      CUDA_OK(cudaEventRecord(h->ev_join.get(), h->s_bulk.get()));
-      CUDA_OK(cudaStreamWaitEvent(origin, h->ev_join.get(), 0));
-    }
+    issue_schedule(h, sch, X, vec_arena, d_vptr, nrhs, false, origin, h->events);
     CUDA_OK(cudaGetLastError());
   } catch (...) {
     cudaStreamEndCapture(origin, &graph);
@@ -777,92 +779,77 @@ static GraphExec capture_schedule(slmm_chol* h, const Schedule& sch, double* X, 
   return GraphExec(exec);
 }
 
+// Walks a launch list.  Single-stream schedules (solves, L*Z) run on the legacy default stream like every other
+// call of the library, or on the auxiliary stream inside an auxiliary section.  The factorization schedule names two
+// streams: its critical chain (diagonal-block factorizations, panel solves, next-panel updates) runs on a
+// highest-priority stream, the look-ahead trailing updates on a second one, ordered by events; both are forked from /
+// joined to the default stream.
+//
+// The lists are static (every kernel argument is fixed once the schedule is uploaded), so each single-stream list is
+// captured ONCE into a CUDA graph and replayed: a 12-column solve is a chain of ~1000 tiny launches whose cost was the
+// host's launch rate, not the kernels.  Two-stream lists are issued launch by launch: replaying the look-ahead pair
+// from a graph loses the stream priorities the chain relies on (measured: factorization 183 -> 190 ms at the 250K
+// config).
+//
+// Profiling mode walks any list serially on the current stream with an event after every kernel, and sums the
+// kernel times per kind.  Timeline mode issues a two-stream list with timed events, so the host can read when each
+// panel / bulk update finished relative to the fork (where is the critical path: the chain or the bulk stream?).
 static void run_schedule(slmm_chol* h, Schedule& sch, double* X, const DevPtr<double>* vec_arena, const int64_t* d_vptr,
                          int nrhs) {
   int64_t nk = 0;
   for (const Launch& L : sch.launches) nk += is_kernel(L) ? 1 : 0;
   if (nk == 0) return;
-  if (!h->profiling) {
+  if (h->profiling) {
+    const Event start = make_event(cudaEventDefault);
+    std::vector<Event> done;
+    CUDA_OK(cudaEventRecord(start.get(), h->cur));
+    issue_schedule(h, sch, X, vec_arena, d_vptr, nrhs, false, h->cur, h->events, &done);
+    CUDA_OK(cudaEventSynchronize(done.back().get()));
+    size_t i = 0;
+    for (const Launch& L : sch.launches) {
+      if (!is_kernel(L)) continue;
+      float ms = 0;
+      CUDA_OK(cudaEventElapsedTime(&ms, (i ? done[i - 1] : start).get(), done[i].get()));
+      const int k = (int)L.kind;
+      h->prof_ms[k] += ms;
+      h->prof_flops[k] += L.flops;
+      h->prof_n[k] += 1;
+      h->prof_launch_ms.push_back(ms);
+      h->prof_launch_flops.push_back(L.flops);
+      h->prof_launch_kind.push_back(k);
+      h->prof_launch_grid.push_back(work_size(L));
+      i++;
+    }
+  } else {
     // schedules with events run on the priority + bulk stream pair; inside an auxiliary section (cur != 0) the
     // pair may already be in use by the solve on stream 0, so the list is walked serially (a valid order)
     const bool two = sch.nevents > 0 && h->s_main != nullptr && h->cur == nullptr;
     while ((int)h->events.size() < sch.nevents) h->events.push_back(make_event(cudaEventDisableTiming));
-    const int gi = two ? 0 : 1;
-    if (h->timeline && two) {
-      // timeline mode: the same two-stream issue with TIMED events, so the host can read when each panel / bulk
-      // update finished relative to the fork (where is the critical path: the chain or the bulk stream?)
-      while ((int)h->tl_events.size() < sch.nevents + 2) h->tl_events.push_back(make_event(cudaEventDefault));
-      for (int q = 0; q < sch.nevents; q++) std::swap(h->events[q], h->tl_events[q + 2]);
-      CUDA_OK(cudaEventRecord(h->tl_events[0].get(), 0));
-      CUDA_OK(cudaStreamWaitEvent(h->s_main.get(), h->tl_events[0].get(), 0));
-      CUDA_OK(cudaStreamWaitEvent(h->s_bulk.get(), h->tl_events[0].get(), 0));
-      issue_schedule(h, sch, X, vec_arena, d_vptr, nrhs, true, nullptr, &h->tl_launch);
-      CUDA_OK(cudaEventRecord(h->ev_join.get(), h->s_bulk.get()));
-      CUDA_OK(cudaStreamWaitEvent(h->s_main.get(), h->ev_join.get(), 0));
-      CUDA_OK(cudaEventRecord(h->tl_events[1].get(), h->s_main.get()));
-      CUDA_OK(cudaStreamWaitEvent(0, h->tl_events[1].get(), 0));
-      CUDA_OK(cudaEventSynchronize(h->tl_events[1].get()));
-      for (int q = 0; q < sch.nevents; q++) std::swap(h->events[q], h->tl_events[q + 2]);
+    if (two && h->timeline) {
+      while ((int)h->tl_events.size() < sch.nevents) h->tl_events.push_back(make_event(cudaEventDefault));
+      forked(h, true, h->tl_fork.get(), h->tl_join.get(), [&] {
+        issue_schedule(h, sch, X, vec_arena, d_vptr, nrhs, true, nullptr, h->tl_events, &h->tl_launch);
+      });
+      CUDA_OK(cudaEventSynchronize(h->tl_join.get()));
       h->tl_count = sch.nevents + 2;
-      g_launch_count += nk;
-      return;
-    }
-    // graphs for the single-stream lists only: replaying the look-ahead pair from a graph loses the stream priorities
-    // the chain relies on (measured: factorization 183 -> 190 ms at the 250K config)
-    const bool use_graph = !two && h->s_main != nullptr && !sch.graph_failed;
-    if (use_graph && sch.gexec[gi] == nullptr) {
-      try {
-        sch.gexec[gi] = capture_schedule(h, sch, X, vec_arena, d_vptr, nrhs, two);
-      } catch (const std::exception&) {
-        sch.graph_failed = true;      // fall back to launch-by-launch for this schedule
-      }
-    }
-    cudaGraphExec_t exec = (use_graph && !sch.graph_failed) ? sch.gexec[gi].get() : nullptr;
-    if (exec != nullptr && h->cur != nullptr) {
-      CUDA_OK(cudaGraphLaunch(exec, h->cur));              // auxiliary section: the whole list on the auxiliary stream
-    } else if (exec != nullptr || two) {
-      // fork from / join to the legacy default stream around the priority stream (and, inside, the bulk stream)
-      CUDA_OK(cudaEventRecord(h->ev_fork.get(), 0));
-      CUDA_OK(cudaStreamWaitEvent(h->s_main.get(), h->ev_fork.get(), 0));
-      if (exec != nullptr) {
-        CUDA_OK(cudaGraphLaunch(exec, h->s_main.get()));
-      } else {
-        CUDA_OK(cudaStreamWaitEvent(h->s_bulk.get(), h->ev_fork.get(), 0));
-        issue_schedule(h, sch, X, vec_arena, d_vptr, nrhs, true, nullptr);
-        CUDA_OK(cudaEventRecord(h->ev_join.get(), h->s_bulk.get()));
-        CUDA_OK(cudaStreamWaitEvent(h->s_main.get(), h->ev_join.get(), 0));
-      }
-      CUDA_OK(cudaEventRecord(h->ev_join.get(), h->s_main.get()));
-      CUDA_OK(cudaStreamWaitEvent(0, h->ev_join.get(), 0));
+    } else if (two) {
+      forked(h, true, h->ev_fork.get(), h->ev_join.get(),
+             [&] { issue_schedule(h, sch, X, vec_arena, d_vptr, nrhs, true, nullptr, h->events); });
     } else {
-      issue_schedule(h, sch, X, vec_arena, d_vptr, nrhs, false, h->cur);
-    }
-  } else {
-    // per-launch CUDA events on the launching stream (serialises nothing: same stream order), summed per kind
-    const DevSym ds = h->devsym();
-    cudaStream_t st = h->cur;
-    std::vector<const Launch*> ks;
-    for (const Launch& L : sch.launches) if (is_kernel(L)) ks.push_back(&L);
-    const size_t nl = ks.size();
-    std::vector<Event> ev(nl + 1);
-    for (auto& e : ev) e = make_event(cudaEventDefault);
-    CUDA_OK(cudaEventRecord(ev[0].get(), st));
-    for (size_t i = 0; i < nl; i++) {
-      launch_one(h, sch, *ks[i], ds, X, vec_arena, d_vptr, nrhs, st);
-      CUDA_OK(cudaEventRecord(ev[i + 1].get(), st));
-    }
-    CUDA_OK(cudaEventSynchronize(ev[nl].get()));
-    for (size_t i = 0; i < nl; i++) {
-      float ms = 0;
-      CUDA_OK(cudaEventElapsedTime(&ms, ev[i].get(), ev[i + 1].get()));
-      const int k = (int)ks[i]->kind;
-      h->prof_ms[k] += ms;
-      h->prof_flops[k] += ks[i]->flops;
-      h->prof_n[k] += 1;
-      h->prof_launch_ms.push_back(ms);
-      h->prof_launch_flops.push_back(ks[i]->flops);
-      h->prof_launch_kind.push_back(k);
-      h->prof_launch_grid.push_back((ks[i]->kind <= Launch::GEMM_SMALL || ks[i]->kind >= Launch::SKINNY_F1) ? ks[i]->grid : ks[i]->count);
+      if (h->s_main != nullptr && sch.gexec == nullptr && !sch.graph_failed) {
+        try {
+          sch.gexec = capture_schedule(h, sch, X, vec_arena, d_vptr, nrhs);
+        } catch (const std::exception&) {
+          sch.graph_failed = true;      // fall back to launch-by-launch for this schedule
+        }
+      }
+      cudaGraphExec_t exec = sch.gexec.get();
+      if (exec == nullptr)
+        issue_schedule(h, sch, X, vec_arena, d_vptr, nrhs, false, h->cur, h->events);
+      else if (h->cur != nullptr)
+        CUDA_OK(cudaGraphLaunch(exec, h->cur));            // auxiliary section: the whole list on the auxiliary stream
+      else
+        forked(h, false, h->ev_fork.get(), h->ev_join.get(), [&] { CUDA_OK(cudaGraphLaunch(exec, h->s_main.get())); });
     }
   }
   g_launch_count += nk;
@@ -919,30 +906,85 @@ static void add_pull_items(Schedule& sch, const Symbolic& S, const std::vector<i
     }
   }
   const int cnt = (int)(sch.pull.size() - off);
-  if (cnt > 0) sch.launches.push_back({kind, off, cnt, 0, (level + 1) & 1, 0.0});
+  if (cnt > 0) sch.add(kind, off, cnt, 0, 0.0, 0).variant = (level + 1) & 1;
 }
 
-// Outer (NBO-wide) diagonal block `ob` of supernode s: column range, and where its inverse lives.  A block made
+// Supernode s as a dense front: first column f, ns columns, ms rows (rs below the diagonal block), and its panel P
+// with leading dimension ld.
+struct Front {
+  int s, f, ns, ms, rs;
+  int64_t ld;
+  double* P;
+};
+static Front front(const slmm_chol* h, int s) {
+  const Symbolic& S = h->S;
+  const int f = S.sn_first[s], ns = S.sn_first[s + 1] - f, ms = S.sn_nrow[s];
+  return Front{s, f, ns, ms, ms - ns, panel_ld(ms), h->Lx.get() + S.sn_lptr[s]};
+}
+
+// Outer (NBO-wide) diagonal block `ob` of a front: column range, and where its inverse lives.  A block made
 // of a single NBI block reuses the POTRF kernel's 64 x 64 inverse slot; wider blocks get their own slot in W.
 struct OuterBlock { int o0, nbo, ldw; double* winv; };
 static int num_outer(int ns) { return (ns + NBO - 1) / NBO; }
-static OuterBlock outer_block(const slmm_chol* h, int s, int ob) {
-  const Symbolic& S = h->S;
-  const int ns = S.sn_first[s + 1] - S.sn_first[s];
+static OuterBlock outer_block(const slmm_chol* h, const Front& F, int ob) {
   OuterBlock b;
   b.o0 = ob * NBO;
-  b.nbo = std::min(ns, b.o0 + NBO) - b.o0;
+  b.nbo = std::min(F.ns, b.o0 + NBO) - b.o0;
   if (b.nbo <= NBI) {
-    b.winv = h->inv.get() + h->invptr[s] + (int64_t)(b.o0 / NBI) * NBI * NBI;
+    b.winv = h->inv.get() + h->invptr[F.s] + (int64_t)(b.o0 / NBI) * NBI * NBI;
     b.ldw = NBI;
   } else {
-    int64_t off = h->wptr[s];
+    int64_t off = h->wptr[F.s];
     for (int q = 0; q < ob; q++) off += (int64_t)NBO * NBO;      // every earlier block of s is a full one
     b.winv = h->W.get() + off;
     b.ldw = b.nbo;
   }
   return b;
 }
+
+// outer blocks of the widest front of level d
+static int max_outer(const Symbolic& S, int d) {
+  int m = 0;
+  for (int q = S.level_ptr[d]; q < S.level_ptr[d + 1]; q++) {
+    const int s = S.level_sn[q];
+    m = std::max(m, num_outer(S.sn_first[s + 1] - S.sn_first[s]));
+  }
+  return m;
+}
+
+// Two-stream look-ahead of the wide fronts.  Each phase of a level puts its critical chain on the main stream and
+// the look-ahead remainders on the bulk stream: `bulk` holds updates that the chain needs only in a later outer
+// block, `below` (factorization only) the rows below the next diagonal block, which that block's triangular panel
+// multiply reads.  The bulk work starts once the chain's launches of the phase have produced its operands; the
+// chain waits for it before anything that touches the same entries again, and at the end of the level.
+struct LookAhead {
+  PhaseBuilder chain, below, bulk;
+  int last_bulk_ev = -1, below_ev = -1;
+  // updated: the chain's launches of this phase write entries the earlier bulk launches may still be writing
+  // reads_below: they read rows `below` updated
+  void flush_phase(Schedule& sch, bool updated, bool reads_below = false) {
+    const bool side = !below.empty() || !bulk.empty();
+    const int ev_chain = side ? sch.record(0) : -1;
+    if (updated && last_bulk_ev >= 0) { sch.wait(last_bulk_ev, 0); last_bulk_ev = -1; }
+    if (reads_below && below_ev >= 0) { sch.wait(below_ev, 0); below_ev = -1; }
+    chain.flush(sch, 0);
+    if (!side) return;
+    sch.wait(ev_chain, 1);
+    if (!below.empty()) {           // rows below the next block first, with their own event
+      below.flush(sch, 1);
+      below_ev = last_bulk_ev = sch.record(1);
+    }
+    if (!bulk.empty()) {
+      bulk.flush(sch, 1);
+      last_bulk_ev = sch.record(1);
+    }
+  }
+  // level boundary: everything of this level is complete before the pulls
+  void end_level(Schedule& sch) {
+    if (last_bulk_ev >= 0) sch.wait(last_bulk_ev, 0);
+    last_bulk_ev = below_ev = -1;
+  }
+};
 
 // One step of a front's factorization program.  Phase p of a level executes step p of every front of the level.
 struct FStep {
@@ -953,9 +995,10 @@ struct FStep {
 static void build_factor_schedule(slmm_chol* h) {
   const Symbolic& S = h->S;
   Schedule& sch = h->fact;
-  PhaseBuilder pb, pb_rest, pb_unrest;
-  pb_rest.allow_split = pb_unrest.allow_split = false;   // bulk-stream ops run beside the chain: the split-K workspace has one user
-  int last_bulk_ev = -1, unrest_ev = -1;
+  LookAhead la;
+  // bulk-stream ops run beside the chain: the split-K workspace has one user
+  la.below.allow_split = la.bulk.allow_split = false;
+  PhaseBuilder& pb = la.chain;
   std::vector<std::vector<FStep>> prog;
   for (int d = S.nlevels - 1; d >= 0; d--) {
     add_pull_items(sch, S, h->uptr, d, 0, Launch::PULL_MAT, 8, 0, 512);
@@ -965,35 +1008,34 @@ static void build_factor_schedule(slmm_chol* h) {
     prog.assign(nl, std::vector<FStep>());
     size_t max_steps = 0;
     for (int q = 0; q < nl; q++) {
-      const int s = S.level_sn[S.level_ptr[d] + q];
-      const int ns = S.sn_first[s + 1] - S.sn_first[s], ms = S.sn_nrow[s], rs = ms - ns;
+      const Front F = front(h, S.level_sn[S.level_ptr[d] + q]);
       std::vector<FStep>& pr = prog[q];
-      if (ns <= NBO) {
+      if (F.ns <= NBO) {
         // narrow front: per 64 columns POTRF, panel solve of ALL rows below, in-block update; Schur complement last
-        const int nib = (ns + NBI - 1) / NBI;
+        const int nib = (F.ns + NBI - 1) / NBI;
         for (int ib = 0; ib < nib; ib++) {
           pr.push_back({FStep::POTRF, ib, 0});
           pr.push_back({FStep::TRSM, ib, 0});
           if (ib + 1 < nib) pr.push_back({FStep::UPD, ib, 0});
         }
-        if (rs > 0) pr.push_back({FStep::SCHUR, 0, 0});
+        if (F.rs > 0) pr.push_back({FStep::SCHUR, 0, 0});
       } else {
         // Wide front (a dense panel chain): the 64-column steps touch ONLY the w x w diagonal block of the current
         // outer block (tiny launches: they find free SMs at once even while bulk updates fill the machine), the
         // block inverse W = L_D^-1 is built by recursive doubling from the 64 x 64 inverses, and the rows below take
         // one triangular multiply L21 = A21 W' (128-column blocks, in place, last block first).
-        for (int ob = 0; ob < num_outer(ns); ob++) {
-          const int o0 = ob * NBO, o1 = std::min(ns, o0 + NBO), w = o1 - o0;
+        for (int ob = 0; ob < num_outer(F.ns); ob++) {
+          const int o0 = ob * NBO, o1 = std::min(F.ns, o0 + NBO), w = o1 - o0;
           for (int c0 = o0; c0 < o1; c0 += NBI) {
             const int ib = c0 / NBI;
             pr.push_back({FStep::POTRF, ib, 0});
             if (std::min(o1, c0 + NBI) < o1) { pr.push_back({FStep::TRSM, ib, 0}); pr.push_back({FStep::UPD, ib, 0}); }
           }
           for (int m = NBI; m < w; m *= 2) { pr.push_back({FStep::WINV1, ob, m}); pr.push_back({FStep::WINV2, ob, m}); }
-          if (ms > o1)
+          if (F.ms > o1)
             for (int j = (w + 127) / 128 - 1; j >= 0; j--) pr.push_back({FStep::CPANEL, ob, j});
-          if (o1 < ns) pr.push_back({FStep::OUTER, ob, 0});
-          else if (rs > 0) pr.push_back({FStep::SCHUR, 0, 0});
+          if (o1 < F.ns) pr.push_back({FStep::OUTER, ob, 0});
+          else if (F.rs > 0) pr.push_back({FStep::SCHUR, 0, 0});
         }
       }
       max_steps = std::max(max_steps, pr.size());
@@ -1005,38 +1047,36 @@ static void build_factor_schedule(slmm_chol* h) {
         if (ph >= prog[q].size()) continue;
         const FStep st = prog[q][ph];
         if (st.kind == FStep::CPANEL || st.kind == FStep::SCHUR) needs_below = true;
-        const int s = S.level_sn[S.level_ptr[d] + q];
-        const int f = S.sn_first[s], ns = S.sn_first[s + 1] - f, ms = S.sn_nrow[s], rs = ms - ns;
-        const bool wide = ns > NBO;
-        double* P = h->Lx.get() + S.sn_lptr[s];
-        const int64_t ld = panel_ld(ms);
+        const Front F = front(h, S.level_sn[S.level_ptr[d] + q]);
+        const bool wide = F.ns > NBO;
         if (st.kind == FStep::POTRF || st.kind == FStep::TRSM || st.kind == FStep::UPD) {
-          const int ib = st.a, c0 = ib * NBI, c1 = std::min(ns, c0 + NBI), nb = c1 - c0;
-          const int ob = c0 / NBO, ob0 = ob * NBO, ob_end = std::min(ns, ob0 + NBO);
+          const int ib = st.a, c0 = ib * NBI, c1 = std::min(F.ns, c0 + NBI), nb = c1 - c0;
+          const int ob = c0 / NBO, ob0 = ob * NBO, ob_end = std::min(F.ns, ob0 + NBO);
           // where the inverse of this 64 x 64 block lives: its private slot, or (wide fronts) the diagonal of W
-          double* inv = h->inv.get() + h->invptr[s] + (int64_t)ib * NBI * NBI;
+          double* inv = h->inv.get() + h->invptr[F.s] + (int64_t)ib * NBI * NBI;
           int64_t inv_ld = NBI;
           if (wide) {
-            const OuterBlock wb = outer_block(h, s, ob);
+            const OuterBlock wb = outer_block(h, F, ob);
             if (wb.nbo > NBI) { inv = wb.winv + (c0 - ob0) + (int64_t)(c0 - ob0) * wb.ldw; inv_ld = wb.ldw; }
           }
-          const int row_end = wide ? ob_end : ms;      // wide fronts: only the diagonal block of the outer block
+          const int row_end = wide ? ob_end : F.ms;      // wide fronts: only the diagonal block of the outer block
           if (st.kind == FStep::POTRF) {
-            pb.potrf.push_back({P + c0 + c0 * ld, inv, (int32_t)ld, nb, f + c0, (int32_t)inv_ld});
+            pb.potrf.push_back({F.P + c0 + c0 * F.ld, inv, (int32_t)F.ld, nb, F.f + c0, (int32_t)inv_ld});
             sch.flops += (double)nb * nb * nb / 3.0;
           } else if (st.kind == FStep::TRSM) {
             // rows below the diagonal block:  X = X * inv^T   (in place, one tile column)
-            pb.add(make_op(P + c1 + c0 * ld, 1, ld, P + c1 + c0 * ld, 1, ld, inv, 1, inv_ld, row_end - c1, nb, nb, 0));
+            pb.add(make_op(F.P + c1 + c0 * F.ld, 1, F.ld, F.P + c1 + c0 * F.ld, 1, F.ld, inv, 1, inv_ld, row_end - c1, nb,
+                           nb, 0));
           } else {
             // update the rest of the current outer block with this inner block
-            pb.add(make_op(P + c1 + c1 * ld, 1, ld, P + c1 + c0 * ld, 1, ld, P + c1 + c0 * ld, 1, ld, row_end - c1,
-                           ob_end - c1, nb, GF_LOWER | GF_ACCUM | GF_NEG));
+            pb.add(make_op(F.P + c1 + c1 * F.ld, 1, F.ld, F.P + c1 + c0 * F.ld, 1, F.ld, F.P + c1 + c0 * F.ld, 1, F.ld,
+                           row_end - c1, ob_end - c1, nb, GF_LOWER | GF_ACCUM | GF_NEG));
           }
         } else if (st.kind == FStep::WINV1 || st.kind == FStep::WINV2) {
           // recursive doubling: inv([A 0; C B]) = [A^-1 0; -B^-1 (C A^-1)  B^-1], pairs of blocks of size m
-          const OuterBlock wb = outer_block(h, s, st.a);
+          const OuterBlock wb = outer_block(h, F, st.a);
           const int m = st.b, o0 = wb.o0;
-          double* T = h->wscratch.get() + h->wscratch_off[s];
+          double* T = h->wscratch.get() + h->wscratch_off[F.s];
           int pair = 0;
           for (int lo = 0; lo + m < wb.nbo; lo += 2 * m, pair++) {
             const int m2 = std::min(m, wb.nbo - lo - m);
@@ -1045,79 +1085,50 @@ static void build_factor_schedule(slmm_chol* h) {
             double* Binv = wb.winv + (lo + m) + (int64_t)(lo + m) * wb.ldw;
             double* X21 = wb.winv + (lo + m) + (int64_t)lo * wb.ldw;
             if (st.kind == FStep::WINV1)       // T = C A^-1
-              pb.add(make_op(Tp, 1, m2, P + (o0 + lo + m) + (int64_t)(o0 + lo) * ld, 1, ld, Ainv, wb.ldw, 1, m2, m, m, 0));
+              pb.add(make_op(Tp, 1, m2, F.P + (o0 + lo + m) + (int64_t)(o0 + lo) * F.ld, 1, F.ld, Ainv, wb.ldw, 1, m2, m,
+                             m, 0));
             else                               // X21 = -B^-1 T
               pb.add(make_op(X21, 1, wb.ldw, Binv, 1, wb.ldw, Tp, m2, 1, m2, m, m2, GF_NEG));
           }
         } else if (st.kind == FStep::CPANEL) {
           // rows below the outer block: L21[:, j-th 128 columns] = A21[:, 0:K) W[j-th rows, 0:K)'  (W lower triangular)
-          const OuterBlock wb = outer_block(h, s, st.a);
+          const OuterBlock wb = outer_block(h, F, st.a);
           const int o0 = wb.o0, o1 = o0 + wb.nbo, j0 = 128 * st.b, nj = std::min(128, wb.nbo - j0);
           const int K = std::min(wb.nbo, j0 + 128);
-          pb.add(make_op(P + o1 + (int64_t)(o0 + j0) * ld, 1, ld, P + o1 + (int64_t)o0 * ld, 1, ld, wb.winv + j0, 1, wb.ldw,
-                         ms - o1, nj, K, GF_BIGTILE));
+          pb.add(make_op(F.P + o1 + (int64_t)(o0 + j0) * F.ld, 1, F.ld, F.P + o1 + (int64_t)o0 * F.ld, 1, F.ld, wb.winv + j0,
+                         1, wb.ldw, F.ms - o1, nj, K, GF_BIGTILE));
         } else if (st.kind == FStep::OUTER) {
           // outer block finished: update all remaining panel columns, K = block width.
           // Look-ahead: the columns of the NEXT outer block are updated on the main stream (they gate the next
           // panel factorization); the columns beyond it go to the bulk stream and overlap with that panel
           // factorization, whose diagonal-block steps leave almost every SM idle.
-          const int ob0 = st.a * NBO, c1 = std::min(ns, ob0 + NBO);
+          const int ob0 = st.a * NBO, c1 = std::min(F.ns, ob0 + NBO);
           outer_done = true;
-          const int nx = std::min(ns, c1 + NBO);
-          const bool split = (ns - nx) >= NBO;
-          const int ncols = split ? nx - c1 : ns - c1;
+          const int nx = std::min(F.ns, c1 + NBO);
+          const bool split = (F.ns - nx) >= NBO;
+          const int ncols = split ? nx - c1 : F.ns - c1;
           // Of the next block's columns only the square diagonal part gates the chain (the 64-column steps of the
           // next outer block); the rows below it are needed when that block's triangular panel multiply starts, so
           // they go to the bulk stream with their own event.
-          const int below = ms - c1 - ncols;
-          pb.add(make_op(P + c1 + c1 * ld, 1, ld, P + c1 + ob0 * ld, 1, ld, P + c1 + ob0 * ld, 1, ld, ncols,
-                         ncols, c1 - ob0, GF_LOWER | GF_ACCUM | GF_NEG));
+          const int below = F.ms - c1 - ncols;
+          pb.add(make_op(F.P + c1 + c1 * F.ld, 1, F.ld, F.P + c1 + ob0 * F.ld, 1, F.ld, F.P + c1 + ob0 * F.ld, 1, F.ld,
+                         ncols, ncols, c1 - ob0, GF_LOWER | GF_ACCUM | GF_NEG));
           if (below > 0)
-            pb_unrest.add(make_op(P + (c1 + ncols) + c1 * ld, 1, ld, P + (c1 + ncols) + ob0 * ld, 1, ld, P + c1 + ob0 * ld, 1, ld,
-                                  below, ncols, c1 - ob0, GF_ACCUM | GF_NEG));
+            la.below.add(make_op(F.P + (c1 + ncols) + c1 * F.ld, 1, F.ld, F.P + (c1 + ncols) + ob0 * F.ld, 1, F.ld,
+                                 F.P + c1 + ob0 * F.ld, 1, F.ld, below, ncols, c1 - ob0, GF_ACCUM | GF_NEG));
           if (split)
-            pb_rest.add(make_op(P + nx + nx * ld, 1, ld, P + nx + ob0 * ld, 1, ld, P + nx + ob0 * ld, 1, ld, ms - nx,
-                                ns - nx, c1 - ob0, GF_LOWER | GF_ACCUM | GF_NEG));
+            la.bulk.add(make_op(F.P + nx + nx * F.ld, 1, F.ld, F.P + nx + ob0 * F.ld, 1, F.ld, F.P + nx + ob0 * F.ld, 1, F.ld,
+                                F.ms - nx, F.ns - nx, c1 - ob0, GF_LOWER | GF_ACCUM | GF_NEG));
         } else {                      // SCHUR: panel done, U = -L21 L21'
-          double* U = h->arena[d & 1].get() + h->uptr[s];
-          pb.add(make_op(U, 1, rs, P + ns, 1, ld, P + ns, 1, ld, rs, rs, ns, GF_LOWER | GF_NEG));
+          double* U = h->arena[d & 1].get() + h->uptr[F.s];
+          pb.add(make_op(U, 1, F.rs, F.P + F.ns, 1, F.ld, F.P + F.ns, 1, F.ld, F.rs, F.rs, F.ns, GF_LOWER | GF_NEG));
         }
       }
-      const bool side = !pb_rest.empty() || !pb_unrest.empty();
-      int ev_panel = -1;
-      if (side) {                     // the panels of this outer block are final from here on
-        ev_panel = sch.nevents++;
-        sch.launches.push_back({Launch::EV_RECORD, 0, ev_panel, 0, 0, 0.0, 0, 0});
-      }
-      // a trailing update writes entries the previous bulk updates may still be writing
-      if (outer_done && last_bulk_ev >= 0) {
-        sch.launches.push_back({Launch::EV_WAIT, 0, last_bulk_ev, 0, 0, 0.0, 0, 0});
-        last_bulk_ev = -1;
-      }
-      // the triangular panel multiply (and the Schur complement) read rows the bulk stream updated
-      if (needs_below && unrest_ev >= 0) {
-        sch.launches.push_back({Launch::EV_WAIT, 0, unrest_ev, 0, 0, 0.0, 0, 0});
-        unrest_ev = -1;
-      }
-      pb.flush(sch, 0);               // critical chain (+ the steps of every other front)
-      if (side) {
-        sch.launches.push_back({Launch::EV_WAIT, 0, ev_panel, 0, 0, 0.0, 0, 1});
-        if (!pb_unrest.empty()) {     // rows below the next block first, with their own event
-          pb_unrest.flush(sch, 1);
-          unrest_ev = sch.nevents++;
-          sch.launches.push_back({Launch::EV_RECORD, 0, unrest_ev, 0, 0, 0.0, 0, 1});
-          last_bulk_ev = unrest_ev;
-        }
-        if (!pb_rest.empty()) {
-          pb_rest.flush(sch, 1);
-          last_bulk_ev = sch.nevents++;
-          sch.launches.push_back({Launch::EV_RECORD, 0, last_bulk_ev, 0, 0, 0.0, 0, 1});
-        }
-      }
+      // a trailing update writes entries the previous bulk updates may still be writing; the triangular panel
+      // multiply (and the Schur complement) read rows the bulk stream updated
+      la.flush_phase(sch, outer_done, needs_below);
     }
-    // level boundary: everything of this level is complete before the pulls
-    if (last_bulk_ev >= 0) sch.launches.push_back({Launch::EV_WAIT, 0, last_bulk_ev, 0, 0, 0.0, 0, 0});
-    last_bulk_ev = unrest_ev = -1;
+    la.end_level(sch);
     add_pull_items(sch, S, h->uptr, d, 1, Launch::PULL_MAT, 8, 0, 512);
     add_pull_items(sch, S, h->uptr, d, 1, Launch::PULL_MAT_BIG, 4, 512);
   }
@@ -1126,23 +1137,21 @@ static void build_factor_schedule(slmm_chol* h) {
   //      substitution by NBI blocks:  W[t,:] = inv_t W[t,:];  W[t+1:,:] -= L[t+1:,t] W[t,:].  The multi-RHS solves
   //      then need 2 GEMMs per NBO columns instead of per 64.
   if (!h->wblocks.empty()) {
-    sch.launches.push_back({Launch::INIT_W, 0, (int32_t)h->wblocks.size(), (int32_t)h->wblocks.size(), 0, 0.0});
+    sch.add(Launch::INIT_W, 0, (int32_t)h->wblocks.size(), (int32_t)h->wblocks.size(), 0.0, 0);
     for (int t = 0; t < NBO / NBI; t++) {
       for (int half = 0; half < 2; half++) {
         for (int s2 = 0; s2 < S.nsuper; s2++) {
-          const int ns = S.sn_first[s2 + 1] - S.sn_first[s2];
-          if (ns <= NBI || ns > NBO) continue;
-          double* P = h->Lx.get() + S.sn_lptr[s2];
-          const int64_t ldp = panel_ld(S.sn_nrow[s2]);
-          for (int ob = 0; ob < num_outer(ns); ob++) {
-            const OuterBlock b = outer_block(h, s2, ob);
+          const Front F = front(h, s2);
+          if (F.ns <= NBI || F.ns > NBO) continue;
+          for (int ob = 0; ob < num_outer(F.ns); ob++) {
+            const OuterBlock b = outer_block(h, F, ob);
             if (b.nbo <= NBI || t * NBI >= b.nbo) continue;
             const int r0 = t * NBI, nbt = std::min(NBI, b.nbo - r0), ncols = std::min(b.nbo, r0 + NBI);
             double* inv64 = h->inv.get() + h->invptr[s2] + (int64_t)((b.o0 + r0) / NBI) * NBI * NBI;
             if (half == 0) {
               pb.add(make_op(b.winv + r0, 1, b.ldw, inv64, 1, NBI, b.winv + r0, b.ldw, 1, nbt, ncols, nbt, 0));
             } else if (r0 + nbt < b.nbo) {
-              pb.add(make_op(b.winv + r0 + nbt, 1, b.ldw, P + (b.o0 + r0 + nbt) + (int64_t)(b.o0 + r0) * ldp, 1, ldp,
+              pb.add(make_op(b.winv + r0 + nbt, 1, b.ldw, F.P + (b.o0 + r0 + nbt) + (int64_t)(b.o0 + r0) * F.ld, 1, F.ld,
                              b.winv + r0, b.ldw, 1, b.nbo - r0 - nbt, ncols, nbt, GF_ACCUM | GF_NEG));
             }
           }
@@ -1188,113 +1197,80 @@ static SolvePlan* get_plan(slmm_chol* h, int nrhs) {
   pl->d_vptr = dev_upload(vptr.data(), vptr.size());
   pl->bytes = ((size_t)2 * n * nrhs + asz[0] + asz[1]) * 8;
   const int64_t R = nrhs;
-  PhaseBuilder pb, pb_rest;
+  LookAhead la;
+  PhaseBuilder& pb = la.chain;
   // bulk-stream ops run beside the chain's: their split-K partials get a workspace of their own.  The bulk updates of
   // consecutive diagonal blocks are serialised (same rows), and the late ones have far fewer tiles than SMs: without
   // split-K each still costs one full-K tile latency (170 us at the 250K config whatever its size)
-  pb_rest.ws_id = 1;
+  la.bulk.ws_id = 1;
   // narrow blocks, up to 32 columns (the local probe block at 4 GPUs): HBM-streaming kernels instead of DMMA tiles
   // (skinny_ops.cuh).  Measured at the 250K config, solve / L*Z in ms, tiles -> streaming: 32 columns 7.7 -> 6.3 /
   // 3.6 -> 2.2; 64 columns 8.2 -> 9.6 / 3.9 -> 3.7 (16 DMMA per streamed fragment: the tensor pipe, not HBM, bounds
   // the stream there).
   if (nrhs <= 32) pb.skinny_mt = nrhs <= 1 ? 1 : nrhs <= 2 ? 2 : nrhs <= 4 ? 4 : nrhs <= 8 ? 8 : nrhs <= 16 ? 16 : 32;
   const bool lookahead = nrhs >= 64;     // narrow solves are launch-latency chains: nothing to overlap with
-  int last_bulk_ev = -1;
-  // One phase: the chain's launches on the main stream; look-ahead remainders (if any) on the bulk stream, after
-  // the diagonal step that produced their operand and before anything that touches the same rows again.
-  auto flush_pair = [&](Schedule& sch, bool updated) {
-    int ev_diag = -1;
-    if (!pb_rest.empty()) {
-      ev_diag = sch.nevents++;
-      sch.launches.push_back({Launch::EV_RECORD, 0, ev_diag, 0, 0, 0.0, 0, 0});
-    }
-    if (updated && last_bulk_ev >= 0) {
-      sch.launches.push_back({Launch::EV_WAIT, 0, last_bulk_ev, 0, 0, 0.0, 0, 0});
-      last_bulk_ev = -1;
-    }
-    pb.flush(sch, 0);
-    if (ev_diag >= 0) {
-      sch.launches.push_back({Launch::EV_WAIT, 0, ev_diag, 0, 0, 0.0, 0, 1});
-      pb_rest.flush(sch, 1);
-      last_bulk_ev = sch.nevents++;
-      sch.launches.push_back({Launch::EV_RECORD, 0, last_bulk_ev, 0, 0, 0.0, 0, 1});
-    }
-  };
   // ---------------- forward:  L y = b  (levels deepest first).  X holds b and the running updates, the solved
   //                  blocks y land in X2 (out of place: Y = Winv * X per NBO-wide diagonal block).
   for (int d = S.nlevels - 1; d >= 0; d--) {
     add_pull_items(pl->fwd, S, vptr, d, 0, Launch::PULL_VEC, 4);
-    int max_nob = 0;
-    for (int q = S.level_ptr[d]; q < S.level_ptr[d + 1]; q++) {
-      const int s = S.level_sn[q];
-      max_nob = std::max(max_nob, num_outer(S.sn_first[s + 1] - S.sn_first[s]));
-    }
+    const int max_nob = max_outer(S, d);
     for (int ph = 0; ph < 2 * max_nob + 1; ph++) {
       bool updated = false;
       for (int q = S.level_ptr[d]; q < S.level_ptr[d + 1]; q++) {
-        const int s = S.level_sn[q];
-        const int f = S.sn_first[s], ns = S.sn_first[s + 1] - f, ms = S.sn_nrow[s], rs = ms - ns;
-        const int nob = num_outer(ns);
-        double* P = h->Lx.get() + S.sn_lptr[s];
-        const int64_t ld = panel_ld(ms);
-        double* Xs = pl->X.get() + (int64_t)f * R;
-        double* Ys = pl->X2.get() + (int64_t)f * R;
+        const Front F = front(h, S.level_sn[q]);
+        const int nob = num_outer(F.ns);
+        double* Xs = pl->X.get() + (int64_t)F.f * R;
+        double* Ys = pl->X2.get() + (int64_t)F.f * R;
         if (ph == 2 * nob) {                       // contribution block  u = -L21 y   (rs x nrhs)
-          if (rs > 0)
-            pb.add(make_op(pl->arena[d & 1].get() + vptr[s], 1, R, Ys, 1, R, P + ns, 1, ld, nrhs, rs, ns, GF_NEG));
+          if (F.rs > 0)
+            pb.add(make_op(pl->arena[d & 1].get() + vptr[F.s], 1, R, Ys, 1, R, F.P + F.ns, 1, F.ld, nrhs, F.rs, F.ns,
+                           GF_NEG));
           continue;
         }
         if (ph > 2 * nob) continue;
-        const OuterBlock b = outer_block(h, s, ph / 2);
+        const OuterBlock b = outer_block(h, F, ph / 2);
         const int o1 = b.o0 + b.nbo;
         if (ph % 2 == 0) {                         // y_b = Winv * x_b      (transposed view: Y^T = X^T Winv^T)
           pb.add(make_op(Ys + (int64_t)b.o0 * R, 1, R, Xs + (int64_t)b.o0 * R, 1, R, b.winv, 1, b.ldw, nrhs, b.nbo,
                          b.nbo, 0));
-        } else if (o1 < ns) {                      // x[o1:ns] -= L[o1:ns, o0:o1] y_b
+        } else if (o1 < F.ns) {                    // x[o1:ns] -= L[o1:ns, o0:o1] y_b
           // Look-ahead (wide fronts, many RHS): only the rows of the next diagonal block gate the chain; the rows
           // beyond go to the bulk stream and overlap with the next diagonal steps (a few tiles each).
           updated = true;
-          const int nx = std::min(ns, o1 + NBO);
-          const bool split = lookahead && (ns - nx) >= NBO;
-          pb.add(make_op(Xs + (int64_t)o1 * R, 1, R, Ys + (int64_t)b.o0 * R, 1, R, P + o1 + (int64_t)b.o0 * ld, 1, ld,
-                         nrhs, (split ? nx : ns) - o1, b.nbo, GF_ACCUM | GF_NEG));
+          const int nx = std::min(F.ns, o1 + NBO);
+          const bool split = lookahead && (F.ns - nx) >= NBO;
+          pb.add(make_op(Xs + (int64_t)o1 * R, 1, R, Ys + (int64_t)b.o0 * R, 1, R, F.P + o1 + (int64_t)b.o0 * F.ld, 1,
+                         F.ld, nrhs, (split ? nx : F.ns) - o1, b.nbo, GF_ACCUM | GF_NEG));
           if (split)
-            pb_rest.add(make_op(Xs + (int64_t)nx * R, 1, R, Ys + (int64_t)b.o0 * R, 1, R, P + nx + (int64_t)b.o0 * ld, 1, ld,
-                                nrhs, ns - nx, b.nbo, GF_ACCUM | GF_NEG));
+            la.bulk.add(make_op(Xs + (int64_t)nx * R, 1, R, Ys + (int64_t)b.o0 * R, 1, R, F.P + nx + (int64_t)b.o0 * F.ld,
+                                1, F.ld, nrhs, F.ns - nx, b.nbo, GF_ACCUM | GF_NEG));
         }
       }
-      flush_pair(pl->fwd, updated);
+      la.flush_phase(pl->fwd, updated);
     }
-    if (last_bulk_ev >= 0) { pl->fwd.launches.push_back({Launch::EV_WAIT, 0, last_bulk_ev, 0, 0, 0.0, 0, 0}); last_bulk_ev = -1; }
+    la.end_level(pl->fwd);
     add_pull_items(pl->fwd, S, vptr, d, 1, Launch::PULL_VEC, 4);
   }
   // ---------------- backward:  L' x = y  (roots first).  X2 holds y and the running updates, the solved blocks x
   //                  land in X; ancestors' final rows are read from X through the row lists.
   for (int d = 0; d < S.nlevels; d++) {
-    int max_nob = 0;
-    for (int q = S.level_ptr[d]; q < S.level_ptr[d + 1]; q++) {
-      const int s = S.level_sn[q];
-      max_nob = std::max(max_nob, num_outer(S.sn_first[s + 1] - S.sn_first[s]));
-    }
+    const int max_nob = max_outer(S, d);
     for (int ph = 0; ph < 2 * max_nob + 1; ph++) {
       bool updated = false;
       for (int q = S.level_ptr[d]; q < S.level_ptr[d + 1]; q++) {
-        const int s = S.level_sn[q];
-        const int f = S.sn_first[s], ns = S.sn_first[s + 1] - f, ms = S.sn_nrow[s], rs = ms - ns;
-        const int nob = num_outer(ns);
-        double* P = h->Lx.get() + S.sn_lptr[s];
-        const int64_t ld = panel_ld(ms);
-        double* Xs = pl->X.get() + (int64_t)f * R;
-        double* Ys = pl->X2.get() + (int64_t)f * R;
+        const Front F = front(h, S.level_sn[q]);
+        const int nob = num_outer(F.ns);
+        double* Xs = pl->X.get() + (int64_t)F.f * R;
+        double* Ys = pl->X2.get() + (int64_t)F.f * R;
         if (ph == 0) {                             // y_top -= L21' x[rows below]   (gathered rows of X)
-          if (rs > 0)
-            pb.add(make_op(Ys, 1, R, pl->X.get(), 1, R, P + ns, ld, 1, nrhs, ns, rs, GF_ACCUM | GF_NEG,
-                           h->d_rows.get() + S.sn_rowptr[s] + ns));
+          if (F.rs > 0)
+            pb.add(make_op(Ys, 1, R, pl->X.get(), 1, R, F.P + F.ns, F.ld, 1, nrhs, F.ns, F.rs, GF_ACCUM | GF_NEG,
+                           h->d_rows.get() + S.sn_rowptr[F.s] + F.ns));
           continue;
         }
         const int step = ph - 1, r = step / 2;     // outer blocks in reverse order
         if (r >= nob) continue;
-        const OuterBlock b = outer_block(h, s, nob - 1 - r);
+        const OuterBlock b = outer_block(h, F, nob - 1 - r);
         if (step % 2 == 0) {                       // x_b = Winv' * y_b
           pb.add(make_op(Xs + (int64_t)b.o0 * R, 1, R, Ys + (int64_t)b.o0 * R, 1, R, b.winv, b.ldw, 1, nrhs, b.nbo,
                          b.nbo, 0));
@@ -1303,28 +1279,27 @@ static SolvePlan* get_plan(slmm_chol* h, int nrhs) {
           const int p0 = b.o0 - NBO;               // the block solved next is [p0, o0)
           const bool split = lookahead && p0 >= NBO;
           const int lo = split ? p0 : 0;
-          pb.add(make_op(Ys + (int64_t)lo * R, 1, R, Xs + (int64_t)b.o0 * R, 1, R, P + b.o0 + (int64_t)lo * ld, ld, 1, nrhs,
-                         b.o0 - lo, b.nbo, GF_ACCUM | GF_NEG));
+          pb.add(make_op(Ys + (int64_t)lo * R, 1, R, Xs + (int64_t)b.o0 * R, 1, R, F.P + b.o0 + (int64_t)lo * F.ld, F.ld,
+                         1, nrhs, b.o0 - lo, b.nbo, GF_ACCUM | GF_NEG));
           if (split)
-            pb_rest.add(make_op(Ys, 1, R, Xs + (int64_t)b.o0 * R, 1, R, P + b.o0, ld, 1, nrhs, p0, b.nbo,
+            la.bulk.add(make_op(Ys, 1, R, Xs + (int64_t)b.o0 * R, 1, R, F.P + b.o0, F.ld, 1, nrhs, p0, b.nbo,
                                 GF_ACCUM | GF_NEG));
         }
       }
-      flush_pair(pl->bwd, updated);
+      la.flush_phase(pl->bwd, updated);
     }
-    if (last_bulk_ev >= 0) { pl->bwd.launches.push_back({Launch::EV_WAIT, 0, last_bulk_ev, 0, 0, 0.0, 0, 0}); last_bulk_ev = -1; }
+    la.end_level(pl->bwd);
   }
   // ---------------- L * Z  (same dataflow as the forward sweep, products instead of solves)
   for (int d = S.nlevels - 1; d >= 0; d--) {
     for (int q = S.level_ptr[d]; q < S.level_ptr[d + 1]; q++) {
-      const int s = S.level_sn[q];
-      const int f = S.sn_first[s], ns = S.sn_first[s + 1] - f, ms = S.sn_nrow[s], rs = ms - ns;
-      double* P = h->Lx.get() + S.sn_lptr[s];
-      const int64_t ld = panel_ld(ms);
+      const Front F = front(h, S.level_sn[q]);
       // out_top = L11 z_top (upper part of the diagonal block is stored as zeros)
-      pb.add(make_op(pl->X2.get() + (int64_t)f * R, 1, R, pl->X.get() + (int64_t)f * R, 1, R, P, 1, ld, nrhs, ns, ns, GF_TRIL_B));
-      if (rs > 0)
-        pb.add(make_op(pl->arena[d & 1].get() + vptr[s], 1, R, pl->X.get() + (int64_t)f * R, 1, R, P + ns, 1, ld, nrhs, rs, ns, 0));
+      pb.add(make_op(pl->X2.get() + (int64_t)F.f * R, 1, R, pl->X.get() + (int64_t)F.f * R, 1, R, F.P, 1, F.ld, nrhs, F.ns,
+                     F.ns, GF_TRIL_B));
+      if (F.rs > 0)
+        pb.add(make_op(pl->arena[d & 1].get() + vptr[F.s], 1, R, pl->X.get() + (int64_t)F.f * R, 1, R, F.P + F.ns, 1, F.ld,
+                       nrhs, F.rs, F.ns, 0));
     }
     pb.flush(pl->lmul);
     add_pull_items(pl->lmul, S, vptr, d, 2, Launch::PULL_VEC, 4);
@@ -1435,6 +1410,8 @@ int slmm_chol_analyze(int32_t n, const int32_t* indptr, const int32_t* indices, 
     h->ev_aux = make_event(cudaEventDisableTiming);
     h->ev_fork = make_event(cudaEventDisableTiming);
     h->ev_join = make_event(cudaEventDisableTiming);
+    h->tl_fork = make_event(cudaEventDefault);
+    h->tl_join = make_event(cudaEventDefault);
   }
   CUDA_OK(cudaMemset(h->Lx.get(), 0, S.lsize * sizeof(double)));
   build_factor_schedule(h.get());
@@ -1659,12 +1636,12 @@ int slmm_chol_export_L(slmm_chol_t* h, int64_t* colptr, int32_t* rowidx, double*
   CUDA_OK(cudaMemcpy(Lh.data(), h->Lx.get(), S.lsize * sizeof(double), cudaMemcpyDeviceToHost));
   int64_t q = 0;
   for (int s = 0; s < S.nsuper; s++) {
-    const int f = S.sn_first[s], ns = S.sn_first[s + 1] - f, ms = S.sn_nrow[s];
+    const Front F = front(h, s);
     const int32_t* rows = S.rows.data() + S.sn_rowptr[s];
     const double* P = Lh.data() + S.sn_lptr[s];
-    for (int c = 0; c < ns; c++) {
-      colptr[f + c] = q;
-      for (int r = c; r < ms; r++) { rowidx[q] = rows[r]; values[q] = P[r + (int64_t)c * panel_ld(ms)]; q++; }
+    for (int c = 0; c < F.ns; c++) {
+      colptr[F.f + c] = q;
+      for (int r = c; r < F.ms; r++) { rowidx[q] = rows[r]; values[q] = P[r + (int64_t)c * F.ld]; q++; }
     }
   }
   colptr[S.n] = q;
@@ -1736,10 +1713,10 @@ int slmm_chol_get_timeline(slmm_chol_t* h, int32_t max_n, int32_t* n_out, float*
   if (ms) {
     std::vector<int> rec_stream(std::max(0, n - 2), 0);
     for (const Launch& L : h->fact.launches)
-      if (L.kind == Launch::EV_RECORD && L.count + 2 < n) rec_stream[L.count] = L.stream;
+      if (L.kind == Launch::EV_RECORD && L.event() + 2 < n) rec_stream[L.event()] = L.stream;
     for (int q = 0; q < n && q < max_n; q++) {
       float v = 0.f;
-      if (q > 0) CUDA_OK(cudaEventElapsedTime(&v, h->tl_events[0].get(), h->tl_events[q].get()));
+      if (q > 0) CUDA_OK(cudaEventElapsedTime(&v, h->tl_fork.get(), (q == 1 ? h->tl_join : h->tl_events[q - 2]).get()));
       ms[q] = v;
       if (stream) stream[q] = q >= 2 ? rec_stream[q - 2] : 0;
     }
@@ -1757,10 +1734,10 @@ int slmm_chol_get_launch_timeline(slmm_chol_t* h, int32_t max_n, int32_t* n_out,
   const int n = (int)std::min(ks.size(), h->tl_launch.size());
   *n_out = n;
   for (int q = 0; q < n && q < max_n; q++) {
-    if (end_ms) { float v = 0.f; CUDA_OK(cudaEventElapsedTime(&v, h->tl_events[0].get(), h->tl_launch[q].get())); end_ms[q] = v; }
+    if (end_ms) { float v = 0.f; CUDA_OK(cudaEventElapsedTime(&v, h->tl_fork.get(), h->tl_launch[q].get())); end_ms[q] = v; }
     if (stream) stream[q] = ks[q]->stream;
     if (kind) kind[q] = (int)ks[q]->kind;
-    if (grid) grid[q] = (ks[q]->kind <= Launch::GEMM_SMALL || ks[q]->kind >= Launch::SKINNY_F1) ? ks[q]->grid : ks[q]->count;
+    if (grid) grid[q] = work_size(*ks[q]);
     if (flops) flops[q] = ks[q]->flops;
   }
   return SLMM_OK;

@@ -9,7 +9,8 @@ doubling steps.  The golden pedigrees never reach a front wider than 64 columns,
 with one front of a chosen (ns, rs) = (columns, rows below) and asserts that the analysis really has it.
 
 Every check runs on the functor's own device factor:
-  * L against scipy.linalg.cholesky, logdet against slogdet, panels of two factorizations bit for bit;
+  * L against scipy.linalg.cholesky, logdet against slogdet; the panels of a second factorization, of a profiled one
+    (one stream, launch by launch) and of a timeline one (look-ahead streams with timed events) bit for bit;
   * per RHS width (every streaming-kernel family, the tile path, look-ahead from 64 columns, more than 160 columns):
     mode 0 (V^-1 B), mode 1 (forward half L^-1 P B), mode 2 (backward half P' L^-T B) and L*Z against LAPACK,
     mode 2 after mode 1 equal to mode 0 bit for bit;
@@ -161,19 +162,31 @@ class BlockDiagRef(object):
 
 
 def check_factor_and_solves(slmm, eng, Vs, make_ref):
-    """Factor Vs (natural order) twice with one functor and check the factor and every solve mode at every width
-    against LAPACK, then once more bit for bit after the solve plans were evicted and rebuilt."""
+    """Factor Vs (natural order) twice with one functor, then profiled and in timeline mode, all bit for bit; check the
+    factor and every solve mode at every width against LAPACK, then once more bit for bit after the solve plans were
+    evicted and rebuilt."""
     chol = slmm.SparseCholesky(ordering_method="natural")
     f = chol(Vs)
     panels = f._chol.panels()
     f = chol(Vs)
     assert np.array_equal(f._chol.panels(), panels), "two factorizations differ"
+    dev = f._chol
+    vals = eng.to_device(eng.canonical_csr(sp.csr_matrix(Vs)).data)
+    for run in ("profiled", "timeline"):
+        dev.add_values(dev._self_map, vals.data_ptr(), 1.0, True)
+        if run == "profiled":
+            dev.set_profiling(True)
+            dev.factorize()
+            dev.set_profiling(False)
+        else:
+            dev.timeline()
+        assert np.array_equal(dev.panels(), panels), "%s factorization differs" % run
+    f = slmm.B200Factor(dev)
     ref = make_ref(f.P())
     n = Vs.shape[0]
     ld = ref.logdet()
     assert abs(f.logdet() - ld) <= 1e-10 * abs(ld), (f.logdet(), ld)
     assert ref.L_err(f.L()) < 1e-11
-    dev = f._chol
     first = {}
     for rep in range(2):
         for k in WIDTHS:

@@ -271,7 +271,8 @@ def test_aux_solve_with_the_same_width_as_the_probe_block(golden_c1mini, slmm):
 
 def test_graph_replay_equals_launch_by_launch(golden_c1mini, slmm, eng):
     """Schedules replayed from CUDA graphs give bit-identical factors / solves to the launch-by-launch walk
-    (profiling mode walks the list eagerly on one stream)."""
+    (profiling mode walks the list eagerly on one stream), and so does the same solve replayed on the auxiliary
+    stream inside an auxiliary section."""
     g = golden_c1mini
     f = slmm.SparseCholesky()(g.csc("V_k4"))
     B = np.random.default_rng(4).standard_normal((g.n, 40))
@@ -284,6 +285,14 @@ def test_graph_replay_equals_launch_by_launch(golden_c1mini, slmm, eng):
     x2, ld2 = f2(B), f2.logdet()
     e.set_profiling(False)
     assert ld1 == ld2 and np.array_equal(x1, x2)
+    Bd = eng.to_device(B)
+    e.aux_begin()
+    try:
+        e.solve_(Bd)
+    finally:
+        e.aux_end()
+    e.aux_join()
+    assert np.array_equal(Bd.cpu().numpy(), x1), "solve in an auxiliary section"
 
 
 def test_cholmod_lower_triangle_rule(golden_small, slmm):
