@@ -280,6 +280,23 @@ int slmm_assoc_genotypes(const int8_t* d_G, int64_t n, int32_t b, int64_t row_st
                          const double* d_P, int32_t np, double* d_X, double* d_proj, int64_t* d_nobs, int64_t* d_sum);
 int slmm_assoc_colsumsq(const double* d_F, int64_t n, int32_t b, double* d_out);
 
+/* ------------------------------------------------------------------ predicted random effects (BLUP) ---- */
+/* Column-mapped products of the relationship matrices over ALL N individuals of the set with blocks over the n
+ * observed ones (the individuals the fit used).  The reference has no counterpart.  Both calls take one pattern group:
+ * nk <= 2 matrices ks[] of the set sharing one sparsity pattern (slmm_matset_pattern_id), with host weights
+ * sigmas[nk].  d_colmap[N] (int32, device) sends column j of A to row d_colmap[j] < nobs of the block, or -1 to skip
+ * the entry (an individual without a phenotype); NULL is the identity and needs nobs == N.  The map is checked on the
+ * device before the pass: an entry outside [-1, nobs) returns SLMM_ERR_INVALID.  Warp per row, entries in stored
+ * order, no atomics: the results are the same bits on every run.
+ *   slmm_blup_spmm: d_out[(g*N + i)*ncols + j] = sigmas[g] * sum_l A_ks[g][i, l] X[map(l), j] for the C-ordered
+ *     nobs x ncols block d_X, ncols <= 32 (u = V^-1 r and V^-1 C in one pass).
+ *   slmm_blup_rowsumsq: with t_ij = sigmas[g] * (A_ks[g][i, obs] W)_ij for the C-ordered nobs x ncols probe block d_W
+ *     (ncols <= 128), d_sum2[i*nk + g] = sum_j t_ij^2 and d_sum4[i*nk + g] = sum_j t_ij^4.  t is not stored. */
+int slmm_blup_spmm(slmm_matset_t* ms, int32_t nk, const int32_t* ks, const double* sigmas, const int32_t* d_colmap,
+                   const double* d_X, int64_t nobs, int32_t ncols, double* d_out);
+int slmm_blup_rowsumsq(slmm_matset_t* ms, int32_t nk, const int32_t* ks, const double* sigmas, const int32_t* d_colmap,
+                       const double* d_W, int64_t nobs, int32_t ncols, double* d_sum2, double* d_sum4);
+
 /* ------------------------------------------------------------------ IBD matrix construction ----------- */
 /* The step before the path (SURVEY 8f-1): numerator relationship matrix from a child -> parents matrix, replacing
  * Matrices/Numerator.py LD() :5-34 (per-individual Python loop) and create_numerator() :37-38 (L D L').  h_rel_*:

@@ -474,6 +474,53 @@ class RemlSession(object):
             torch.cuda.synchronize()                   # no copy may still target the buffers when they are freed
         return out
 
+    def blup(self, sigmas, matset, groups, colmap=None, probes=0, block_begin=0, block_end=None):
+        """Device side of blup(): the predicted random effects of the K matrices of `matset` (over all N individuals;
+        `groups`: their pattern groups of <= 2) from this session's fit on the observed individuals, at `sigmas` (this
+        session's components, the residual last).  colmap: device int32 map of the N columns to this session's rows
+        (-1 = no phenotype) or None when the matset is this session's own.  In the units of the standardised y.
+
+        Returns a dict: U (N x K, sigma_k A_k[:, obs] u with u = V^-1 (y_s - C beta)), u (n), beta, corr (N x K, the
+        fixed-effect term diag(sigma_k A_k V^-1 C M^-1 C'V^-1 A_k sigma_k) of the PEV, M = C'V^-1 C) and, with
+        probes > 0, parts: one [nblocks, 2, N, G] CUDA tensor per group holding sum_j t_ij^2 and sum_j t_ij^4 of
+        t = sigma_k A_k[:, obs] W for the probe blocks [block_begin, block_end) of BLUP_BLOCK columns (other slots 0).
+        W = P' L^-T Z with Z from the device Philox stream (functor.seed, BLUP_PROBE_STREAM) whatever functor.rng is,
+        one block of columns at a time (the draw and backward half-sweep of probes() for rng='device')."""
+        torch = self.torch
+        c = self.C.shape[1]
+        if c + 1 > BLUP_MAX_COLUMNS:
+            raise ValueError("blup takes at most %d covariates, got %d" % (BLUP_MAX_COLUMNS - 1, c))
+        self.factor_at(sigmas)
+        ViC, chol, beta, Viy = self.fixed_effects()
+        u = Viy - ViC @ torch.from_numpy(beta).to("cuda")
+        X = torch.cat([u.unsqueeze(1), ViC], dim=1).contiguous()          # [u | V^-1 C], c + 1 <= 32 columns
+        Minv = torch.from_numpy(la.cho_solve(chol, np.eye(c))).to("cuda")
+        N, K = matset.n, len(sigmas) - 1
+        U = torch.empty(N, K, dtype=torch.float64, device="cuda")
+        corr = torch.empty(N, K, dtype=torch.float64, device="cuda")
+        for ks in groups:
+            Y = matset.blup_spmm(ks, [sigmas[k] for k in ks], X, colmap)
+            for g, k in enumerate(ks):
+                U[:, k] = Y[g, :, 0]
+                Yc = Y[g, :, 1:]
+                corr[:, k] = ((Yc @ Minv) * Yc).sum(dim=1)
+        out = {"U": U, "u": u, "beta": beta, "corr": corr}
+        if probes <= 0:
+            return out
+        nblocks = -(-int(probes) // BLUP_BLOCK)
+        block_end = nblocks if block_end is None else block_end
+        parts = [torch.zeros(nblocks, 2, N, len(ks), dtype=torch.float64, device="cuda") for ks in groups]
+        for b in range(block_begin, block_end):
+            c0 = b * BLUP_BLOCK
+            w = min(int(probes), c0 + BLUP_BLOCK) - c0
+            Z = self.eng.probe_normals(self.n, w, c0, self.functor.seed, BLUP_PROBE_STREAM)
+            W = self.eng.solve_(Z, mode=3)
+            for ks, part in zip(groups, parts):
+                matset.blup_rowsumsq(ks, [sigmas[k] for k in ks], W, part[b, 0], part[b, 1], colmap)
+            del Z, W
+        out["parts"] = parts
+        return out
+
     def _is_identity(self, k):
         m = self.mats_host[k]
         return m.nnz == self.n and np.array_equal(m.indices, np.arange(self.n)) and np.all(m.data == 1.0)
@@ -933,6 +980,125 @@ def association(cholesky_func, mats, covariates, y, sigmas, G):
     part["beta"] = part["beta"] * scale
     part["se"] = part["se"] * scale
     return {k: part[k] for k in keys}
+
+
+# ------------------------------------------------------------------------------------------- predicted random effects
+BLUP_MAX_COLUMNS = 32       # [u | V^-1 C] goes through slmm_blup_spmm in one pass, one column per lane (csrc/blup.cu)
+BLUP_BLOCK = 128            # probe columns per block of the PEV estimate (one mode-3 sweep, one rowsumsq pass)
+BLUP_PROBE_STREAM = 2 ** 62   # Philox stream of the PEV probes: REML evaluations count their streams up from 0
+
+
+def blup(cholesky_func, mats, covariates, y, sigmas, pev_probes=0):
+    """Predicted random effects (BLUP) of every individual, phenotyped or not, at the variance components `sigmas`.
+
+    mats: the K relationship matrices over all N individuals, without the identity (as for REML()).  covariates: N x c,
+    finite on every row (the unphenotyped rows give their fixed part); c + 1 <= 32.  y: length N, NaN for an individual
+    without a phenotype.  sigmas: REML()['covariance coefficients'] (K + 1 values, the residual last) of the fit on the
+    phenotyped individuals:
+
+        obs = ~np.isnan(y)
+        sigmas = REML(chol, [A[obs][:, obs] for A in mats], covariates[obs], y[obs])['covariance coefficients']
+
+    The model is REML's: s = y[obs].std(), y_s = y[obs] / s, V = sum_k sigma_k A_k[obs, obs] + sigma_e I,
+    u = V^-1 (y_s - C beta) with the GLS beta.  Returns a dict:
+      u: N x K, u_k = s sigma_k A_k[:, obs] u (the usual BLUP on the phenotyped rows, E[u_k | y] on the others);
+      residual: length N, s sigma_e u on the phenotyped rows, NaN elsewhere;
+      fixed: length N, s C beta;  beta: s beta;  yhat: fixed + u.sum(1).
+    With pev_probes = p >= 2, also N x K arrays (units of y^2 for the first two):
+      pev: prediction error variance sigma_k A_k,ii - sigma_k^2 (A_k P A_k)_ii, P = V^-1 - V^-1 C M^-1 C'V^-1,
+        M = C'V^-1 C.  The fixed-effect term is exact; diag(A_k V^-1 A_k) is a Monte Carlo estimate from p probe
+        columns W = P' L^-T Z (E[W W'] = V^-1), about sqrt(2 / p) relative error per entry (12 % at 128, 4 % at 1024);
+      pev_se: its Monte Carlo standard error;
+      reliability: 1 - pev / (sigma_k A_k,ii), NaN where that is 0.
+    The probes always come from the device Philox stream keyed by the functor's `seed` (stream BLUP_PROBE_STREAM,
+    which no REML evaluation uses), whatever its `rng` setting: the same seed gives the same bits.
+
+    Without a NaN in y this is the in-sample prediction and a call after REML() on the same functor and inputs reuses
+    its device session.  With NaN the phenotyped blocks A_k[obs][:, obs] are cut on the host and a session is set up on
+    them (the cached analysis is reused when their pattern is the one REML() fitted); like any new session on the
+    functor, it replaces the one REML() left, so a later call on the full inputs sets its session up again.  With
+    torch.distributed initialised every rank sweeps a slice of the probe blocks; the PEV is the same bits for any
+    number of ranks."""
+    functor = _need_functor(cholesky_func)
+    torch = _eng.require_cuda()
+    y = np.asarray(y, dtype=np.float64)
+    C = np.asarray(covariates, dtype=np.float64)
+    K = len(mats)
+    N = y.shape[0]
+    if y.ndim != 1:
+        raise ValueError("y must be a vector")
+    if K == 0 or any(m.shape != (N, N) for m in mats):
+        raise ValueError("every matrix must be N x N with N = len(y) = %d" % N)
+    sigmas = np.asarray(sigmas, dtype=float)
+    if sigmas.shape != (K + 1,):
+        raise ValueError("need %d variance components (the residual last), got %d" % (K + 1, sigmas.size))
+    if C.ndim != 2 or C.shape[0] != N:
+        raise ValueError("covariates must be N x c with N = %d" % N)
+    if not np.all(np.isfinite(C)):
+        raise ValueError("covariates must be finite on every row, the unphenotyped ones included")
+    if C.shape[1] + 1 > BLUP_MAX_COLUMNS:
+        raise ValueError("blup takes at most %d covariates, got %d" % (BLUP_MAX_COLUMNS - 1, C.shape[1]))
+    if np.any(np.isinf(y)):
+        raise ValueError("y must be finite or NaN (no phenotype)")
+    obs = ~np.isnan(y)
+    n = int(obs.sum())
+    if n < C.shape[1] + 1:
+        raise ValueError("need at least c + 1 = %d phenotyped individuals, got %d" % (C.shape[1] + 1, n))
+    p = int(pev_probes)
+    if p < 0 or p == 1:
+        raise ValueError("pev_probes must be 0 or at least 2")
+    scale = y[obs].std()
+    if n == N:
+        ses = _scan_session(functor, mats, covariates, y / scale)
+        matset = ses.matset
+        groups = [[k for k in ks if k < K] for ks in ses._groups]
+        groups = [ks for ks in groups if ks]
+        colmap = None
+    else:
+        idx = np.flatnonzero(obs)
+        sub = [_eng.canonical_csr(m)[idx][:, idx] for m in mats]
+        ses = _scan_session(functor, sub, C[idx], y[idx] / scale)
+        matset = _eng.MatSet(mats)
+        groups = matset.pattern_groups(2)
+        colmap = np.full(N, -1, dtype=np.int32)
+        colmap[idx] = np.arange(n, dtype=np.int32)
+        colmap = _eng.to_device(colmap, torch)
+    rank, world = _shard.rank_world()
+    nblocks = -(-p // BLUP_BLOCK)
+    lo, hi = _shard.column_block(nblocks, rank, world)
+    res = ses.blup(sigmas, matset, groups, colmap, p, lo, hi)
+    U = res["U"].cpu().numpy()
+    resid = np.full(N, np.nan)
+    resid[obs] = sigmas[-1] * res["u"].cpu().numpy()
+    fixed = C @ res["beta"]
+    out = {"u": scale * U, "residual": scale * resid, "fixed": scale * fixed, "yhat": scale * (fixed + U.sum(axis=1)),
+           "beta": scale * res["beta"]}
+    if p == 0:
+        return out
+    # every rank filled its own blocks' slots and zeros elsewhere: the sum over ranks adds exact zeros, and the
+    # blocks are then added in one fixed order, so the estimate is the same bits for any number of ranks
+    flat = torch.cat([part.reshape(-1) for part in res["parts"]])
+    _shard.allreduce_sum_(flat)
+    s2 = torch.empty(N, K, dtype=torch.float64, device="cuda")
+    s4 = torch.empty(N, K, dtype=torch.float64, device="cuda")
+    off = 0
+    for ks, part in zip(groups, res["parts"]):
+        part = flat[off:off + part.numel()].view(part.shape)
+        off += part.numel()
+        acc = part[0].clone()
+        for b in range(1, nblocks):
+            acc += part[b]
+        for g, k in enumerate(ks):
+            s2[:, k], s4[:, k] = acc[0, :, g], acc[1, :, g]
+    diag = np.stack([sigmas[k] * _eng.canonical_csr(m).diagonal() for k, m in enumerate(mats)], axis=1)
+    s2, s4, corr = s2.cpu().numpy(), s4.cpu().numpy(), res["corr"].cpu().numpy()
+    pev = diag - s2 / p + corr
+    se = np.sqrt(np.maximum(s4 - s2 * s2 / p, 0.0) / (p * (p - 1.0)))
+    with np.errstate(invalid="ignore", divide="ignore"):
+        out["reliability"] = np.where(diag != 0, 1.0 - pev / np.where(diag != 0, diag, 1.0), np.nan)
+    out["pev"] = scale * scale * pev
+    out["pev_se"] = scale * scale * se
+    return out
 
 
 # ------------------------------------------------------------------------------------------- Haseman-Elston

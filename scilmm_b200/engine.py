@@ -436,6 +436,45 @@ class MatSet(object):
                                         dots.data_ptr(), half.data_ptr() if nb > 0 else None))
         return dots, (half + half.transpose(1, 2)) if nb > 0 else None
 
+    def _blup_args(self, ks, sigmas, colmap, X, max_cols):
+        """(ks, sigmas, device map or None, contiguous X) for the two BLUP passes; a host map is uploaded (the library
+        checks the entries of the map on the device)."""
+        torch = _torch()
+        X2 = X.contiguous()
+        if X2.dim() != 2 or X2.dtype != torch.float64 or not X2.is_cuda or not 1 <= X2.shape[1] <= max_cols:
+            raise ValueError("need a CUDA float64 block of 1 to %d columns" % max_cols)
+        if colmap is not None:
+            if not torch.is_tensor(colmap):
+                colmap = to_device(np.ascontiguousarray(colmap, dtype=np.int32), torch)
+            if colmap.shape != (self.n,) or colmap.dtype != torch.int32 or not colmap.is_cuda \
+                    or not colmap.is_contiguous():
+                raise ValueError("the column map needs n contiguous int32 entries")
+        return (np.asarray(ks, dtype=np.int32), np.asarray(sigmas, dtype=np.float64), colmap, X2)
+
+    def blup_spmm(self, ks, sigmas, X, colmap=None):
+        """Y[g] = sigmas[g] A_ks[g][:, obs] X for matrices `ks` (<= 2, one pattern) over all n rows: a [len(ks), n,
+        ncols] CUDA tensor (slmm_blup_spmm).  X: nobs x ncols (<= 32) CUDA float64 block over the observed individuals;
+        colmap: n int32 entries, column j of A -> row of X or -1 to skip (host array, uploaded here, or a CUDA tensor);
+        None = the identity (nobs = n)."""
+        torch = _torch()
+        ks, sig, cm, X2 = self._blup_args(ks, sigmas, colmap, X, 32)
+        out = torch.empty(len(ks), self.n, X2.shape[1], dtype=torch.float64, device="cuda")
+        check(lib().slmm_blup_spmm(self._h, len(ks), np_ptr(ks), np_ptr(sig), None if cm is None else cm.data_ptr(),
+                                   X2.data_ptr(), int(X2.shape[0]), int(X2.shape[1]), out.data_ptr()))
+        return out
+
+    def blup_rowsumsq(self, ks, sigmas, W, sum2, sum4, colmap=None):
+        """sum2[i, g] = sum_j t_ij^2 and sum4[i, g] = sum_j t_ij^4 for t = sigmas[g] A_ks[g][i, obs] W, into the
+        contiguous (n, len(ks)) CUDA float64 tensors sum2 / sum4 (slmm_blup_rowsumsq).  W: nobs x ncols (<= 128) probe
+        block; colmap as for blup_spmm."""
+        ks, sig, cm, W2 = self._blup_args(ks, sigmas, colmap, W, 128)
+        for s in (sum2, sum4):
+            if not s.is_contiguous() or s.numel() != self.n * len(ks):
+                raise ValueError("sum2 / sum4 need n * len(ks) contiguous entries")
+        check(lib().slmm_blup_rowsumsq(self._h, len(ks), np_ptr(ks), np_ptr(sig), None if cm is None else cm.data_ptr(),
+                                       W2.data_ptr(), int(W2.shape[0]), int(W2.shape[1]), sum2.data_ptr(),
+                                       sum4.data_ptr()))
+
     def is_symmetric(self, k):
         v = C.c_int32(0)
         check(lib().slmm_matset_is_symmetric(self._h, int(k), C.byref(v)))
