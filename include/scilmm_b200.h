@@ -279,6 +279,14 @@ int slmm_symbolic_entry_map_tri(const slmm_symbolic_t* s, const int32_t* h_indpt
 int slmm_assoc_genotypes(const int8_t* d_G, int64_t n, int32_t b, int64_t row_stride, int64_t col_stride,
                          const double* d_P, int32_t np, double* d_X, double* d_proj, int64_t* d_nobs, int64_t* d_sum);
 int slmm_assoc_colsumsq(const double* d_F, int64_t n, int32_t b, double* d_out);
+/* Region tests (burden, SKAT): the full Gram of each region of a swept block.  d_F is the C-ordered n x b block F = L^-1
+ * P x~; h_bounds (host, nregions + 1 entries) cuts its columns into regions [h_bounds[r], h_bounds[r+1]), starting at 0,
+ * strictly increasing, at most 512 columns each, ending at b.  d_out receives F_r' F_r (w_r x w_r, row-major) of every
+ * region, packed one after another at offset sum_{r' < r} w_r'^2.  Each square is symmetric bit for bit, and its bits
+ * depend only on the region's columns of F, not on where they sit in the block.  No atomics.  Bad bounds return
+ * SLMM_ERR_INVALID before any device work. */
+int slmm_assoc_region_gram(const double* d_F, int64_t n, int32_t b, int32_t nregions, const int32_t* h_bounds,
+                           double* d_out);
 
 /* ------------------------------------------------------------------ predicted random effects (BLUP) ---- */
 /* Column-mapped products of the relationship matrices over ALL N individuals of the set with blocks over the n

@@ -20,6 +20,7 @@ import scipy.linalg as la
 import scipy.optimize as optimize
 import scipy.sparse as sparse
 import scipy.special as special
+import scipy.stats as stats
 
 from . import engine as _eng
 from . import sharding as _shard
@@ -370,17 +371,97 @@ class RemlSession(object):
             Z = Z[:, col_begin:col_end].clone(memory_format=torch.contiguous_format)
         return self.eng.solve_(Z, mode=3)
 
+    def _scan_blocks(self, sigmas, G, spans, red_len, reduce, finish, timing=None):
+        """The genotype block pipeline of the association scan and the region tests.  For each column span (j0, j1) of
+        the host (n, m) int8 matrix G, in order: int8 upload on a copy stream (span i + 1 goes up while span i is
+        swept), one decode / centre / project kernel, one forward half-sweep F = L^-1 P x~ (solve mode 1), then
+        reduce(i, F, buf), which queues the device reduction of span i's F into the float64 buffer buf of red_len(i)
+        entries.  While the device sweeps span i, the host calls finish(i - 1, chol, q, t, nobs, gsum, red) with the
+        host copies of span i - 1's projections q = (V^-1 C)' x~ (c x w) and t = (V^-1 r)' x~ (w), its non-missing
+        counts and allele sums, and its reduction; chol is the Cholesky factor of C'V^-1 C (scipy.linalg.cho_factor).
+        timing: a list that receives, per span, five timing events recorded on the compute stream around the upload
+        wait, the genotype kernel, the sweep and the reduction (scripts/assoc_scan.py, scripts/region_scan.py)."""
+        torch = self.torch
+        n = self.n
+        self.factor_at(sigmas)
+        ViC, chol, beta, Viy = self.fixed_effects()
+        Vir = Viy - ViC @ torch.from_numpy(beta).to("cuda")
+        P = torch.cat([ViC, Vir.unsqueeze(1)], dim=1).contiguous()       # n x (c + 1)
+        c1 = P.shape[1]
+        block = max(j1 - j0 for j0, j1 in spans)
+        nred = max(red_len(i) for i in range(len(spans)))
+        # one int8 buffer: the upload of span i + 1 is issued after assoc_genotypes has returned for span i, and that
+        # call waits for its kernels (device-side input check), so nothing still reads the buffer
+        g8 = torch.empty(n * block, dtype=torch.int8, device="cuda")
+        X = torch.empty(n * block, dtype=torch.float64, device="cuda")
+        small = [dict(proj=torch.empty(c1 * block, dtype=torch.float64, device="cuda"),
+                      nobs=torch.empty(block, dtype=torch.int64, device="cuda"),
+                      gsum=torch.empty(block, dtype=torch.int64, device="cuda"),
+                      red=torch.empty(nred, dtype=torch.float64, device="cuda")) for _ in range(2)]
+        if getattr(self, "_copy_stream", None) is None:
+            self._copy_stream = torch.cuda.Stream()
+        copy, main = self._copy_stream, torch.cuda.current_stream()
+        uploaded = torch.cuda.Event()
+        strides = [None]
+        finish_s = self.last["finish_s"] = []          # host seconds per span: copies back + finish
+
+        def upload(i):
+            strides[0] = _eng.upload_genotype_block(G, spans[i][0], spans[i][1], g8, copy)
+            uploaded.record(copy)
+
+        def collect(i):
+            """Host copies of span i's small outputs, whose kernels have completed.  They come back on the copy
+            stream, so the host does not wait behind the sweep of span i + 1 queued on the compute stream."""
+            w = spans[i][1] - spans[i][0]
+            s = small[i % 2]
+            t0 = time.perf_counter()
+            with torch.cuda.stream(copy):
+                proj = s["proj"][:c1 * w].view(c1, w).cpu().numpy()
+                red = s["red"][:red_len(i)].cpu().numpy()
+                nobs, gsum = s["nobs"][:w].cpu().numpy(), s["gsum"][:w].cpu().numpy()
+            finish(i, chol, proj[:c1 - 1], proj[c1 - 1], nobs, gsum, red)
+            finish_s.append(time.perf_counter() - t0)
+
+        def mark(marks):
+            if marks is not None:
+                marks.append(torch.cuda.Event(enable_timing=True))
+                marks[-1].record(main)
+
+        upload(0)
+        try:
+            for i, (j0, j1) in enumerate(spans):
+                w = j1 - j0
+                s = small[i % 2]
+                Xb = X[:n * w].view(n, w)
+                marks = None if timing is None else []
+                mark(marks)
+                main.wait_event(uploaded)
+                mark(marks)
+                # returns once the kernels are done (device-side input check): span i - 1 is swept and reduced by then
+                _eng.assoc_genotypes(g8, n, w, strides[0], P, Xb, s["proj"], s["nobs"], s["gsum"])
+                mark(marks)
+                self.eng.solve_(Xb, mode=1)
+                mark(marks)
+                reduce(i, Xb, s["red"])
+                mark(marks)
+                if timing is not None:
+                    timing.append(marks)
+                # while the device sweeps span i: statistics of span i - 1, then the host stages span i + 1
+                if i > 0:
+                    collect(i - 1)
+                if i + 1 < len(spans):
+                    upload(i + 1)
+            main.synchronize()
+            collect(len(spans) - 1)
+        finally:
+            torch.cuda.synchronize()                   # no copy may still target the buffers when they are freed
+
     def association(self, sigmas, G, block, col_begin=0, col_end=None, timing=None):
         """Mixed-model association test of the variants (columns) [col_begin, col_end) of the host (n, m) int8 genotype
         matrix G at the variance components `sigmas` (see association() for the statistic), in blocks of `block`
-        variants.  Per block: int8 upload on a copy stream (the next block goes up while this one is swept), one
-        decode / centre / project kernel, one forward half-sweep F = L^-1 P x~ (solve mode 1), one column sum of
-        squares, and the c x c finalisation on the host.  Returns a dict of arrays of length col_end - col_begin in the
-        units of the standardised y: beta, se, chi2, p, af, n_obs.  timing: a list that receives, per block, five
-        timing events recorded on the compute stream around the upload wait, the genotype kernel, the sweep and the
-        sum of squares (scripts/assoc_scan.py)."""
-        torch = self.torch
-        n = self.n
+        variants through _scan_blocks, with a column sum of squares as the reduction and the c x c finalisation on the
+        host.  Returns a dict of arrays of length col_end - col_begin in the units of the standardised y: beta, se,
+        chi2, p, af, n_obs.  timing: as for _scan_blocks."""
         if self.C.shape[1] > ASSOC_MAX_COVARIATES:
             raise ValueError("the association scan takes at most %d covariates, got %d"
                              % (ASSOC_MAX_COVARIATES, self.C.shape[1]))
@@ -390,46 +471,14 @@ class RemlSession(object):
         out["n_obs"] = np.zeros(m_loc, dtype=np.int64)
         if m_loc == 0:
             return out
-        self.factor_at(sigmas)
-        ViC, chol, beta, Viy = self.fixed_effects()
-        Vir = Viy - ViC @ torch.from_numpy(beta).to("cuda")
-        P = torch.cat([ViC, Vir.unsqueeze(1)], dim=1).contiguous()       # n x (c + 1)
-        c1 = P.shape[1]
         block = max(1, min(int(block), m_loc))
-        starts = list(range(col_begin, col_end, block))
-        # one int8 buffer: the upload of block i + 1 is issued after assoc_genotypes has returned for block i, and that
-        # call waits for its kernels (device-side input check), so nothing still reads the buffer
-        g8 = torch.empty(n * block, dtype=torch.int8, device="cuda")
-        X = torch.empty(n * block, dtype=torch.float64, device="cuda")
-        small = [dict(proj=torch.empty(c1 * block, dtype=torch.float64, device="cuda"),
-                      nobs=torch.empty(block, dtype=torch.int64, device="cuda"),
-                      gsum=torch.empty(block, dtype=torch.int64, device="cuda"),
-                      ss=torch.empty(block, dtype=torch.float64, device="cuda")) for _ in range(2)]
-        if getattr(self, "_copy_stream", None) is None:
-            self._copy_stream = torch.cuda.Stream()
-        copy, main = self._copy_stream, torch.cuda.current_stream()
-        uploaded = torch.cuda.Event()
-        strides = [None]
+        spans = [(j0, min(j0 + block, col_end)) for j0 in range(col_begin, col_end, block)]
 
-        def upload(i):
-            j0 = starts[i]
-            strides[0] = _eng.upload_genotype_block(G, j0, min(j0 + block, col_end), g8, copy)
-            uploaded.record(copy)
-
-        def finish(i):
-            """Statistics of block i, whose kernels have completed.  The small outputs come back on the copy stream, so
-            the host does not wait behind the sweep of block i + 1 queued on the compute stream."""
-            j0 = starts[i]
-            w = min(j0 + block, col_end) - j0
-            s = small[i % 2]
-            with torch.cuda.stream(copy):
-                proj = s["proj"][:c1 * w].view(c1, w).cpu().numpy()
-                ss = s["ss"][:w].cpu().numpy()
-                nobs, gsum = s["nobs"][:w].cpu().numpy(), s["gsum"][:w].cpu().numpy()
-            q, t = proj[:c1 - 1], proj[c1 - 1]
+        def finish(i, chol, q, t, nobs, gsum, ss):
+            j0, j1 = spans[i]
             xPx = ss - np.sum(q * la.cho_solve(chol, q), axis=0)
             ok = xPx > 1e-10 * ss                      # monomorphic (ss = 0) or in the span of C: NaN
-            sl = slice(j0 - col_begin, j0 - col_begin + w)
+            sl = slice(j0 - col_begin, j1 - col_begin)
             with np.errstate(invalid="ignore", divide="ignore"):
                 xPx = np.where(ok, xPx, np.nan)
                 out["beta"][sl] = t / xPx
@@ -439,39 +488,70 @@ class RemlSession(object):
                 out["af"][sl] = gsum / nobs / 2.0
             out["n_obs"][sl] = nobs
 
-        def mark(marks):
-            if marks is not None:
-                marks.append(torch.cuda.Event(enable_timing=True))
-                marks[-1].record(main)
+        self._scan_blocks(sigmas, G, spans, lambda i: spans[i][1] - spans[i][0],
+                          lambda i, F, buf: _eng.assoc_colsumsq(F, buf), finish, timing)
+        return out
 
-        upload(0)
-        try:
-            for i, j0 in enumerate(starts):
-                w = min(j0 + block, col_end) - j0
-                s = small[i % 2]
-                Xb = X[:n * w].view(n, w)
-                marks = None if timing is None else []
-                mark(marks)
-                main.wait_event(uploaded)
-                mark(marks)
-                # returns once the kernels are done (device-side input check): block i - 1 is swept and reduced by then
-                _eng.assoc_genotypes(g8, n, w, strides[0], P, Xb, s["proj"], s["nobs"], s["gsum"])
-                mark(marks)
-                self.eng.solve_(Xb, mode=1)
-                mark(marks)
-                _eng.assoc_colsumsq(Xb, s["ss"])
-                mark(marks)
-                if timing is not None:
-                    timing.append(marks)
-                # while the device sweeps block i: statistics of block i - 1, then the host stages block i + 1
-                if i > 0:
-                    finish(i - 1)
-                if i + 1 < len(starts):
-                    upload(i + 1)
-            main.synchronize()
-            finish(len(starts) - 1)
-        finally:
-            torch.cuda.synchronize()                   # no copy may still target the buffers when they are freed
+    def region_test(self, sigmas, G, bounds, weights, block, reg_begin=0, reg_end=None, timing=None):
+        """Burden and SKAT tests of the regions [reg_begin, reg_end) of the host (n, m) int8 genotype matrix G (region r
+        is the columns [bounds[r], bounds[r+1])) at the variance components `sigmas`; see region_test() for the
+        statistics.  Consecutive whole regions are packed greedily into spans of `block` columns (no region straddles
+        two), and each span goes through _scan_blocks with the region Gram (slmm_assoc_region_gram) as the
+        reduction.  weights: length-m per-variant weights, or None for the default beta(maf; 1, 25).  Returns a dict of
+        arrays of length reg_end - reg_begin in the units of the standardised y.  timing: as for _scan_blocks."""
+        if self.C.shape[1] > ASSOC_MAX_COVARIATES:
+            raise ValueError("the association scan takes at most %d covariates, got %d"
+                             % (ASSOC_MAX_COVARIATES, self.C.shape[1]))
+        bounds = np.asarray(bounds, dtype=np.int64)
+        reg_end = len(bounds) - 1 if reg_end is None else int(reg_end)
+        R = max(reg_end - reg_begin, 0)
+        out = {k: np.full(R, np.nan) for k in REGION_FLOAT_KEYS}
+        out["n_variants"] = (bounds[reg_begin + 1:reg_end + 1] - bounds[reg_begin:reg_end]).astype(np.int64)
+        out["n_poly"] = np.zeros(R, dtype=np.int64)
+        if R == 0:
+            return out
+        if int(out["n_variants"].max()) > block:
+            raise ValueError("a region of %d variants does not fit a block of %d" % (out["n_variants"].max(), block))
+        groups = []                                    # per span: its region indices [r0, r1)
+        r0 = reg_begin
+        for r in range(reg_begin, reg_end):
+            if bounds[r + 1] - bounds[r0] > block:
+                groups.append((r0, r))
+                r0 = r
+        groups.append((r0, reg_end))
+        # every span is `block` columns wide (short only at the end of G): the sweep keeps one solve plan instead of
+        # building one per width.  The columns after a span's last region are swept too and go to the Gram as regions
+        # of at most 64 columns, cut at the 64-column strips, whose squares are ignored.
+        m = G.shape[1]
+        spans, rel = [], []
+        for a, b in groups:
+            j0 = int(bounds[a])
+            width = min(block, m - j0)
+            used = int(bounds[b]) - j0
+            pad = list(range((used // 64 + 1) * 64, width, 64)) + [width] if used < width else []
+            spans.append((j0, j0 + width))
+            rel.append(np.concatenate([bounds[a:b + 1] - j0, pad]).astype(np.int32))
+
+        def finish(i, chol, q, t, nobs, gsum, red):
+            j0, j1 = spans[i]
+            if weights is None:
+                with np.errstate(invalid="ignore", divide="ignore"):
+                    wts = skat_weights(gsum / nobs / 2.0)
+            else:
+                wts = weights[j0:j1]
+            off = 0
+            for k in range(groups[i][1] - groups[i][0]):
+                a, b = int(rel[i][k]), int(rel[i][k + 1])
+                FtF = red[off:off + (b - a) ** 2].reshape(b - a, b - a)
+                off += (b - a) ** 2
+                qr = q[:, a:b]
+                Phi = FtF - qr.T @ la.cho_solve(chol, qr)
+                r = groups[i][0] + k - reg_begin
+                for key, v in region_statistics(t[a:b], Phi, FtF, wts[a:b]).items():
+                    out[key][r] = v
+
+        self._scan_blocks(sigmas, G, spans, lambda i: int(np.sum(np.diff(rel[i]).astype(np.int64) ** 2)),
+                          lambda i, F, buf: _eng.assoc_region_gram(F, rel[i], buf), finish, timing)
         return out
 
     def blup(self, sigmas, matset, groups, colmap=None, probes=0, block_begin=0, block_end=None):
@@ -980,6 +1060,158 @@ def association(cholesky_func, mats, covariates, y, sigmas, G):
     part["beta"] = part["beta"] * scale
     part["se"] = part["se"] * scale
     return {k: part[k] for k in keys}
+
+
+# ------------------------------------------------------------------------------------------- region tests
+REGION_MAX = 512            # widest region: the region Gram gathers its square from at most 8 x 8 64-column tiles
+REGION_FLOAT_KEYS = ("burden_beta", "burden_se", "burden_chi2", "burden_p", "skat_q", "skat_p")
+REGION_KEYS = ("n_variants", "n_poly") + REGION_FLOAT_KEYS
+
+
+def skat_weights(af):
+    """Default SKAT weights beta.pdf(maf; 1, 25), maf = min(af, 1 - af); 0 where af is undefined (no genotype)."""
+    af = np.asarray(af, dtype=np.float64)
+    maf = np.minimum(af, 1.0 - af)
+    return np.where(np.isnan(af), 0.0, stats.beta.pdf(np.nan_to_num(maf), 1, 25))
+
+
+def chi2_mixture_sf(q, lam):
+    """P(sum_i lam_i chi2_1 > q) for positive weights lam (independent chi2_1 terms).
+
+    All weights equal (within 1e-9 relative): the exact chi2_r survival function.  Otherwise the Lugannani-Rice
+    saddlepoint approximation (Kuonen 1999), with its limit 1/2 - K3(0) / (6 sqrt(2 pi) K2(0)^3/2) (K2, K3: second and
+    third derivatives of the cumulant generating function) where the signed root w is within 1e-3 of 0 (q near
+    sum lam, where the formula is 0/0).  Against the closed form for lam = (a, a, b, b), a/b from 1.5 to 1000, the
+    relative error stays within 0.63 % for p > 0.5, 4.0 % for 1e-6 < p <= 0.5 and 7.3 % down to 1e-300.  One dominant
+    weight with tiny others nears the single chi2_1 case, where the saddlepoint is about 15 % off in the far tail
+    (DESIGN.md 6e).  q <= 0 gives 1."""
+    lam = np.asarray(lam, dtype=np.float64).ravel()
+    r = lam.size
+    if q <= 0:
+        return 1.0
+    lmax = lam.max()
+    if lmax - lam.min() <= 1e-9 * lmax:
+        return float(stats.chi2.sf(q / lam.mean(), r))
+    lam, q = lam / lmax, q / lmax                  # scale-free: the root lies in (lo, 1/2)
+
+    def K1(z):
+        return np.sum(lam / (1.0 - 2.0 * z * lam))
+
+    lo = -r / (2.0 * q) - 1.0                      # K'(lo) < q
+    hi = 0.5 * (1.0 - 1.0 / (q + lam.sum()))       # K'(hi) > 1 / (1 - 2 hi) = q + sum lam > q
+    z = optimize.brentq(lambda z: K1(z) - q, lo, hi, xtol=1e-15, rtol=4 * np.finfo(float).eps, maxiter=500)
+    d = 1.0 - 2.0 * z * lam
+    K = -0.5 * np.sum(np.log(d))
+    w = np.sign(z) * np.sqrt(max(2.0 * (z * q - K), 0.0))
+    if abs(w) < 1e-3:
+        k2, k3 = 2.0 * np.sum(lam ** 2), 8.0 * np.sum(lam ** 3)
+        return float(0.5 - k3 / (6.0 * np.sqrt(2.0 * np.pi) * k2 ** 1.5))
+    v = z * np.sqrt(2.0 * np.sum(lam ** 2 / d ** 2))
+    p = stats.norm.sf(w) + stats.norm.pdf(w) * (1.0 / v - 1.0 / w)
+    return float(min(max(p, 0.0), 1.0))
+
+
+def region_statistics(t, Phi, FtF, w):
+    """Burden and SKAT statistics of one region from t = (V^-1 r)' X~ (length w_r), Phi = X~' P_V X~ and
+    FtF = X~' V^-1 X~ (w_r x w_r) and the weights w, in the units of the standardised y (see region_test()).  Returns a
+    dict with n_poly and the finite entries of REGION_FLOAT_KEYS; the others are NaN."""
+    out = {"n_poly": int(np.sum(np.diag(FtF) > 0))}
+    s, v, vF = w @ t, w @ Phi @ w, w @ FtF @ w
+    if v > 1e-10 * vF:                             # not monomorphic, not in the span of C
+        chi2 = s * s / v
+        out.update(burden_beta=s / v, burden_se=1.0 / np.sqrt(v), burden_chi2=chi2, burden_p=special.chdtrc(1, chi2))
+    lam = np.linalg.eigvalsh(w[:, None] * Phi * w[None, :])
+    if lam[-1] > 1e-10 * np.sum(w * w * np.diag(FtF)):     # trace(W F'F W) >= its largest eigenvalue
+        lam = lam[lam > 1e-10 * lam[-1]]
+        Q = float(np.sum((w * t) ** 2))
+        out.update(skat_q=Q, skat_p=chi2_mixture_sf(Q, lam))
+    return out
+
+
+def check_regions(bounds, weights, m):
+    """(bounds as int64, weights as float64 or None) after the input rules of region_test(); ValueError otherwise."""
+    bounds = np.asarray(bounds)
+    if bounds.ndim != 1 or bounds.size < 2 or not np.issubdtype(bounds.dtype, np.integer):
+        raise ValueError("bounds must be a 1-D int array of at least 2 region offsets")
+    bounds = bounds.astype(np.int64)
+    if bounds[0] != 0 or bounds[-1] != m:
+        raise ValueError("bounds must start at 0 and end at m = %d, got %d and %d" % (m, bounds[0], bounds[-1]))
+    widths = np.diff(bounds)
+    if np.any(widths <= 0):
+        raise ValueError("bounds must strictly increase")
+    if widths.max() > REGION_MAX:
+        raise ValueError("a region has %d variants; at most %d are supported" % (widths.max(), REGION_MAX))
+    if weights is not None:
+        weights = np.asarray(weights, dtype=np.float64)
+        if weights.shape != (m,):
+            raise ValueError("weights must have one entry per variant (%d), got shape %s" % (m, weights.shape))
+        if not np.all(np.isfinite(weights)) or np.any(weights < 0):
+            raise ValueError("weights must be finite and >= 0")
+    return bounds, weights
+
+
+def region_test(cholesky_func, mats, covariates, y, sigmas, G, bounds, weights=None):
+    """Region-based rare-variant tests (burden and SKAT against the kinship-aware null, as famSKAT) of the variants in G
+    at the variance components `sigmas`.
+
+    cholesky_func, mats, covariates, y, sigmas and G as for association() (int8 allele counts, C or Fortran order, at
+    most 31 covariates, a call after REML() reuses its device session).  bounds: int array like an indptr; region r is
+    the columns [bounds[r], bounds[r+1]) of G, with bounds[0] = 0, bounds[-1] = m, strictly increasing, 1 to
+    REGION_MAX = 512 variants per region.  weights: one finite weight >= 0 per variant; by default beta.pdf(maf; 1, 25)
+    with maf = min(af, 1 - af) from the allele frequency of the non-missing entries (0 for a variant without any).
+
+    Per region, in the units of y_s = y / y.std(): t = (V^-1 r)' X~, Phi = X~' P_V X~ = F'F - q' M^-1 q (F = L^-1 P X~,
+    q = (V^-1 C)' X~, M = C'V^-1 C) and W = diag(w).
+      burden: s = w't, v = w'Phi w, beta = s / v, se = v^-1/2, chi2 = s^2 / v and p its chi^2_1 survival function: the
+        coefficient of the burden score X~ w and its standard error in the GLS fit of [C | X~ w] under the same V.
+        beta and se are in the units of y per unit of the burden score.  NaN when v <= 1e-10 w'F'F w (no polymorphic
+        variant, or the burden score in the span of C).
+      SKAT: Q = sum_j w_j^2 t_j^2.  Under the null t ~ N(0, Phi), so Q ~ sum_i lam_i chi2_1 with lam = eig(W Phi W);
+        eigenvalues <= 1e-10 lam_max are dropped and p = chi2_mixture_sf(Q, lam).  Q is left in the standardised units
+        (the p-value is scale-free).  NaN when lam_max <= 1e-10 trace(W F'F W): the region carries no variation
+        beyond C (for one variant this is association()'s rule).
+
+    Returns a dict of length-R arrays: n_variants, n_poly (variants with F_j'F_j > 0), burden_beta, burden_se,
+    burden_chi2, burden_p, skat_q, skat_p.  With torch.distributed initialised every rank tests a contiguous slice of
+    the regions and one all-reduce gives every rank the whole result."""
+    functor = _need_functor(cholesky_func)
+    G = np.asarray(G)
+    if G.ndim != 2 or G.dtype != np.int8:
+        raise ValueError("G must be a 2-D int8 array of allele counts (negative = missing)")
+    if G.shape[0] != y.shape[0]:
+        raise ValueError("G has %d rows for %d individuals" % (G.shape[0], y.shape[0]))
+    if not (G.flags.c_contiguous or G.flags.f_contiguous):
+        G = np.ascontiguousarray(G)
+    if np.shape(covariates)[1] > ASSOC_MAX_COVARIATES:
+        raise ValueError("the association scan takes at most %d covariates, got %d"
+                         % (ASSOC_MAX_COVARIATES, np.shape(covariates)[1]))
+    sigmas = np.asarray(sigmas, dtype=float)
+    if sigmas.shape != (len(mats) + 1,):
+        raise ValueError("need %d variance components (the residual last), got %d" % (len(mats) + 1, sigmas.size))
+    n, m = G.shape
+    bounds, weights = check_regions(bounds, weights, m)
+    torch = _eng.require_cuda()
+    free = torch.cuda.mem_get_info()[0]
+    block = int(max(8, min(ASSOC_BLOCK, free // 2 // (ASSOC_BYTES_PER_ENTRY * n))))
+    if np.diff(bounds).max() > block:
+        raise ValueError("the widest region (%d variants) does not fit the %d columns that device memory allows"
+                         % (np.diff(bounds).max(), block))
+    scale = y.std()
+    ses = _scan_session(functor, mats, covariates, y / scale)
+    R = bounds.size - 1
+    rank, world = _shard.rank_world()
+    lo, hi = _shard.column_block(R, rank, world)
+    part = ses.region_test(sigmas, G, bounds, weights, block, lo, hi)
+    if world > 1:
+        full = torch.zeros(len(REGION_KEYS), R, dtype=torch.float64, device="cuda")
+        full[:, lo:hi] = torch.from_numpy(np.stack([part[k].astype(np.float64) for k in REGION_KEYS]))
+        full = _shard.allreduce_sum_(full).cpu().numpy()
+        part = {k: full[i] for i, k in enumerate(REGION_KEYS)}
+        for k in ("n_variants", "n_poly"):
+            part[k] = part[k].astype(np.int64)
+    part["burden_beta"] = part["burden_beta"] * scale
+    part["burden_se"] = part["burden_se"] * scale
+    return {k: part[k] for k in REGION_KEYS}
 
 
 # ------------------------------------------------------------------------------------------- predicted random effects

@@ -6,7 +6,7 @@ Mirrors the reference package facade (scilmm/__init__.py:1-2 star-imports Sparse
 from .SparseCholesky import (HE, MINQUE, REML, B200Factor, association, NotPositiveDefiniteError, SlmmError,  # noqa: F401
                              SparseCholesky, blup, bolt_gradient_estimation, compute_gradients, compute_hess,
                              compute_varcomp_stderr, estimate_fixed_effects, estimate_var_comps,
-                             matrices_weighted_sum, negative_log_likelihood, run_estimates,
+                             matrices_weighted_sum, negative_log_likelihood, region_test, run_estimates,
                              run_estimates_from_paths, simulate_vector)
 
 from .legacy import LMM, compute_HE  # noqa: F401,E402  (reference scilmm/Estimation/LMM.py:154, HE.py:22)

@@ -122,6 +122,15 @@ def assoc_colsumsq(F, out):
     return out
 
 
+def assoc_region_gram(F, bounds, out):
+    """Region Gram of a contiguous n x width CUDA float64 block (slmm_assoc_region_gram): out (CUDA float64) receives
+    F_r' F_r for the column regions [bounds[r], bounds[r+1]) of F, row-major and packed one region after another."""
+    b = np.ascontiguousarray(bounds, dtype=np.int32)
+    check(lib().slmm_assoc_region_gram(F.data_ptr(), int(F.shape[0]), int(F.shape[1]), int(b.size - 1),
+                                       b.ctypes.data, out.data_ptr()))
+    return out
+
+
 # ------------------------------------------------------------------------------------------------ symbolic
 class SymbolicView(object):
     """Host-only symbolic analysis (no GPU needed)."""
