@@ -288,6 +288,31 @@ int slmm_assoc_colsumsq(const double* d_F, int64_t n, int32_t b, double* d_out);
 int slmm_assoc_region_gram(const double* d_F, int64_t n, int32_t b, int32_t nregions, const int32_t* h_bounds,
                            double* d_out);
 
+/* ------------------------------------------------------------------ binary traits (logistic mixed model) */
+/* PQL fit and saddlepoint-calibrated score test of a 0/1 trait (GMMAT glmmkin, SAIGE).  The reference has no
+ * counterpart.
+ *   slmm_glmm_working: the elementwise step between two PQL iterations, for n individuals, all device vectors of n
+ *     doubles.  In: d_ytilde = the working vector Y~ of the last iteration, d_vir = Sigma^-1 (Y~ - C alpha), d_dvals =
+ *     the values D = 1 / w of the diagonal component, d_y = the 0/1 trait.  Computes eta = Y~ - D o d_vir, mu =
+ *     1 / (1 + e^-eta) clamped to [2.22e-16, 1 - 2.22e-16], w = mu (1 - mu), and writes in place d_ytilde = eta +
+ *     (y - mu) / w and d_dvals = 1 / w, and d_eta = eta, d_mu = mu.  A y entry other than 0 or 1 returns
+ *     SLMM_ERR_INVALID (checked on the device; the outputs are then undefined).  Returns when the kernel is done.
+ *   slmm_assoc_spa: two-sided saddlepoint p-values of b variants.  d_X: the C-ordered n x b block x~ of
+ *     slmm_assoc_genotypes called with P = W C (n x c, c <= 31), d_proj its c x b output (W C)' x~; d_Minv: c x c
+ *     (C'WC)^-1, row-major; d_C: C-ordered n x c covariates; d_mu, d_w: the fitted means and weights (n); d_score,
+ *     d_var: U and Var(U) of the mixed-model score test (b each).  Per variant: g~ = x~ - C Minv proj, Var* = g~'W g~,
+ *     q = U sqrt(Var* / Var(U)); with K the cumulant generating function of sum_i g~_i (Y_i - mu_i) under independent
+ *     Bernoulli(mu_i), the roots of K'(zeta) = +-|q| (bracket-safeguarded Newton) and the sum of the two
+ *     Lugannani-Rice tails.  d_work: n x b doubles of scratch (g~, variant-major).  Out (b each): d_p, d_status (1 =
+ *     saddlepoint p; -1 = no root in range or bracketed, or |w| < 1e-3: d_p is NaN), d_iters (passes over the n
+ *     individuals, both sides).  One CTA per variant, sums in a fixed order without atomics: a variant's outputs do
+ *     not depend on b or on its position in the block.  Asynchronous on the default stream. */
+int slmm_glmm_working(double* d_ytilde, const double* d_vir, double* d_dvals, const double* d_y, int64_t n,
+                      double* d_eta, double* d_mu);
+int slmm_assoc_spa(const double* d_X, int64_t n, int32_t b, const double* d_proj, int32_t c, const double* d_Minv,
+                   const double* d_C, const double* d_mu, const double* d_w, const double* d_score,
+                   const double* d_var, double* d_work, double* d_p, int32_t* d_status, int32_t* d_iters);
+
 /* ------------------------------------------------------------------ predicted random effects (BLUP) ---- */
 /* Column-mapped products of the relationship matrices over ALL N individuals of the set with blocks over the n
  * observed ones (the individuals the fit used).  The reference has no counterpart.  Both calls take one pattern group:

@@ -116,6 +116,7 @@ class SparseCholesky(object):
         self.probe_source = None      # callable(n, sim_num) -> host block, used when rng == 'host_buffer'
         self._engines = {}
         self._sessions = {}
+        self._glmm = None             # the PQL session of glmm(): its device y and W^-1 change, so it is kept apart
         self.timings = {}
 
     def _engine_for(self, pattern, key=None):
@@ -171,6 +172,7 @@ class SparseCholesky(object):
         """Forget the cached REML sessions (device copies of mats / covariates / y).  The cache notices in-place
         edits through a sampled content fingerprint; call this after an edit it could miss."""
         self._sessions.clear()
+        self._glmm = None
 
     # ---- fused session for the REML objective: matrices resident, patterns registered once
     def _session(self, mats, covariates, y):
@@ -461,13 +463,13 @@ class RemlSession(object):
         matrix G at the variance components `sigmas` (see association() for the statistic), in blocks of `block`
         variants through _scan_blocks, with a column sum of squares as the reduction and the c x c finalisation on the
         host.  Returns a dict of arrays of length col_end - col_begin in the units of the standardised y: beta, se,
-        chi2, p, af, n_obs.  timing: as for _scan_blocks."""
+        chi2, p, af, n_obs, and the score t with its variance xPx (score, var).  timing: as for _scan_blocks."""
         if self.C.shape[1] > ASSOC_MAX_COVARIATES:
             raise ValueError("the association scan takes at most %d covariates, got %d"
                              % (ASSOC_MAX_COVARIATES, self.C.shape[1]))
         col_end = G.shape[1] if col_end is None else int(col_end)
         m_loc = max(col_end - col_begin, 0)
-        out = {k: np.full(m_loc, np.nan) for k in ("beta", "se", "chi2", "p", "af")}
+        out = {k: np.full(m_loc, np.nan) for k in ("beta", "se", "chi2", "p", "af", "score", "var")}
         out["n_obs"] = np.zeros(m_loc, dtype=np.int64)
         if m_loc == 0:
             return out
@@ -486,6 +488,8 @@ class RemlSession(object):
                 out["chi2"][sl] = t * t / xPx
                 out["p"][sl] = special.chdtrc(1, out["chi2"][sl])
                 out["af"][sl] = gsum / nobs / 2.0
+                out["score"][sl] = np.where(ok, t, np.nan)
+                out["var"][sl] = xPx
             out["n_obs"][sl] = nobs
 
         self._scan_blocks(sigmas, G, spans, lambda i: spans[i][1] - spans[i][0],
@@ -600,6 +604,51 @@ class RemlSession(object):
             del Z, W
         out["parts"] = parts
         return out
+
+    def spa(self, G, cols, score, var, mu, w, block, timing=None):
+        """Saddlepoint p-values (slmm_assoc_spa) of the columns `cols` of the host (n, m) int8 genotype matrix G, given
+        their scores U (`score`) and Var(U) (`var`) and the fitted means `mu` and weights `w` (host, length n).  The
+        columns are gathered on the host in order and go up `block` at a time; slmm_assoc_genotypes with P = W C decodes
+        and centres them and gives (W C)' x~.  Returns (p, status, iters) of length len(cols); see glmm_association().
+        timing: a list that receives two timing events per block around the saddlepoint kernel."""
+        torch = self.torch
+        n, c, m = self.n, self.C.shape[1], len(cols)
+        p, status, iters = np.full(m, np.nan), np.zeros(m, dtype=np.int8), np.zeros(m, dtype=np.int32)
+        if m == 0:
+            return p, status, iters
+        CtWC = self.C_host.T @ (w[:, None] * self.C_host)
+        Minv = _eng.to_device(la.cho_solve(la.cho_factor(CtWC), np.eye(c)), torch)
+        mu_d, w_d = _eng.to_device(mu, torch), _eng.to_device(w, torch)
+        WC = (w_d[:, None] * self.C).contiguous()
+        block = max(1, min(int(block), m))
+        f64 = dict(dtype=torch.float64, device="cuda")
+        g8 = torch.empty(n * block, dtype=torch.int8, device="cuda")
+        X = torch.empty(n * block, **f64)
+        work = torch.empty(n * block, **f64)
+        proj, sc, vr, pd = (torch.empty(k, **f64) for k in (c * block, block, block, block))
+        nobs, gsum = (torch.empty(block, dtype=torch.int64, device="cuda") for _ in range(2))
+        st, it = (torch.empty(block, dtype=torch.int32, device="cuda") for _ in range(2))
+        for j0 in range(0, m, block):
+            j1 = min(j0 + block, m)
+            wd = j1 - j0
+            Gb = G[:, cols[j0:j1]]
+            if not (Gb.flags.c_contiguous or Gb.flags.f_contiguous):
+                Gb = np.ascontiguousarray(Gb)
+            strides = _eng.upload_genotype_block(Gb, 0, wd, g8)
+            Xb = X[:n * wd].view(n, wd)
+            _eng.assoc_genotypes(g8, n, wd, strides, WC, Xb, proj, nobs, gsum)
+            sc[:wd].copy_(torch.from_numpy(np.ascontiguousarray(score[j0:j1], dtype=np.float64)))
+            vr[:wd].copy_(torch.from_numpy(np.ascontiguousarray(var[j0:j1], dtype=np.float64)))
+            if timing is not None:
+                timing.append([torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)])
+                timing[-1][0].record()
+            _eng.assoc_spa(Xb, proj, Minv, self.C, mu_d, w_d, sc, vr, work, pd, st, it)
+            if timing is not None:
+                timing[-1][1].record()
+            p[j0:j1] = pd[:wd].cpu().numpy()
+            status[j0:j1] = st[:wd].cpu().numpy()
+            iters[j0:j1] = it[:wd].cpu().numpy()
+        return p, status, iters
 
     def _is_identity(self, k):
         m = self.mats_host[k]
@@ -1331,6 +1380,243 @@ def blup(cholesky_func, mats, covariates, y, sigmas, pev_probes=0):
     out["pev"] = scale * scale * pev
     out["pev_se"] = scale * scale * se
     return out
+
+
+# ------------------------------------------------------------------------------------------- binary traits
+GLMM_TOL = 1e-5             # GMMAT's stopping rule on the relative changes of alpha and tau
+GLMM_MAX_ITER = 50
+GLMM_MU_EPS = 2.220446049250313e-16   # mu is clamped to [eps, 1 - eps], as R's binomial() (csrc/glmm.cu)
+IRLS_TOL = 1e-10            # GLM start: stop when max |delta alpha| < IRLS_TOL (1 + max |alpha|)
+IRLS_MAX_ITER = 100
+# device bytes a saddlepoint block holds per (individual, variant): x~ and g~ in float64 and the int8 block
+SPA_BYTES_PER_ENTRY = 20
+GLMM_ASSOC_KEYS = ("beta", "se", "score", "chi2", "p", "p_normal", "spa", "af", "n_obs")
+
+
+def _logit_working(eta, y):
+    """(mu, w, Y~) of the logit link at eta, the formulas of slmm_glmm_working."""
+    mu = np.clip(special.expit(eta), GLMM_MU_EPS, 1.0 - GLMM_MU_EPS)
+    w = mu * (1.0 - mu)
+    return mu, w, eta + (y - mu) / w
+
+
+def _irls(C, y):
+    """Logistic GLM (no random effects) by iteratively reweighted least squares from mu = (y + 1/2) / 2.  Returns alpha."""
+    mu = (y + 0.5) / 2.0
+    eta = np.log(mu / (1.0 - mu))
+    alpha = np.zeros(C.shape[1])
+    for _ in range(IRLS_MAX_ITER):
+        _, w, z = _logit_working(eta, y)
+        new = la.solve(C.T @ (w[:, None] * C), C.T @ (w * z), assume_a="pos")
+        step = np.max(np.abs(new - alpha))
+        alpha = new
+        eta = C @ alpha
+        if step < IRLS_TOL * (1.0 + np.max(np.abs(alpha))):
+            break
+    return alpha
+
+
+def _check_binary(mats, covariates, y):
+    """(C, y) as float64 after the input rules of glmm(); ValueError otherwise."""
+    y = np.asarray(y, dtype=np.float64)
+    if y.ndim != 1:
+        raise ValueError("y must be a vector")
+    n = y.shape[0]
+    if len(mats) == 0 or any(m.shape != (n, n) for m in mats):
+        raise ValueError("every matrix must be n x n with n = len(y) = %d" % n)
+    C = np.asarray(covariates, dtype=np.float64)
+    if C.ndim != 2 or C.shape[0] != n:
+        raise ValueError("covariates must be n x c with n = %d" % n)
+    if not np.all(np.isfinite(C)):
+        raise ValueError("covariates must be finite")
+    if np.any(np.isnan(y)):
+        raise ValueError("y must not contain NaN")
+    if not np.all((y == 0.0) | (y == 1.0)):
+        raise ValueError("y must be 0 (control) or 1 (case)")
+    if y.min() == y.max():
+        raise ValueError("y needs both cases and controls")
+    return C, y
+
+
+def _glmm_session(functor, mats, covariates, Yt, w):
+    """The functor's PQL session over mats + [W^-1] (W^-1 a diagonal CSR) with its device phenotype set to the working
+    vector Yt and its diagonal values to 1 / w.  The session of an earlier call on the same mats and covariates (content
+    fingerprint) is reused: only the two device vectors are rewritten, and not even those when they
+    already hold Yt and 1 / w.  The session is never in the content-keyed cache (SparseCholesky._session): its host
+    copies of y and W^-1 stop describing its device state after the first iteration."""
+    torch = _eng.require_cuda()
+    key = (tuple((m.shape, int(m.nnz), _fingerprint(m.data)) for m in mats),
+           _fingerprint(covariates, with_sum=True))
+    ses = functor._glmm
+    D = 1.0 / w
+    if ses is None or ses.glmm_key != key:
+        functor._glmm = None                       # the old session's device memory goes before the new one is set up
+        n = Yt.shape[0]
+        Dm = sparse.csr_matrix((D, np.arange(n, dtype=np.int32), np.arange(n + 1, dtype=np.int32)), shape=(n, n))
+        ses = RemlSession(functor, list(mats) + [Dm], covariates, Yt)
+        ses.glmm_key = key
+        functor._glmm = ses
+    elif not (np.array_equal(ses.glmm_state[0], Yt) and np.array_equal(ses.glmm_state[1], w)):
+        ses.y.copy_(torch.from_numpy(np.ascontiguousarray(Yt)))
+        ses.matset.device_arrays(ses.K - 1)[2].copy_(torch.from_numpy(D))
+    ses.glmm_state = (np.array(Yt, dtype=np.float64), np.array(w, dtype=np.float64))
+    return ses
+
+
+def glmm(cholesky_func, mats, covariates, y, sim_num=100, verbose=False):
+    """Logistic mixed model of a 0/1 trait, fitted by penalised quasi-likelihood (PQL; Breslow & Clayton 1993) with
+    GMMAT's average-information scheme (glmmkin, Chen et al. 2016): logit P(y_i = 1) = (C alpha)_i + b_i with random
+    effects b ~ N(0, sum_k tau_k A_k) and the dispersion fixed at 1.
+
+    mats: the K relationship matrices (n x n) without an identity; covariates: n x c, finite, with the intercept
+    column; y: length n, 0 (control) or 1 (case), both present.  Anything else raises ValueError before any device work.
+
+    Start: a logistic GLM by IRLS on the host gives alpha and eta = C alpha; tau_k = var(Y~) / (K + 1).  Per iteration:
+    mu = logistic(eta) clamped to [eps, 1 - eps] (eps = 2.22e-16), w = mu (1 - mu), the working vector
+    Y~ = eta + (y - mu) / w and Sigma = W^-1 + sum_k tau_k A_k; one REML evaluation with the average-information matrix
+    on (Sigma, Y~) (RemlSession.evaluate), then an EM step tau_k <- max(floor, tau_k - 2 tau_k^2 grad_k / n) in the
+    first iteration and the AI-REML step of REML(aireml=True) restricted to the K components after; alpha = the GLS
+    coefficients of the evaluation and eta = Y~ - W^-1 Sigma^-1 (Y~ - C alpha) (the BLUP identity: no product with the
+    A_k).  Stops when 2 max(|d alpha| / (|alpha| + |alpha_old| + tol), |d tau| / (|tau| + |tau_old| + tol)) < tol,
+    tol = 1e-5, or after GLMM_MAX_ITER iterations (reported as REML() reports non-convergence).  Every iteration uses
+    the same probe block (one numpy draw, one probe_source call or one device stream index), as REML(aireml=True) does,
+    and under torch.distributed the probe columns are sharded the same way.  The working vector, W^-1 and eta stay on
+    the device between iterations: slmm_glmm_working updates them in place.
+
+    Returns a dict: 'covariance coefficients' (tau, logit scale) and 'covariance std' (sqrt(diag(AI^-1) (1 + 1/sim_num))
+    from the last iteration's AI matrix); 'covariates coefficients' (alpha) and 'covariates std' (from (C'Sigma^-1 C)^-1
+    of the last iteration); 'latent fractions' tau_k / (sum tau + pi^2 / 3), the liability-scale variance shares; 'mu',
+    'eta', 'weights' (w) and 'working y' (Y~) of the returned alpha and random effects; 'glmm': {'iterations',
+    'converged'}.  The fit's device session stays on the functor for glmm_association()."""
+    functor = _need_functor(cholesky_func)
+    C, y = _check_binary(mats, covariates, y)
+    torch = _eng.require_cuda()
+    n, K = y.shape[0], len(mats)
+    alpha = _irls(C, y)
+    eta = C @ alpha
+    _, w, Yt = _logit_working(eta, y)
+    tau = np.full(K, np.var(Yt, ddof=1) / (K + 1))
+    ses = _glmm_session(functor, mats, covariates, Yt, w)
+    if not all(ses._sym):
+        raise ValueError("glmm needs symmetric relationship matrices; asymmetric: %s"
+                         % [k for k in range(K) if not ses._sym[k]])
+    Z, stream = None, None
+    if functor.rng == 'numpy':
+        Z = np.random.randn(n, sim_num)
+    elif functor.rng == 'host_buffer':
+        Z = functor.probe_source(n, sim_num)
+    else:
+        stream = ses.n_eval
+    y_d = _eng.to_device(y, torch)
+    dvals = ses.matset.device_arrays(K)[2]
+    eta_d = torch.empty(n, dtype=torch.float64, device="cuda")
+    mu_d = torch.empty(n, dtype=torch.float64, device="cuda")
+    converged, it = False, 0
+    while it < GLMM_MAX_ITER:
+        it += 1
+        if verbose:
+            t0 = time.time()
+        nll, grad, AI = ses.evaluate(np.concatenate([tau, [1.0]]), True, sim_num, Z=Z, ai=True, probe_stream=stream)
+        grad, AI = grad[:K], AI[:K, :K]
+        tau_old, alpha_old = tau, alpha
+        if it == 1:
+            tau = np.maximum(AIREML_FLOOR, tau - 2.0 * tau * tau * grad / n)
+        else:
+            tau = _aireml_step(tau, grad, AI)[0]
+        alpha = ses.last["beta"]
+        _eng.glmm_working(ses.y, ses.last["Vir"], dvals, y_d, eta_d, mu_d)
+        change = 2.0 * max(np.max(np.abs(alpha - alpha_old) / (np.abs(alpha) + np.abs(alpha_old) + GLMM_TOL)),
+                           np.max(np.abs(tau - tau_old) / (np.abs(tau) + np.abs(tau_old) + GLMM_TOL)))
+        if verbose:
+            print('PQL iteration %d: nll %0.8e, tau %s, alpha %s, change %.3e, %.2f seconds'
+                  % (it, nll, tau, alpha, change, time.time() - t0))
+        if change < GLMM_TOL:
+            converged = True
+            break
+    if not converged:
+        print('optimization failed with message: PQL did not converge in %d iterations' % GLMM_MAX_ITER)
+    mu = mu_d.cpu().numpy()
+    w = mu * (1.0 - mu)                            # the kernel's w, bit for bit
+    Yt = ses.y.cpu().numpy()
+    ses.glmm_state = (Yt.copy(), w.copy())
+    var_alpha = la.cho_solve(ses.last["chol"], np.eye(C.shape[1]))
+    return {"covariance coefficients": tau,
+            "covariance std": np.sqrt(np.diag(la.inv(AI)) * (1 + 1.0 / sim_num)),
+            "covariates coefficients": alpha,
+            "covariates std": np.sqrt(np.diag(var_alpha)),
+            "latent fractions": tau / (tau.sum() + np.pi ** 2 / 3),
+            "mu": mu, "eta": eta_d.cpu().numpy(), "weights": w, "working y": Yt,
+            "glmm": {"iterations": it, "converged": converged}}
+
+
+def glmm_association(cholesky_func, mats, covariates, y, fit, G, spa_cutoff=2.0):
+    """Score test of each variant (column) of G against the logistic mixed model `fit` = glmm(...) of the same
+    cholesky_func, mats, covariates and y, with saddlepoint-calibrated p-values (SAIGE, Zhou et al. 2018).
+
+    G: (n, m) int8 ndarray in C or Fortran order, 0 / 1 / 2 allele counts and negative values for missing (any other
+    value raises SlmmError), at most 31 covariates.  Phase 1 is the association scan (RemlSession.association) on the
+    fit's session (Sigma = W^-1 + sum_k tau_k A_k, Y~; reused after glmm() on the same functor, otherwise set up from
+    the fit's arrays without refitting): the score U = x~' P Y~ = x~' (y - mu) at the fixed point, Var(U) = x~' P x~,
+    z = U / sqrt(Var(U)) and its normal p.  Phase 2 takes the variants with finite |z| > spa_cutoff: per variant
+    g~ = x~ - C (C'WC)^-1 C'W x~, q = U sqrt(g~'W g~ / Var(U)) (the variance ratio of this variant, exactly), and the
+    two-sided saddlepoint p-value of q under the cumulant generating function
+    K(t) = sum_i log(1 - mu_i + mu_i e^{g~_i t}) - t sum_i g~_i mu_i: the roots of K'(zeta) = +-|q| and the
+    Lugannani-Rice tail of each side, on the device (slmm_assoc_spa).  A variant whose |q| is outside the range of K',
+    whose root is not bracketed, or whose signed root w is within 1e-3 of 0 keeps its normal p.
+
+    Returns a dict of length-m arrays: beta = U / Var(U) (the one-step logit-scale effect) and se = Var(U)^-1/2, score
+    (U), chi2 = z^2, p (the saddlepoint p where it was applied, the normal p otherwise), p_normal, spa (int8: 1 applied,
+    0 below the cutoff, -1 fell back), af, n_obs.  Monomorphic variants and those in the span of C get NaN as in
+    association().  With torch.distributed initialised every rank tests a contiguous slice of the variants in both
+    phases and one all-reduce gives every rank the whole result."""
+    functor = _need_functor(cholesky_func)
+    C, y = _check_binary(mats, covariates, y)
+    n, K = y.shape[0], len(mats)
+    G = np.asarray(G)
+    if G.ndim != 2 or G.dtype != np.int8:
+        raise ValueError("G must be a 2-D int8 array of allele counts (negative = missing)")
+    if G.shape[0] != n:
+        raise ValueError("G has %d rows for %d individuals" % (G.shape[0], n))
+    if not (G.flags.c_contiguous or G.flags.f_contiguous):
+        G = np.ascontiguousarray(G)
+    if C.shape[1] > ASSOC_MAX_COVARIATES:
+        raise ValueError("the association scan takes at most %d covariates, got %d" % (ASSOC_MAX_COVARIATES, C.shape[1]))
+    spa_cutoff = float(spa_cutoff)
+    if not spa_cutoff >= 0.0:
+        raise ValueError("spa_cutoff must be >= 0")
+    tau = np.asarray(fit["covariance coefficients"], dtype=np.float64)
+    if tau.shape != (K,) or not np.all(np.isfinite(tau)) or np.any(tau < 0):
+        raise ValueError("fit has %s covariance coefficients for %d matrices" % (tau.shape, K))
+    mu, w, Yt = (np.asarray(fit[k], dtype=np.float64) for k in ("mu", "weights", "working y"))
+    if any(a.shape != (n,) or not np.all(np.isfinite(a)) for a in (mu, w, Yt)) or not np.all(w > 0):
+        raise ValueError("fit's mu, weights and working y must be finite vectors of length n = %d (weights > 0)" % n)
+    torch = _eng.require_cuda()
+    ses = _glmm_session(functor, mats, covariates, Yt, w)
+    m = G.shape[1]
+    rank, world = _shard.rank_world()
+    lo, hi = _shard.column_block(m, rank, world)
+    block = int(max(8, min(ASSOC_BLOCK, torch.cuda.mem_get_info()[0] // 2 // (ASSOC_BYTES_PER_ENTRY * n))))
+    part = ses.association(np.concatenate([tau, [1.0]]), G, block, lo, hi)
+    U, V = part["score"], part["var"]
+    with np.errstate(invalid="ignore", divide="ignore"):
+        z = U / np.sqrt(V)
+    part["p_normal"] = part["p"].copy()
+    part["spa"] = np.zeros(hi - lo, dtype=np.int8)
+    flag = np.flatnonzero(np.isfinite(z) & (np.abs(np.nan_to_num(z)) > spa_cutoff))
+    sblock = int(max(1, min(ASSOC_BLOCK, torch.cuda.mem_get_info()[0] // 2 // (SPA_BYTES_PER_ENTRY * n))))
+    ps, status, iters = ses.spa(G, lo + flag, U[flag], V[flag], mu, w, sblock)
+    ses.last["spa_iters"] = iters
+    part["spa"][flag] = status
+    ok = status == 1
+    part["p"][flag[ok]] = ps[ok]
+    if world > 1:
+        full = torch.zeros(len(GLMM_ASSOC_KEYS), m, dtype=torch.float64, device="cuda")
+        full[:, lo:hi] = torch.from_numpy(np.stack([part[k].astype(np.float64) for k in GLMM_ASSOC_KEYS]))
+        full = _shard.allreduce_sum_(full).cpu().numpy()
+        part = {k: full[i] for i, k in enumerate(GLMM_ASSOC_KEYS)}
+        part["spa"] = part["spa"].astype(np.int8)
+        part["n_obs"] = part["n_obs"].astype(np.int64)
+    return {k: part[k] for k in GLMM_ASSOC_KEYS}
 
 
 # ------------------------------------------------------------------------------------------- Haseman-Elston

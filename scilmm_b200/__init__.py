@@ -5,7 +5,7 @@ Mirrors the reference package facade (scilmm/__init__.py:1-2 star-imports Sparse
 """
 from .SparseCholesky import (HE, MINQUE, REML, B200Factor, association, NotPositiveDefiniteError, SlmmError,  # noqa: F401
                              SparseCholesky, blup, bolt_gradient_estimation, compute_gradients, compute_hess,
-                             compute_varcomp_stderr, estimate_fixed_effects, estimate_var_comps,
+                             compute_varcomp_stderr, estimate_fixed_effects, estimate_var_comps, glmm, glmm_association,
                              matrices_weighted_sum, negative_log_likelihood, region_test, run_estimates,
                              run_estimates_from_paths, simulate_vector)
 

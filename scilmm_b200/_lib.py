@@ -51,6 +51,8 @@ SIGNATURES = {
     "slmm_assoc_genotypes": (C.c_int, [vp, i64, i32, i64, i64, vp, i32, vp, vp, vp, vp]),
     "slmm_assoc_colsumsq": (C.c_int, [vp, i64, i32, vp]),
     "slmm_assoc_region_gram": (C.c_int, [vp, i64, i32, i32, vp, vp]),
+    "slmm_glmm_working": (C.c_int, [vp, vp, vp, vp, i64, vp, vp]),
+    "slmm_assoc_spa": (C.c_int, [vp, i64, i32, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
     "slmm_blup_spmm": (C.c_int, [vp, i32, vp, vp, vp, vp, i64, i32, vp]),
     "slmm_blup_rowsumsq": (C.c_int, [vp, i32, vp, vp, vp, vp, i64, i32, vp, vp]),
     "slmm_matset_nnz": (C.c_int, [vp, i32, C.POINTER(i64)]),

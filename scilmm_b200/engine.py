@@ -131,6 +131,24 @@ def assoc_region_gram(F, bounds, out):
     return out
 
 
+def glmm_working(ytilde, vir, dvals, y, eta, mu):
+    """The elementwise step between two PQL iterations (slmm_glmm_working), in place on the CUDA float64 vectors ytilde
+    (Y~ in, the new Y~ out) and dvals (1 / w); eta and mu receive the new linear predictor and mean.  A y entry other
+    than 0 or 1 raises SlmmError."""
+    check(lib().slmm_glmm_working(ytilde.data_ptr(), vir.data_ptr(), dvals.data_ptr(), y.data_ptr(), int(y.shape[0]),
+                                  eta.data_ptr(), mu.data_ptr()))
+
+
+def assoc_spa(X, proj, Minv, C, mu, w, score, var, work, p, status, iters):
+    """Saddlepoint p-values of the b variants of one block (slmm_assoc_spa): X (n x b) and proj (c x b) as
+    assoc_genotypes leaves them for P = W C, Minv = (C'WC)^-1 (c x c), C (n x c), mu / w (n), score / var (b); work:
+    n * b float64 scratch; p (float64), status and iters (int32) receive b values each."""
+    n, b = int(X.shape[0]), int(X.shape[1])
+    check(lib().slmm_assoc_spa(X.data_ptr(), n, b, proj.data_ptr(), int(C.shape[1]), Minv.data_ptr(), C.data_ptr(),
+                               mu.data_ptr(), w.data_ptr(), score.data_ptr(), var.data_ptr(), work.data_ptr(),
+                               p.data_ptr(), status.data_ptr(), iters.data_ptr()))
+
+
 # ------------------------------------------------------------------------------------------------ symbolic
 class SymbolicView(object):
     """Host-only symbolic analysis (no GPU needed)."""
