@@ -12,6 +12,7 @@ All sparse / factorization arithmetic runs in libscilmm_b200.so on the GPU.  The
 which is the structural change against the reference (it re-analyses on every call, :22-26 from :92).
 There is no CPU fallback: without the CUDA library these functions raise.
 """
+import functools
 import hashlib
 import time
 
@@ -272,7 +273,7 @@ class RemlSession(object):
         return B200Factor(self.eng)
 
     def fixed_effects(self):
-        """V^-1 C, chol(C'V^-1C), mu, beta, V^-1 y   (reference :29-34, one multi-RHS solve)."""
+        """V^-1 C, chol(C'V^-1C), beta, V^-1 y, V^-1 (y - C beta)   (reference :29-34, one multi-RHS solve)."""
         return self._fixed_effects_finish(self._fixed_effects_start(overlap=False))
 
     def _fixed_effects_start(self, overlap=True):
@@ -303,39 +304,61 @@ class RemlSession(object):
         CtViy = (self.C.t() @ Viy).cpu().numpy()
         chol = la.cho_factor(CtViC)
         beta = la.cho_solve(chol, CtViy)
-        return ViC, chol, beta, Viy
+        Vir = Viy - ViC @ self.torch.from_numpy(beta).to("cuda")       # V^-1 (y - C beta) by linearity
+        return ViC, chol, beta, Viy, Vir
+
+    def nll(self, logdet, beta, Vir, chol, reml):
+        """Negative log-likelihood (reference :37-46) at the factored V from what fixed_effects() returned."""
+        r = self.y - self.C @ self.torch.from_numpy(beta).to("cuda")
+        nll = 0.5 * (float(r @ Vir) + self.n * LOG_2PI + logdet)
+        if reml:
+            nll += 0.5 * 2 * np.sum(np.log(np.diag(chol[0])))
+        return nll
+
+    @functools.cached_property
+    def copy_stream(self):
+        """CUDA stream of the host -> device copies that run under device work: probe and genotype blocks."""
+        return self.torch.cuda.Stream()
+
+    def draw_probes(self, sim_num):
+        """The n x sim_num probe block of the next evaluation by functor.rng, as (Z, stream): Z drawn from the
+        reference's global numpy stream (rng='numpy') or returned by probe_source (rng='host_buffer'), stream None;
+        for rng='device' Z is None and stream is the evaluation index, the device stream that probes() draws only the
+        local columns from."""
+        if self.functor.rng == 'numpy':
+            return np.random.randn(self.n, sim_num), None
+        if self.functor.rng == 'host_buffer':
+            return self.functor.probe_source(self.n, sim_num), None
+        return None, self.n_eval
 
     def prefetch_probes(self, sim_num, Z, col_begin, col_end):
-        """Host probe block -> device BEFORE the factorization is queued, on a copy stream of its own: the DMA of the
-        local columns (207 MB at 128 columns and 250K individuals) then runs under the factorization instead of
-        after it.  Returns (device block of the local columns, event) or None when the block is drawn on the device."""
+        """The local columns [col_begin, col_end) of the probe block Z (or of draw_probes() when Z is None) on the
+        device: (device block, event to wait for or None), or (None, None) when the block is drawn on the device.
+        Called BEFORE the factorization is queued: a whole contiguous float64 host tensor (pinned) goes up on the copy
+        stream, so its DMA (207 MB at 128 columns and 250K individuals) runs under the factorization instead of after
+        it; a host slice goes up by one pitched DMA; a CUDA block is copied, as the probe solve works in place."""
         torch = self.torch
         if Z is None:
-            if self.functor.rng == 'numpy':               # the reference's global stream: the whole block is drawn
-                Z = np.random.randn(self.n, sim_num)
-            elif self.functor.rng == 'host_buffer':       # caller-supplied host block (pinned tensor or ndarray)
-                Z = self.functor.probe_source(self.n, sim_num)
-            else:
-                return None
-        if torch.is_tensor(Z) and Z.is_cuda:               # a copy: the probe solve works in place
+            Z, _ = self.draw_probes(sim_num)
+        if Z is None:
+            return None, None
+        if torch.is_tensor(Z) and Z.is_cuda:
             return Z[:, col_begin:col_end].clone(memory_format=torch.contiguous_format), None
-        sliced = bool(col_begin or col_end != Z.shape[1])
-        if torch.is_tensor(Z) and not sliced and Z.dtype == torch.float64 and Z.is_contiguous():
-            if getattr(self, "_copy_stream", None) is None:
-                self._copy_stream = torch.cuda.Stream()
-            with torch.cuda.stream(self._copy_stream):
-                Zd = Z.to("cuda", non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record(self._copy_stream)
-            Zd.record_stream(torch.cuda.current_stream())
-            return Zd, ev
         if not torch.is_tensor(Z):
             Z = np.ascontiguousarray(Z, dtype=np.float64)
-            # only the local columns are uploaded, by one pitched DMA (no packing of the slice on the host)
-            return (_eng.upload_columns(Z, col_begin, col_end, torch) if sliced else _eng.to_device(Z, torch)), None
-        if sliced and Z.is_contiguous() and Z.dtype == torch.float64:
+        sliced = bool(col_begin or col_end != Z.shape[1])
+        if torch.is_tensor(Z) and not (Z.dtype == torch.float64 and Z.is_contiguous()):
+            return (Z[:, col_begin:col_end] if sliced else Z).contiguous().to("cuda", non_blocking=True), None
+        if sliced:                                     # no packing of the slice on the host
             return _eng.upload_columns(Z, col_begin, col_end, torch), None
-        return (Z[:, col_begin:col_end] if sliced else Z).contiguous().to("cuda", non_blocking=True), None
+        if not torch.is_tensor(Z):
+            return _eng.to_device(Z, torch), None
+        with torch.cuda.stream(self.copy_stream):
+            Zd = Z.to("cuda", non_blocking=True)
+            ev = torch.cuda.Event()
+            ev.record(self.copy_stream)
+        Zd.record_stream(torch.cuda.current_stream())
+        return Zd, ev
 
     def probes(self, sim_num, Z=None, col_begin=0, col_end=None, pre=None, probe_stream=None):
         """W = V^-1 (L Z)[argsort P]   (reference :49-52) for the probe columns [col_begin, col_end) of the
@@ -343,35 +366,14 @@ class RemlSession(object):
         backward half-sweep on Z (solve mode 3) replaces L Z and the full solve.  rng == 'device' draws ONLY those
         columns, from the counter-based stream keyed by (functor.seed, evaluation index or probe_stream, row, global
         column): the same values for any number of GPUs.  pre: what prefetch_probes returned for the same arguments."""
-        torch = self.torch
         col_end = sim_num if col_end is None else col_end
-        if pre is not None:
-            Zd, ev = pre
-            if ev is not None:
-                torch.cuda.current_stream().wait_event(ev)
-            return self.eng.solve_(Zd, mode=3)
-        if Z is None:
-            if self.functor.rng == 'numpy':               # the reference's global stream: the whole block is drawn
-                Z = np.random.randn(self.n, sim_num)
-            elif self.functor.rng == 'host_buffer':       # caller-supplied host block (pinned tensor or ndarray)
-                Z = self.functor.probe_source(self.n, sim_num)
-            else:
-                stream = self.n_eval if probe_stream is None else probe_stream
-                Z = self.eng.probe_normals(self.n, col_end - col_begin, col_begin, self.functor.seed, stream)
-                return self.eng.solve_(Z, mode=3)
-        sliced = bool(col_begin or col_end != Z.shape[1])
-        if not torch.is_tensor(Z):
-            Z = np.ascontiguousarray(Z, dtype=np.float64)
-            # only the local columns are uploaded, by one pitched DMA (no packing of the slice on the host)
-            Z = _eng.upload_columns(Z, col_begin, col_end, torch) if sliced else _eng.to_device(Z, torch)
-        elif not Z.is_cuda:
-            if sliced and Z.is_contiguous() and Z.dtype == torch.float64:
-                Z = _eng.upload_columns(Z, col_begin, col_end, torch)
-            else:
-                Z = (Z[:, col_begin:col_end] if sliced else Z).contiguous().to("cuda", non_blocking=True)
-        else:                                          # a copy: the caller's block is not overwritten
-            Z = Z[:, col_begin:col_end].clone(memory_format=torch.contiguous_format)
-        return self.eng.solve_(Z, mode=3)
+        Zd, ev = self.prefetch_probes(sim_num, Z, col_begin, col_end) if pre is None else pre
+        if Zd is None:
+            stream = self.n_eval if probe_stream is None else probe_stream
+            Zd = self.eng.probe_normals(self.n, col_end - col_begin, col_begin, self.functor.seed, stream)
+        elif ev is not None:
+            self.torch.cuda.current_stream().wait_event(ev)
+        return self.eng.solve_(Zd, mode=3)
 
     def _scan_blocks(self, sigmas, G, spans, red_len, reduce, finish, timing=None):
         """The genotype block pipeline of the association scan and the region tests.  For each column span (j0, j1) of
@@ -386,8 +388,7 @@ class RemlSession(object):
         torch = self.torch
         n = self.n
         self.factor_at(sigmas)
-        ViC, chol, beta, Viy = self.fixed_effects()
-        Vir = Viy - ViC @ torch.from_numpy(beta).to("cuda")
+        ViC, chol, _, _, Vir = self.fixed_effects()
         P = torch.cat([ViC, Vir.unsqueeze(1)], dim=1).contiguous()       # n x (c + 1)
         c1 = P.shape[1]
         block = max(j1 - j0 for j0, j1 in spans)
@@ -400,9 +401,7 @@ class RemlSession(object):
                       nobs=torch.empty(block, dtype=torch.int64, device="cuda"),
                       gsum=torch.empty(block, dtype=torch.int64, device="cuda"),
                       red=torch.empty(nred, dtype=torch.float64, device="cuda")) for _ in range(2)]
-        if getattr(self, "_copy_stream", None) is None:
-            self._copy_stream = torch.cuda.Stream()
-        copy, main = self._copy_stream, torch.cuda.current_stream()
+        copy, main = self.copy_stream, torch.cuda.current_stream()
         uploaded = torch.cuda.Event()
         strides = [None]
         finish_s = self.last["finish_s"] = []          # host seconds per span: copies back + finish
@@ -464,9 +463,7 @@ class RemlSession(object):
         variants through _scan_blocks, with a column sum of squares as the reduction and the c x c finalisation on the
         host.  Returns a dict of arrays of length col_end - col_begin in the units of the standardised y: beta, se,
         chi2, p, af, n_obs, and the score t with its variance xPx (score, var).  timing: as for _scan_blocks."""
-        if self.C.shape[1] > ASSOC_MAX_COVARIATES:
-            raise ValueError("the association scan takes at most %d covariates, got %d"
-                             % (ASSOC_MAX_COVARIATES, self.C.shape[1]))
+        _check_scan_covariates(self.C.shape[1])
         col_end = G.shape[1] if col_end is None else int(col_end)
         m_loc = max(col_end - col_begin, 0)
         out = {k: np.full(m_loc, np.nan) for k in ("beta", "se", "chi2", "p", "af", "score", "var")}
@@ -503,9 +500,7 @@ class RemlSession(object):
         two), and each span goes through _scan_blocks with the region Gram (slmm_assoc_region_gram) as the
         reduction.  weights: length-m per-variant weights, or None for the default beta(maf; 1, 25).  Returns a dict of
         arrays of length reg_end - reg_begin in the units of the standardised y.  timing: as for _scan_blocks."""
-        if self.C.shape[1] > ASSOC_MAX_COVARIATES:
-            raise ValueError("the association scan takes at most %d covariates, got %d"
-                             % (ASSOC_MAX_COVARIATES, self.C.shape[1]))
+        _check_scan_covariates(self.C.shape[1])
         bounds = np.asarray(bounds, dtype=np.int64)
         reg_end = len(bounds) - 1 if reg_end is None else int(reg_end)
         R = max(reg_end - reg_begin, 0)
@@ -575,8 +570,7 @@ class RemlSession(object):
         if c + 1 > BLUP_MAX_COLUMNS:
             raise ValueError("blup takes at most %d covariates, got %d" % (BLUP_MAX_COLUMNS - 1, c))
         self.factor_at(sigmas)
-        ViC, chol, beta, Viy = self.fixed_effects()
-        u = Viy - ViC @ torch.from_numpy(beta).to("cuda")
+        ViC, chol, beta, _, u = self.fixed_effects()
         X = torch.cat([u.unsqueeze(1), ViC], dim=1).contiguous()          # [u | V^-1 C], c + 1 <= 32 columns
         Minv = torch.from_numpy(la.cho_solve(chol, np.eye(c))).to("cuda")
         N, K = matset.n, len(sigmas) - 1
@@ -703,22 +697,16 @@ class RemlSession(object):
         pre = self.prefetch_probes(sim_num, Z, lo, hi)      # a host block goes up under the factorization
         self.factor_at(sigmas)
         logdet = self.eng.logdet()
-        n = self.n
         pending = self._fixed_effects_start(self.overlap)   # narrow solve on the auxiliary stream ...
         # ... beside the probe pipeline
         W = self.probes(sim_num, Z, lo, hi, pre=pre, probe_stream=probe_stream)
         self.n_eval += 1
-        ViC, chol, beta, Viy = self._fixed_effects_finish(pending)
-        beta_t = torch.from_numpy(beta).to("cuda")
-        Vir = Viy - ViC @ beta_t                       # V^-1 (y - C beta) by linearity
+        ViC, chol, beta, Viy, Vir = self._fixed_effects_finish(pending)
         if ai:
             if not all(self._sym):
                 raise ValueError("the average-information matrix needs symmetric components")
             ai_pending = self._ai_start(Vir, ViC)      # forward sweep on the auxiliary stream ...
-        r = self.y - self.C @ beta_t
-        nll = 0.5 * (float(r @ Vir) + n * LOG_2PI + logdet)
-        if reml:
-            nll += 0.5 * 2 * np.sum(np.log(np.diag(chol[0])))
+        nll = self.nll(logdet, beta, Vir, chol, reml)
         c = self.C.shape[1]
         K = self.K
         comp1 = torch.zeros(K, dtype=torch.float64, device="cuda")
@@ -906,13 +894,7 @@ def _aireml_fit(functor, mats, covariates, y, reml, sim_num, verbose):
     if not all(ses._sym):
         raise ValueError("aireml=True needs symmetric components (AI = -hess holds only for symmetric A_k); "
                          "asymmetric: %s" % [k for k in range(ses.K) if not ses._sym[k]])
-    Z, stream = None, None
-    if functor.rng == 'numpy':
-        Z = np.random.randn(ses.n, sim_num)
-    elif functor.rng == 'host_buffer':
-        Z = functor.probe_source(ses.n, sim_num)
-    else:
-        stream = ses.n_eval
+    Z, stream = ses.draw_probes(sim_num)
     converged, it = False, 0
     while it < AIREML_MAX_ITER:
         it += 1
@@ -1019,14 +1001,8 @@ def REML(cholesky_func, mats, covariates, y, reml=True, sim_num=100, verbose=Fal
         varcomp_estimates = estimate_var_comps(functor, mats, covariates, y, reml, sim_num, verbose)
     ses = functor._session(mats, covariates, y)
     factor = ses.factor_at(varcomp_estimates)
-    ViC, chol, fixed_effects, Viy = ses.fixed_effects()
-    torch = ses.torch
-    beta_t = torch.from_numpy(fixed_effects).to("cuda")
-    Vir = Viy - ViC @ beta_t
-    r = ses.y - ses.C @ beta_t
-    nll = 0.5 * (float(r @ Vir) + y.size * LOG_2PI + factor.logdet())
-    if reml:
-        nll += 0.5 * 2 * np.sum(np.log(np.diag(chol[0])))
+    ViC, chol, fixed_effects, Viy, Vir = ses.fixed_effects()
+    nll = ses.nll(factor.logdet(), fixed_effects, Vir, chol, reml)
     hess = _hess_device(ses, ses.eng, pre=(ViC, chol, Viy))
     sigmas_sigmas = np.sqrt(np.diag(la.inv(-hess)) * (1 + 1.0 / sim_num))
     out = {"covariance coefficients": varcomp_estimates,
@@ -1046,6 +1022,38 @@ ASSOC_MAX_COVARIATES = 31   # [V^-1 C | V^-1 r] is projected in registers, c + 1
 # 40.7 / 41.9 / 49.3 at widths 512 / 256 / 128 (profiles/r05_assoc_scan.json).  The width is chosen so that these fit
 # in half the free memory; the other half covers the plan of a narrower tail block, which is no larger.
 ASSOC_BYTES_PER_ENTRY = 50
+
+
+def _check_genotypes(G, n):
+    """G as a C- or Fortran-ordered (n, m) int8 ndarray (a copy in C order when it is neither); ValueError otherwise."""
+    G = np.asarray(G)
+    if G.ndim != 2 or G.dtype != np.int8:
+        raise ValueError("G must be a 2-D int8 array of allele counts (negative = missing)")
+    if G.shape[0] != n:
+        raise ValueError("G has %d rows for %d individuals" % (G.shape[0], n))
+    if not (G.flags.c_contiguous or G.flags.f_contiguous):
+        G = np.ascontiguousarray(G)
+    return G
+
+
+def _check_sigmas(sigmas, K):
+    """sigmas as a float array of K + 1 variance components (the residual last); ValueError otherwise."""
+    sigmas = np.asarray(sigmas, dtype=float)
+    if sigmas.shape != (K + 1,):
+        raise ValueError("need %d variance components (the residual last), got %d" % (K + 1, sigmas.size))
+    return sigmas
+
+
+def _check_scan_covariates(c):
+    if c > ASSOC_MAX_COVARIATES:
+        raise ValueError("the association scan takes at most %d covariates, got %d" % (ASSOC_MAX_COVARIATES, c))
+
+
+def _scan_width(n, bytes_per_entry, floor):
+    """Columns per genotype block: ASSOC_BLOCK, or as many as fit bytes_per_entry per (individual, column) into half
+    the free device memory, and at least `floor`."""
+    free = _eng.require_cuda().cuda.mem_get_info()[0]
+    return int(max(floor, min(ASSOC_BLOCK, free // 2 // (bytes_per_entry * n))))
 
 
 def _scan_session(functor, mats, covariates, y):
@@ -1077,35 +1085,17 @@ def association(cholesky_func, mats, covariates, y, sigmas, G):
     With torch.distributed initialised every rank scans a contiguous slice of the variants and one all-reduce gives
     every rank the whole result."""
     functor = _need_functor(cholesky_func)
-    torch = _eng.require_cuda()
-    G = np.asarray(G)
-    if G.ndim != 2 or G.dtype != np.int8:
-        raise ValueError("G must be a 2-D int8 array of allele counts (negative = missing)")
-    if G.shape[0] != y.shape[0]:
-        raise ValueError("G has %d rows for %d individuals" % (G.shape[0], y.shape[0]))
-    if not (G.flags.c_contiguous or G.flags.f_contiguous):
-        G = np.ascontiguousarray(G)
-    if np.shape(covariates)[1] > ASSOC_MAX_COVARIATES:
-        raise ValueError("the association scan takes at most %d covariates, got %d"
-                         % (ASSOC_MAX_COVARIATES, np.shape(covariates)[1]))
-    sigmas = np.asarray(sigmas, dtype=float)
-    if sigmas.shape != (len(mats) + 1,):
-        raise ValueError("need %d variance components (the residual last), got %d" % (len(mats) + 1, sigmas.size))
+    G = _check_genotypes(G, y.shape[0])
+    _check_scan_covariates(np.shape(covariates)[1])
+    sigmas = _check_sigmas(sigmas, len(mats))
     scale = y.std()
     ses = _scan_session(functor, mats, covariates, y / scale)
     n, m = G.shape
-    free = torch.cuda.mem_get_info()[0]
-    block = int(max(8, min(ASSOC_BLOCK, free // 2 // (ASSOC_BYTES_PER_ENTRY * n))))
+    block = _scan_width(n, ASSOC_BYTES_PER_ENTRY, 8)
     rank, world = _shard.rank_world()
     lo, hi = _shard.column_block(m, rank, world)
-    part = ses.association(sigmas, G, block, lo, hi)
     keys = ("beta", "se", "chi2", "p", "af", "n_obs")
-    if world > 1:
-        full = torch.zeros(len(keys), m, dtype=torch.float64, device="cuda")
-        full[:, lo:hi] = torch.from_numpy(np.stack([part[k].astype(np.float64) for k in keys]))
-        full = _shard.allreduce_sum_(full).cpu().numpy()
-        part = {k: full[i] for i, k in enumerate(keys)}
-        part["n_obs"] = part["n_obs"].astype(np.int64)
+    part = _shard.gather_slices(ses.association(sigmas, G, block, lo, hi), keys, m, lo, hi, "cuda")
     part["beta"] = part["beta"] * scale
     part["se"] = part["se"] * scale
     return {k: part[k] for k in keys}
@@ -1224,24 +1214,12 @@ def region_test(cholesky_func, mats, covariates, y, sigmas, G, bounds, weights=N
     burden_chi2, burden_p, skat_q, skat_p.  With torch.distributed initialised every rank tests a contiguous slice of
     the regions and one all-reduce gives every rank the whole result."""
     functor = _need_functor(cholesky_func)
-    G = np.asarray(G)
-    if G.ndim != 2 or G.dtype != np.int8:
-        raise ValueError("G must be a 2-D int8 array of allele counts (negative = missing)")
-    if G.shape[0] != y.shape[0]:
-        raise ValueError("G has %d rows for %d individuals" % (G.shape[0], y.shape[0]))
-    if not (G.flags.c_contiguous or G.flags.f_contiguous):
-        G = np.ascontiguousarray(G)
-    if np.shape(covariates)[1] > ASSOC_MAX_COVARIATES:
-        raise ValueError("the association scan takes at most %d covariates, got %d"
-                         % (ASSOC_MAX_COVARIATES, np.shape(covariates)[1]))
-    sigmas = np.asarray(sigmas, dtype=float)
-    if sigmas.shape != (len(mats) + 1,):
-        raise ValueError("need %d variance components (the residual last), got %d" % (len(mats) + 1, sigmas.size))
+    G = _check_genotypes(G, y.shape[0])
+    _check_scan_covariates(np.shape(covariates)[1])
+    sigmas = _check_sigmas(sigmas, len(mats))
     n, m = G.shape
     bounds, weights = check_regions(bounds, weights, m)
-    torch = _eng.require_cuda()
-    free = torch.cuda.mem_get_info()[0]
-    block = int(max(8, min(ASSOC_BLOCK, free // 2 // (ASSOC_BYTES_PER_ENTRY * n))))
+    block = _scan_width(n, ASSOC_BYTES_PER_ENTRY, 8)
     if np.diff(bounds).max() > block:
         raise ValueError("the widest region (%d variants) does not fit the %d columns that device memory allows"
                          % (np.diff(bounds).max(), block))
@@ -1250,14 +1228,8 @@ def region_test(cholesky_func, mats, covariates, y, sigmas, G, bounds, weights=N
     R = bounds.size - 1
     rank, world = _shard.rank_world()
     lo, hi = _shard.column_block(R, rank, world)
-    part = ses.region_test(sigmas, G, bounds, weights, block, lo, hi)
-    if world > 1:
-        full = torch.zeros(len(REGION_KEYS), R, dtype=torch.float64, device="cuda")
-        full[:, lo:hi] = torch.from_numpy(np.stack([part[k].astype(np.float64) for k in REGION_KEYS]))
-        full = _shard.allreduce_sum_(full).cpu().numpy()
-        part = {k: full[i] for i, k in enumerate(REGION_KEYS)}
-        for k in ("n_variants", "n_poly"):
-            part[k] = part[k].astype(np.int64)
+    part = _shard.gather_slices(ses.region_test(sigmas, G, bounds, weights, block, lo, hi), REGION_KEYS, R, lo, hi,
+                                "cuda")
     part["burden_beta"] = part["burden_beta"] * scale
     part["burden_se"] = part["burden_se"] * scale
     return {k: part[k] for k in REGION_KEYS}
@@ -1301,7 +1273,6 @@ def blup(cholesky_func, mats, covariates, y, sigmas, pev_probes=0):
     torch.distributed initialised every rank sweeps a slice of the probe blocks; the PEV is the same bits for any
     number of ranks."""
     functor = _need_functor(cholesky_func)
-    torch = _eng.require_cuda()
     y = np.asarray(y, dtype=np.float64)
     C = np.asarray(covariates, dtype=np.float64)
     K = len(mats)
@@ -1310,9 +1281,7 @@ def blup(cholesky_func, mats, covariates, y, sigmas, pev_probes=0):
         raise ValueError("y must be a vector")
     if K == 0 or any(m.shape != (N, N) for m in mats):
         raise ValueError("every matrix must be N x N with N = len(y) = %d" % N)
-    sigmas = np.asarray(sigmas, dtype=float)
-    if sigmas.shape != (K + 1,):
-        raise ValueError("need %d variance components (the residual last), got %d" % (K + 1, sigmas.size))
+    sigmas = _check_sigmas(sigmas, K)
     if C.ndim != 2 or C.shape[0] != N:
         raise ValueError("covariates must be N x c with N = %d" % N)
     if not np.all(np.isfinite(C)):
@@ -1328,6 +1297,7 @@ def blup(cholesky_func, mats, covariates, y, sigmas, pev_probes=0):
     p = int(pev_probes)
     if p < 0 or p == 1:
         raise ValueError("pev_probes must be 0 or at least 2")
+    torch = _eng.require_cuda()
     scale = y[obs].std()
     if n == N:
         ses = _scan_session(functor, mats, covariates, y / scale)
@@ -1500,13 +1470,7 @@ def glmm(cholesky_func, mats, covariates, y, sim_num=100, verbose=False):
     if not all(ses._sym):
         raise ValueError("glmm needs symmetric relationship matrices; asymmetric: %s"
                          % [k for k in range(K) if not ses._sym[k]])
-    Z, stream = None, None
-    if functor.rng == 'numpy':
-        Z = np.random.randn(n, sim_num)
-    elif functor.rng == 'host_buffer':
-        Z = functor.probe_source(n, sim_num)
-    else:
-        stream = ses.n_eval
+    Z, stream = ses.draw_probes(sim_num)
     y_d = _eng.to_device(y, torch)
     dvals = ses.matset.device_arrays(K)[2]
     eta_d = torch.empty(n, dtype=torch.float64, device="cuda")
@@ -1572,15 +1536,8 @@ def glmm_association(cholesky_func, mats, covariates, y, fit, G, spa_cutoff=2.0)
     functor = _need_functor(cholesky_func)
     C, y = _check_binary(mats, covariates, y)
     n, K = y.shape[0], len(mats)
-    G = np.asarray(G)
-    if G.ndim != 2 or G.dtype != np.int8:
-        raise ValueError("G must be a 2-D int8 array of allele counts (negative = missing)")
-    if G.shape[0] != n:
-        raise ValueError("G has %d rows for %d individuals" % (G.shape[0], n))
-    if not (G.flags.c_contiguous or G.flags.f_contiguous):
-        G = np.ascontiguousarray(G)
-    if C.shape[1] > ASSOC_MAX_COVARIATES:
-        raise ValueError("the association scan takes at most %d covariates, got %d" % (ASSOC_MAX_COVARIATES, C.shape[1]))
+    G = _check_genotypes(G, n)
+    _check_scan_covariates(C.shape[1])
     spa_cutoff = float(spa_cutoff)
     if not spa_cutoff >= 0.0:
         raise ValueError("spa_cutoff must be >= 0")
@@ -1590,32 +1547,23 @@ def glmm_association(cholesky_func, mats, covariates, y, fit, G, spa_cutoff=2.0)
     mu, w, Yt = (np.asarray(fit[k], dtype=np.float64) for k in ("mu", "weights", "working y"))
     if any(a.shape != (n,) or not np.all(np.isfinite(a)) for a in (mu, w, Yt)) or not np.all(w > 0):
         raise ValueError("fit's mu, weights and working y must be finite vectors of length n = %d (weights > 0)" % n)
-    torch = _eng.require_cuda()
     ses = _glmm_session(functor, mats, covariates, Yt, w)
     m = G.shape[1]
     rank, world = _shard.rank_world()
     lo, hi = _shard.column_block(m, rank, world)
-    block = int(max(8, min(ASSOC_BLOCK, torch.cuda.mem_get_info()[0] // 2 // (ASSOC_BYTES_PER_ENTRY * n))))
-    part = ses.association(np.concatenate([tau, [1.0]]), G, block, lo, hi)
+    part = ses.association(np.concatenate([tau, [1.0]]), G, _scan_width(n, ASSOC_BYTES_PER_ENTRY, 8), lo, hi)
     U, V = part["score"], part["var"]
     with np.errstate(invalid="ignore", divide="ignore"):
         z = U / np.sqrt(V)
     part["p_normal"] = part["p"].copy()
     part["spa"] = np.zeros(hi - lo, dtype=np.int8)
     flag = np.flatnonzero(np.isfinite(z) & (np.abs(np.nan_to_num(z)) > spa_cutoff))
-    sblock = int(max(1, min(ASSOC_BLOCK, torch.cuda.mem_get_info()[0] // 2 // (SPA_BYTES_PER_ENTRY * n))))
-    ps, status, iters = ses.spa(G, lo + flag, U[flag], V[flag], mu, w, sblock)
+    ps, status, iters = ses.spa(G, lo + flag, U[flag], V[flag], mu, w, _scan_width(n, SPA_BYTES_PER_ENTRY, 1))
     ses.last["spa_iters"] = iters
     part["spa"][flag] = status
     ok = status == 1
     part["p"][flag[ok]] = ps[ok]
-    if world > 1:
-        full = torch.zeros(len(GLMM_ASSOC_KEYS), m, dtype=torch.float64, device="cuda")
-        full[:, lo:hi] = torch.from_numpy(np.stack([part[k].astype(np.float64) for k in GLMM_ASSOC_KEYS]))
-        full = _shard.allreduce_sum_(full).cpu().numpy()
-        part = {k: full[i] for i, k in enumerate(GLMM_ASSOC_KEYS)}
-        part["spa"] = part["spa"].astype(np.int8)
-        part["n_obs"] = part["n_obs"].astype(np.int64)
+    part = _shard.gather_slices(part, GLMM_ASSOC_KEYS, m, lo, hi, "cuda")
     return {k: part[k] for k in GLMM_ASSOC_KEYS}
 
 

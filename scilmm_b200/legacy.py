@@ -50,7 +50,7 @@ def LMM(cholesky, mats, covariates, y, with_intercept=True, reml=True, sim_num=1
     mats_coefficients = compute_sigmas(functor, mats, covariates, y, reml, sim_num, verbose)
     ses = functor._session(mats, covariates, y)
     ses.factor_at(mats_coefficients)
-    _, chol, fixed_effects, _ = ses.fixed_effects()
+    _, chol, fixed_effects, _, _ = ses.fixed_effects()
     p_values = compute_fixed_effects_p_value(y, covariates, fixed_effects, chol)
     sigmas_sigmas = compute_sig_of_sig(ses, sim_num)
     return {"covariance coefficients": mats_coefficients,

@@ -80,3 +80,19 @@ def allreduce_sum_(t):
     if dist is not None:
         dist.all_reduce(t)
     return t
+
+
+def gather_slices(part, keys, total, lo, hi, device):
+    """Whole length-`total` result arrays on every rank from each rank's slice [lo, hi): part[k] holds this rank's
+    entries of key k.  One all-reduce of a float64 (len(keys), total) tensor on `device`, zero outside each rank's
+    slice (NaN entries survive the sum); every array comes back with the dtype of its part[k].  Without a process
+    group, part itself."""
+    dist = active_group()
+    if dist is None:
+        return part
+    import torch
+    full = torch.zeros(len(keys), total, dtype=torch.float64, device=device)
+    full[:, lo:hi] = torch.from_numpy(np.stack([part[k].astype(np.float64) for k in keys]))
+    dist.all_reduce(full)
+    full = full.cpu().numpy()
+    return {k: full[i].astype(part[k].dtype, copy=False) for i, k in enumerate(keys)}

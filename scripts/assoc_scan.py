@@ -129,8 +129,7 @@ def main():
 
     # first block against a device full solve: gamma = t / (x'V^-1 x - q' M^-1 q) with V^-1 x from mode 0
     w, res = first_block
-    ViC, chol, beta, Viy = ses.fixed_effects()
-    Vir = Viy - ViC @ torch.from_numpy(beta).to("cuda")
+    ViC, chol, _, _, Vir = ses.fixed_effects()
     P = torch.cat([ViC, Vir.unsqueeze(1)], dim=1).contiguous()
     g8 = torch.empty(n * w, dtype=torch.int8, device="cuda")
     strides = E.upload_genotype_block(G, 0, w, g8)

@@ -105,8 +105,7 @@ def main():
     colmap = np.full(N, -1, dtype=np.int32)
     colmap[idx] = np.arange(n, dtype=np.int32)
     cm = E.to_device(colmap, torch)
-    ViC, chol_c, beta, Viy = ses.fixed_effects()
-    u = Viy - ViC @ torch.from_numpy(beta).to("cuda")
+    ViC, _, _, _, u = ses.fixed_effects()
     X = torch.cat([u.unsqueeze(1), ViC], dim=1).contiguous()
     spmm = {}
     for ks in ms.pattern_groups(2):

@@ -27,7 +27,7 @@ T("lmul", lambda: ses.eng.lmul(Z))
 U = ses.eng.lmul(Z)
 T("solve_ 128", lambda: ses.eng.solve_(U.clone()))
 W = ses.eng.solve_(U.clone())
-ViC, chol_, beta, Viy = ses.fixed_effects()
+ViC, chol_, beta, Viy, _ = ses.fixed_effects()
 X = torch.cat([W, Viy.unsqueeze(1)], dim=1).contiguous()
 T("cat X", lambda: torch.cat([W, Viy.unsqueeze(1)], dim=1).contiguous())
 groups = ses.matset.pattern_groups(2)

@@ -69,7 +69,7 @@ def main():
         p1_s = time.time() - t0
         z = part["score"] / np.sqrt(part["var"])
         flag = np.flatnonzero(np.isfinite(z) & (np.abs(np.nan_to_num(z)) > 2.0))
-        sblock = int(max(1, min(S.ASSOC_BLOCK, torch.cuda.mem_get_info()[0] // 2 // (S.SPA_BYTES_PER_ENTRY * n))))
+        sblock = S._scan_width(n, S.SPA_BYTES_PER_ENTRY, 1)
         ses.spa(G, flag[:8], part["score"][flag[:8]], part["var"][flag[:8]], fit["mu"], fit["weights"], 8)  # warm-up
         timing = []
         torch.cuda.synchronize()

@@ -1,6 +1,9 @@
 """CPU checks of the association-scan oracle (oracle/association.py): its coefficient and standard error are those of
 an explicit GLS refit with the variant as one more covariate, and the genotype decoding rules (missing values, allele
-frequency, counts, NaN for monomorphic variants and for variants in the span of the covariates)."""
+frequency, counts, NaN for monomorphic variants and for variants in the span of the covariates).  Also the input rules
+of association(), region_test() and blup(), which need no device."""
+import sys
+
 import numpy as np
 import pytest
 
@@ -77,3 +80,23 @@ def test_decoding_rules(golden_small):
     bad[7, 6] = 3
     with pytest.raises(ValueError):
         oa.decode(bad)
+
+
+def test_refused_inputs_need_no_device(golden_small):
+    """association(), region_test() and blup() check G, the variance components and the covariates before they look
+    for a device: bad input raises ValueError on any host, not the missing-device RuntimeError."""
+    import scilmm_b200.SparseCholesky  # noqa: F401
+    S = sys.modules["scilmm_b200.SparseCholesky"]
+    g = golden_small
+    mats, sig, y, cov = g.mats("k3"), g["sig_k4"], g["y"], g["cov"]
+    G = make_genotypes(g.n, 40, 5)
+    wide = np.hstack([cov, np.random.default_rng(0).standard_normal((g.n, 32 - cov.shape[1]))])
+    scans = (lambda C, s, G: S.association(S.SparseCholesky(), mats, C, y, s, G),
+             lambda C, s, G: S.region_test(S.SparseCholesky(), mats, C, y, s, G, np.array([0, 20, 40])))
+    for call in scans:
+        for C, s, bad_G in ((cov, sig, G.astype(np.int16)), (cov, sig, G[1:]), (cov, sig[1:], G), (wide, sig, G)):
+            with pytest.raises(ValueError):
+                call(C, s, bad_G)
+    for C, s in ((cov, sig[1:]), (cov, np.r_[sig, 0.1]), (wide, sig)):
+        with pytest.raises(ValueError):
+            S.blup(S.SparseCholesky(), mats, C, y, s)

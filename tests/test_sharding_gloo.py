@@ -86,11 +86,48 @@ def test_two_rank_partition_and_allreduce():
     assert abs(nnz[0] - nnz[1]) <= 2 * np.diff(mats[0].indptr).max()      # balanced by nonzeros
 
 
+def _scan_result(total):
+    """A per-variant result as the scans return it: float64 with NaN slots, int64 counts, int8 flags with -1."""
+    rng = np.random.default_rng(2)
+    x = rng.standard_normal(total)
+    x[[0, 3, total - 1]] = np.nan
+    return {"p": x, "n_obs": rng.integers(0, 1 << 40, total), "spa": rng.integers(-1, 2, total).astype(np.int8)}
+
+
+def _gather_worker(rank, world, port, out):
+    os.environ["MASTER_ADDR"] = "127.0.0.1"
+    os.environ["MASTER_PORT"] = str(port)
+    dist.init_process_group("gloo", rank=rank, world_size=world)
+    try:
+        total = 7
+        lo, hi = sharding.column_block(total, rank, world)
+        part = {k: v[lo:hi].copy() for k, v in _scan_result(total).items()}
+        out[rank] = sharding.gather_slices(part, ("p", "n_obs", "spa"), total, lo, hi, "cpu")
+    finally:
+        dist.destroy_process_group()
+
+
+def test_two_rank_gather_slices():
+    """Slices of 3 and 4 entries: every rank gets the unsharded arrays, NaN slots and dtypes included."""
+    world = 2
+    mgr = mp.Manager()
+    out = mgr.dict()
+    mp.spawn(_gather_worker, args=(world, _free_port(), out), nprocs=world, join=True)
+    full = _scan_result(7)
+    assert (full["spa"] == -1).any()
+    for rank in range(world):
+        for k, v in full.items():
+            assert out[rank][k].dtype == v.dtype, (rank, k)
+            assert np.array_equal(out[rank][k], v, equal_nan=True), (rank, k)
+
+
 def test_partition_helpers_edge_cases():
     assert sharding.rank_world() == (0, 1)
     assert sharding.active_group() is None
     t = torch.ones(3)
     assert sharding.allreduce_sum_(t) is t and torch.all(t == 1)
+    part = _scan_result(5)
+    assert sharding.gather_slices(part, tuple(part), 5, 0, 5, "cpu") is part
     for s, w in ((128, 8), (100, 8), (3, 8), (0, 2)):
         blocks = [sharding.column_block(s, r, w) for r in range(w)]
         assert blocks[0][0] == 0 and blocks[-1][1] == s
